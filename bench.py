@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload train|detect|stress] [--batch B] [--collective peer|nccl] [--no-others]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic head outputs:
   train  (default)  match + hard-negative-mined CE + L1 loss, forward AND gradients, SSD300 (8732 priors, 1-10 gt/image)
@@ -18,6 +19,8 @@ sharded step in which every rank feeds rank 0's shard is compared bit for bit wi
 Rank 0 prints ONE JSON line.  `--impl reference` times the reference's own CPU implementation (the unmodified
 `Losses.ssd` / `Losses.inference` from oracle/_ref when it travelled with the tree, else the oracle port) on all host
 cores, on a bounded sample of the same workload.
+`--dump-outputs DIR` writes what the last timed step returned (losses and gradients, or the detections) as .npy files;
+the inputs depend only on the arguments, so the dumps of two builds can be compared file by file.
 """
 from __future__ import annotations
 
@@ -131,6 +134,35 @@ class ClockSampler:
                 "reasons": sorted(self.reasons), "samples_in_timed_region": len(timed)}
 
 
+DUMP_BYTES = 64_000_000 - 4096      # --dump-outputs: 64 MB in all, .npy headers included
+
+
+def dump_sample(whole, per_image, seed=0):
+    """Host copies of one step's outputs for --dump-outputs: float32 / float64 arrays (integers widened to float64,
+    exactly).  The `per_image` tensors share their leading batch axis; when the dump would exceed DUMP_BYTES they all
+    keep the same fixed, seeded subset of images, in batch order."""
+    def host(t):
+        return t.detach().cpu().numpy() if t.dtype.is_floating_point else t.detach().cpu().to(torch.float64).numpy()
+
+    out = {k: host(t) for k, t in whole.items()}
+    per_img = sum(t[0].numel() * (t.element_size() if t.dtype.is_floating_point else 8) for t in per_image.values())
+    B = next(iter(per_image.values())).shape[0]
+    keep = min(B, (DUMP_BYTES - sum(a.nbytes for a in out.values())) // per_img)
+    idx = None
+    if keep < B:
+        idx = np.sort(np.random.default_rng(seed).choice(B, keep, replace=False))
+    for k, t in per_image.items():
+        out[k] = host(t if idx is None else t[torch.from_numpy(idx).to(t.device)])
+    return out
+
+
+def dump_outputs(path, outputs):
+    os.makedirs(path, exist_ok=True)
+    for k, a in outputs.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+    print(f"bench.py: wrote {', '.join(f'{k}.npy {list(a.shape)}' for k, a in outputs.items())} to {path}", file=sys.stderr)
+
+
 def dist_env():
     return int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1")), int(os.environ.get("LOCAL_RANK", "0"))
 
@@ -194,8 +226,8 @@ def reference_inputs(workload, B):
 
 class ReferenceImpl:
     """The reference's CPU implementation of the path: the UNMODIFIED Losses.ssd / Losses.inference when the reference
-    sources are importable (oracle/ref_import: /root/reference in the build container, oracle/_ref on the GPU box),
-    else the oracle's port of them (torch-CPU ops, same algorithm)."""
+    sources are importable (oracle/ref_import: $SSD_REFERENCE_DIR or oracle/_ref), else the oracle's port of them
+    (torch-CPU ops, same algorithm)."""
 
     def __init__(self, workload):
         from oracle import ssd_oracle as O
@@ -287,14 +319,14 @@ def run_reference(args):
     warm = min(args.warmup, 1)
     for _ in range(warm):
         impl.step(data)
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
         impl.step(data)
     dt = (time.perf_counter() - t0) / steps
     val = B / dt
-    sample = (f"{impl.describe(B)} per step (bounded sample of the {args.batch}-image workload), {steps} timed steps "
-              f"(requested {args.steps}), torch {torch.__version__} CPU ops, {torch.get_num_threads()} threads")
+    sample = (f"{impl.describe(B)} per step (bounded sample of the {args.batch}-image workload), {steps} timed steps, "
+              f"torch {torch.__version__} CPU ops, {torch.get_num_threads()} threads")
     line = {
         "impl": "reference", "metric": metric_name(args.workload),
         "value": val, "unit": "images/s", "n_gpus": args.gpus, "steps": steps, "warmup": warm,
@@ -433,8 +465,9 @@ class LossRunner:
         self.ctx.close()
 
 
-def time_loss(args, rank, world, dev, sampler, workload, B, steps, warmup, kernel_alone=True, e2e=True):
-    """The training-head step (match + loss fwd + gradients) of `workload` ('train' or 'stress') at batch B per GPU."""
+def time_loss(args, rank, world, dev, sampler, workload, B, steps, warmup, kernel_alone=True, e2e=True, capture=False):
+    """The training-head step (match + loss fwd + gradients) of `workload` ('train' or 'stress') at batch B per GPU.
+    capture: r["outputs"] holds what the last timed step returned (see dump_outputs)."""
     from objectdetection_ssd_b200 import _lib, synth, priors as PR
     from objectdetection_ssd_b200.ctx import SparseRows, pinned_empty
     lib = _lib.load()
@@ -479,6 +512,8 @@ def time_loss(args, rank, world, dev, sampler, workload, B, steps, warmup, kerne
     if run.collective == "peer" and ctx.xchg_error():
         raise SystemExit("bench.py: a wait for a peer rank expired inside the sharded step (results invalid)")
     r = dict(ms_total=ms, launches=launches, P=P, algo=algo_bytes(P, "train"), collective=run.collective, kern_ms=None)
+    if capture:
+        r["outputs"] = dump_sample({"losses": losses, "loss_sums": sums}, {"grad_loc": gl, "grad_conf": gcf})
     # losses of set 0 (the data the end-to-end leg uses), for the e2e cross-check
     step(0)
     torch.cuda.synchronize()
@@ -562,7 +597,7 @@ def time_loss(args, rank, world, dev, sampler, workload, B, steps, warmup, kerne
     return r
 
 
-def time_detect(args, rank, world, dev, sampler, B, steps, warmup, workload="detect", e2e=True):
+def time_detect(args, rank, world, dev, sampler, B, steps, warmup, workload="detect", e2e=True, capture=False):
     from objectdetection_ssd_b200 import _lib, synth
     from objectdetection_ssd_b200.head import MultiboxHead
     from objectdetection_ssd_b200.ctx import SSDHeadContext, pinned_empty
@@ -608,6 +643,11 @@ def time_detect(args, rank, world, dev, sampler, B, steps, warmup, workload="det
     ms = max_over_ranks(e0.elapsed_time(e1), world, dev)
     r = dict(ms_total=ms, launches=launches, kern_ms=None, B=B, steps=steps, P=P, algo=algo_bytes(P, "detect"),
              kernel="detect kernels (whole step)", detections=int(out["cnt"].clamp(min=0).sum()))
+    if capture:
+        # slots past an image's count hold whatever the buffers held before: zeroed, they are not part of the result
+        valid = torch.arange(top_k, device=dev)[None, :] < out["cnt"][:, None]
+        r["outputs"] = dump_sample({}, {"cnt": out["cnt"], "boxes": out["boxes"] * valid[..., None],
+                                        **{k: out[k] * valid for k in ("prob", "cls", "prior")}})
     import ctypes
     nfb = ctypes.c_int32(-1)
     _lib.check(lib.ssdhead_detect_fallbacks(ws.data_ptr(), ws.numel(), B, P, C, 0, ctypes.addressof(nfb), st), "ssdhead_detect_fallbacks")
@@ -765,11 +805,14 @@ def run_ours(args):
     sampler = ClockSampler(local)
     sampler.start()
     B = args.batch
+    capture = bool(args.dump_outputs) and rank == 0
     if args.workload == "detect":
-        r = time_detect(args, rank, world, dev, sampler, B, args.steps, args.warmup)
+        r = time_detect(args, rank, world, dev, sampler, B, args.steps, args.warmup, capture=capture)
     else:
-        r = time_loss(args, rank, world, dev, sampler, args.workload, B, args.steps, args.warmup)
+        r = time_loss(args, rank, world, dev, sampler, args.workload, B, args.steps, args.warmup, capture=capture)
         args.collective = r["collective"] if world > 1 else args.collective       # what actually ran
+    if capture:
+        dump_outputs(args.dump_outputs, r.pop("outputs"))
     clocks = sampler.stop()
     ms_step = r["ms_total"] / args.steps
     value = B * world / (ms_step * 1e-3)
@@ -969,7 +1012,8 @@ def others(args, rank, dev, local, peak):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 2000 train / detect, 200 stress, 5 for --impl reference)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="train", choices=["train", "detect", "stress"])
@@ -979,11 +1023,18 @@ def main():
                     help="N > 1: how Npos and the loss sums cross GPUs - 'peer' = stores into peer memory over NVLink "
                          "from inside the mining kernel (2 kernels/step, no NCCL call), 'nccl' = two NCCL all-reduces "
                          "around the mining kernel (3 kernels/step)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32 / "
+                         "float64, at most 64 MB; rank 0 only) so that two builds can be compared output for output")
     args = ap.parse_args()
     if args.batch is None:
         args.batch = WORKLOADS[args.workload][1]
-    if args.workload == "stress" and args.steps == 2000:
-        args.steps = 200
+    if args.steps is None:
+        args.steps = 5 if args.impl == "reference" else (200 if args.workload == "stress" else 2000)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

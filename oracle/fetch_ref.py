@@ -1,13 +1,13 @@
 """Copy recipe for the UNMODIFIED reference sources (test infrastructure only).
 
 The reference is pure Python: there is nothing to compile into ``oracle/_ref``.  What this recipe does instead is copy
-the reference's seven ``*.py`` files, byte for byte, from ``/root/reference`` (or ``$SSD_REFERENCE_DIR``) into
-``oracle/_ref/`` - a directory that is git-ignored (no reference source enters the history) but travels to the GPU box
-with the working tree.  There the parity tests import the unmodified ``Losses.py`` / ``Util.py`` / ``train_function.py``
-from it (``oracle/ref_import.py``), and ``bench.py --impl reference`` times the reference's own ``ssd()`` on the host
-cores (``cpu_baseline.kind = "reference"``).  Nothing in the product package reads this directory.
+the reference's seven ``*.py`` files, byte for byte, from a checkout of the reference (the argument, else
+``$SSD_REFERENCE_SRC``, else ``/root/reference`` where the original project is mounted) into ``oracle/_ref/`` - a directory that is git-ignored (no reference source enters the history).
+The parity tests import the unmodified ``Losses.py`` / ``Util.py`` / ``train_function.py`` from it
+(``oracle/ref_import.py``), and ``bench.py --impl reference`` times the reference's own ``ssd()`` on the host cores
+(``cpu_baseline.kind = "reference"``).  Nothing in the product package reads this directory.
 
-    python oracle/fetch_ref.py          # idempotent; prints what it did
+    python oracle/fetch_ref.py <reference checkout>          # idempotent; prints what it did
 """
 from __future__ import annotations
 
@@ -42,4 +42,4 @@ def fetch(src: str | None = None, quiet: bool = False) -> bool:
 
 
 if __name__ == "__main__":
-    sys.exit(0 if fetch() else 1)
+    sys.exit(0 if fetch(sys.argv[1] if len(sys.argv) > 1 else None) else 1)

@@ -1,8 +1,12 @@
-"""Import the UNMODIFIED reference (``/root/reference``) for fixture generation.
+"""Import the UNMODIFIED reference for fixture generation.
 
-TEST INFRASTRUCTURE ONLY.  This module is used by ``tests/golden/make_golden.py``
-and by the CPU-side pinning tests (which skip when ``/root/reference`` is
-absent, as it is on the GPU box).  Nothing in the product package imports it.
+TEST INFRASTRUCTURE ONLY.  The reference sources are not part of this repository:
+they are read from ``$SSD_REFERENCE_DIR``, else from ``/root/reference`` where the
+original project is mounted, else from the copy ``oracle/fetch_ref.py`` makes in
+``oracle/_ref``.  This module is used by the fixture generators under ``tests/golden``
+and by the pinning tests against the live reference (which skip where the sources
+are absent; the frozen fixtures are checked everywhere).  Nothing in the product
+package imports it.
 
 The reference cannot be imported as-is in this image: ``Util.py:7,11`` import
 matplotlib (not installed) and ``Util.py:14-16`` parse the VOC annotation set
@@ -24,11 +28,12 @@ import warnings
 _HERE = os.path.dirname(os.path.abspath(__file__))
 
 
+MOUNT = "/root/reference"      # where a checkout of the original project is mounted read-only, when it is
+
+
 def _default_dir() -> str:
-    # /root/reference exists in the build container only; on the GPU box the byte-for-byte copy made by
-    # oracle/fetch_ref.py (git-ignored oracle/_ref/) is used
-    if os.path.isfile("/root/reference/Losses.py"):
-        return "/root/reference"
+    if os.path.isfile(os.path.join(MOUNT, "Losses.py")):
+        return MOUNT
     return os.path.join(_HERE, "_ref")
 
 

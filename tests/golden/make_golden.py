@@ -1,6 +1,6 @@
-"""Generate tests/golden/ssd_golden.npz by running the UNMODIFIED reference (/root/reference, imported with
-the stubs of oracle/ref_import.py) on seeded synthetic inputs.  Run in the container where the reference is
-mounted:  python tests/golden/make_golden.py
+"""Generate tests/golden/ssd_golden.npz by running the UNMODIFIED reference (imported with the stubs of
+oracle/ref_import.py) on seeded synthetic inputs.  Needs the reference sources:
+SSD_REFERENCE_DIR=<reference checkout> python tests/golden/make_golden.py
 
 What is frozen (all from the reference's own functions, nothing from the oracle or the kernels):
   priors          sha256 of the 8732x4 table + its corner form

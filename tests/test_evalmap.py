@@ -1,11 +1,16 @@
 """get_map (VOC 11-point AP, Util.py:783-885): oracle pinned against the live reference on the CPU; the GPU kernel
 against the oracle (exact: integer TP/FP decisions from bit-exact IoU, fp64 precision/recall)."""
+import os
+
 import numpy as np
 import pytest
 import torch
 
 from oracle import ref_import
 from oracle import ssd_oracle as O
+
+
+MAP_CASES = [(5, 6), (6, 25)]         # (seed, images) of the get_map comparisons with the reference
 
 
 def synth_eval(seed, images, classes=4, ties=False):
@@ -29,8 +34,8 @@ def synth_eval(seed, images, classes=4, ties=False):
     return dbx, dcl, dsc, gtb, gtc
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference sources not mounted (GPU box)")
-@pytest.mark.parametrize("seed,images", [(5, 6), (6, 25)])
+@pytest.mark.skipif(not ref_import.available(), reason="unmodified reference sources not available (SSD_REFERENCE_DIR)")
+@pytest.mark.parametrize("seed,images", MAP_CASES)
 def test_oracle_voc_ap_equals_reference_get_map(seed, images):
     RU, _ = ref_import.load()
     dbx, dcl, dsc, gtb, gtc = synth_eval(seed, images)
@@ -39,6 +44,21 @@ def test_oracle_voc_ap_equals_reference_get_map(seed, images):
     mine = O.voc_ap(dbx, dcl, dsc, gtb, gtc)
     assert all(float(ref[c]) == mine[c] for c in range(20))
     assert mine[:4].max() > 0.1 and (mine[4:] == 0).all()      # classes without detections score 0
+    # the frozen values (tests/golden/parity_golden.npz) are the reference's
+    assert np.array_equal(_frozen_ap(seed, images), [float(ref[c]) for c in range(20)])
+
+
+def _frozen_ap(seed, images):
+    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "parity_golden.npz"))
+    return g["map_ap"][MAP_CASES.index((seed, images))]
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("seed,images", MAP_CASES)
+def test_gpu_get_map_equals_frozen_reference_get_map(seed, images):
+    from objectdetection_ssd_b200 import Util
+    got = Util.get_map(*synth_eval(seed, images))
+    assert np.array_equal(np.array([got[c] for c in range(20)]), _frozen_ap(seed, images))
 
 
 @pytest.mark.gpu

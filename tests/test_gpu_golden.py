@@ -1,5 +1,5 @@
 """GPU: the CUDA kernels against the FROZEN outputs of the unmodified reference (tests/golden/ssd_golden.npz, made by
-tests/golden/make_golden.py from /root/reference) - directly, without the oracle in between, so that a regression of the
+tests/golden/make_golden.py from the reference sources) - directly, without the oracle in between, so that a regression of the
 oracle cannot hide one of the kernels.  Integer / boolean results (class map, object map, positive counts, rows that
 carry a gradient) are compared exactly; losses, gradient checksums, probabilities and boxes to 1e-5 relative (fp32)."""
 import os

@@ -1,4 +1,8 @@
-"""CPU, only where /root/reference is mounted: the oracle against the live, unmodified reference."""
+"""CPU, only where the reference sources are available (oracle/ref_import.py): the oracle against the live, unmodified
+reference."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
@@ -6,7 +10,7 @@ from objectdetection_ssd_b200 import synth
 from oracle import ref_import
 from oracle import ssd_oracle as O
 
-pytestmark = pytest.mark.skipif(not ref_import.available(), reason="reference sources not mounted (GPU box)")
+pytestmark = pytest.mark.skipif(not ref_import.available(), reason="unmodified reference sources not available (SSD_REFERENCE_DIR)")
 
 
 def test_loss_grads_and_maps_bit_identical():
@@ -74,3 +78,16 @@ def test_detect_bit_identical():
     with ref_import.quiet():
         assert RL.inference(torch.from_numpy(dl[0]), z, 0, toDraw=False) == ([], [], [])
     assert O.detect_image(torch.from_numpy(dl[0]), z, pri)[0].shape[0] == 0
+
+
+def test_frozen_fixture_holds_the_reference_values():
+    """tests/golden/parity_golden.npz (what tests/test_parity_golden.py compares with) against the live reference."""
+    from tests.golden.make_parity_golden import frozen_values
+    G = np.load(os.path.join(os.path.dirname(__file__), "golden", "parity_golden.npz"), allow_pickle=False)
+    want = frozen_values(live=True)
+    assert set(want) <= set(G.files)
+    for k, v in want.items():
+        if k == "loss_old" or k.startswith("sgd_"):     # ssd_per_image_mean is pinned to 1e-6 / 1e-5, the loop to fp32
+            assert np.allclose(G[k], v, rtol=1e-5, atol=1e-6), k
+        else:
+            assert np.array_equal(G[k], v), k
