@@ -1607,7 +1607,8 @@ static int run_detect(const float* loc, const float* conf, const float* pri_cxcy
     const int T = dl ? dl->tile0[dl->n] : detect_tiles(P);
     if (T > NT) return SSDHEAD_E_UNSUPPORTED;                                 // P <= 131072
     const size_t smem_nms = nms_smem_bytes(NF, top_k, T);
-    if (smem_nms > 200 * 1024) return SSDHEAD_E_UNSUPPORTED;                 // top_k <= ~1400 for 20 classes
+    if (smem_nms > 200 * 1024) return SSDHEAD_E_UNSUPPORTED;                 // 20 classes: top_k <= 1729 at SSD300 (T = 35),
+                                                                              // <= 1589 at T = 512
     DetectWs w;
     const size_t need = detect_ws_layout(B, P, C, n_cap, &w, ws);
     if (ws_bytes < need) return SSDHEAD_E_WORKSPACE;
