@@ -374,8 +374,8 @@ void ssdhead_ctx_destroy(ssdhead_ctx* ctx);
 void* ssdhead_host_alloc(size_t bytes);
 void  ssdhead_host_free(void* p);
 
-/* One training-head step on DEVICE tensors in a single call: ssdhead_match on the context's auxiliary
- * stream beside ssdhead_ce_stream on `stream`, joined before ssdhead_mine.  Asynchronous on `stream`;
+/* One training-head step on DEVICE tensors in a single call: ssdhead_multibox_step, or ssdhead_multibox_step_sharded
+ * after ssdhead_ctx_xchg_import - two kernels on `stream`.  Asynchronous on `stream`;
  * sums double[2], losses float[2], grads nullable as a pair (all device pointers). */
 int ssdhead_ctx_multibox_loss_dev(ssdhead_ctx* ctx, const float* loc_dev, const float* conf_dev,
                                   const float* gt_xyxy_dev, const float* gt_cls_dev, const int32_t* gt_off_dev,
@@ -424,7 +424,7 @@ int ssdhead_ctx_xchg_error(ssdhead_ctx* ctx);
  * Copies, kernels and copies back are pipelined in image chunks on the context's streams; pass
  * page-locked buffers (ssdhead_host_alloc) so the copies are asynchronous - a page-locked `loc` is not copied at
  * all (the kernels read the few rows they need in place), and page-locked gradient buffers are zeroed by host threads
- * and receive only their non-zero rows from the GPU (environment SSDHEAD_E2E_SPARSE=0 restores the dense copy back).
+ * and receive only their non-zero rows from the GPU.
  * Blocks until done. */
 int ssdhead_ctx_multibox_loss_host(ssdhead_ctx* ctx, const float* loc_host, const float* conf_host,
                                    const float* gt_xyxy_host, const float* gt_cls_host, const int32_t* gt_off_host,

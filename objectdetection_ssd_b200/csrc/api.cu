@@ -36,7 +36,7 @@ size_t ssdhead_workspace_bytes(int which, int B, int P, int C, int n)
     if (B < 0 || P < 0 || C < 0 || n < 0) return 0;
     switch (which) {
         case SSDHEAD_WS_MATCH:
-            return round_up((size_t)n * 8, 16) + 2 * round_up((size_t)B * 4, 16) + 16;
+            return match_ws_bytes(B, n);
         case SSDHEAD_WS_LOSS:
             return loss_workspace_bytes(B, P, C);
         case SSDHEAD_WS_DETECT:

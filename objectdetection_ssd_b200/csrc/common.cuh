@@ -185,22 +185,47 @@ __device__ __forceinline__ int ld_cg_s32(const int* p) {
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
-template <typename... KArgs, typename... Args>
-static inline cudaError_t launch_pdl(int which, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args)
+// COOP: also a cooperative launch (every CTA co-resident).
+template <bool COOP = false, typename... KArgs, typename... Args>
+static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args)
 {
-    static const int mask = getenv("SSDHEAD_PDL") ? atoi(getenv("SSDHEAD_PDL")) : 253;  // 1 CE stream, 2 finaliser, 4 mine; detect: 8 / 32 exhaustive score / sweep, 16 fused short-list kernel, 64 / 128 fallback score / sweep, 256 sampling kernel (off: 40 us slower at batch 256); measured: CE + mine best, chaining the finaliser (2) is slower
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = block;
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
-    cudaLaunchAttribute attr[1];
+    cudaLaunchAttribute attr[2];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = (mask & which) ? 1 : 0;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    attr[1].id = cudaLaunchAttributeCooperative;
+    attr[1].val.cooperative = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = 1;
+    cfg.numAttrs = COOP ? 2 : 1;
     return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
+
+// Workspace of the match (ssdhead_match, and the match fused into the loss steps), zero on entry and on exit:
+// best_key u64[sumG] | tile_counter u32[B] | npos_acc i32[B] | image_counter u32, and in the same 16-byte tail the
+// u64 arrive_total of the mining kernel's fused finaliser.
+struct MatchWs {
+    unsigned long long* best_key;
+    unsigned int* tile_counter;
+    int* npos_acc;
+    unsigned int* image_counter;
+    unsigned long long* arrive_total;
+};
+static inline MatchWs match_ws(void* ws, int B, int sumG)
+{
+    uintptr_t w = (uintptr_t)ws;
+    MatchWs m;
+    m.best_key = (unsigned long long*)w;          w += round_up((size_t)sumG * 8, 16);
+    m.tile_counter = (unsigned int*)w;            w += round_up((size_t)B * 4, 16);
+    m.npos_acc = (int*)w;                         w += round_up((size_t)B * 4, 16);
+    m.image_counter = (unsigned int*)w;
+    m.arrive_total = (unsigned long long*)(w + 8);
+    return m;
+}
+static inline size_t match_ws_bytes(int B, int sumG) { return (uintptr_t)match_ws(nullptr, B, sumG).image_counter + 16; }
 
 // system-scope accesses for the cross-GPU exchange over NVLink peer memory (sharded batches)
 __device__ __forceinline__ void st_release_sys_u64(unsigned long long* p, unsigned long long v) {

@@ -1633,8 +1633,9 @@ static int run_detect(const float* loc, const float* conf, const float* pri_cxcy
             SSD_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ks, (SCW + 1) * 32, smem_stream));
             if (per_sm < 1) return SSDHEAD_E_UNSUPPORTED;
             const int grid = (int)std::min<long long>((long long)B * ipi_a, (long long)per_sm * sm_count());
-            SSD_CHECK_CUDA(launch_pdl(256, ks, dim3(grid), dim3((SCW + 1) * 32), smem_stream, st, fl, B, P, ipi_a, *dl, w.cand, capI, T));
-            SSD_CHECK_CUDA(launch_pdl(32, kw, dim3(B), dim3(NT), smem_sweep, st, fl, ipi_a, ipi_b, *dl, (const float4*)pri_cxcywh,
+            ks<<<grid, (SCW + 1) * 32, smem_stream, st>>>(fl, B, P, ipi_a, *dl, w.cand, capI, T);
+            SSD_LAUNCH_CHECK();
+            SSD_CHECK_CUDA(launch_pdl(kw, dim3(B), dim3(NT), smem_sweep, st, fl, ipi_a, ipi_b, *dl, (const float4*)pri_cxcywh,
                                       w.cand, w.scr_a, w.scr_b, img_wh, P, NF, T, capI, top_k, iou_thr,
                                       (float4*)out_boxes, out_prob, out_cls, out_prior, out_cnt));
         } else {
@@ -1645,8 +1646,9 @@ static int run_detect(const float* loc, const float* conf, const float* pri_cxcy
             SSD_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ks, (SCW + 1) * 32, smem_stream));
             if (per_sm < 1) return SSDHEAD_E_UNSUPPORTED;
             const int grid = (int)std::min<long long>((long long)B * ipi_a, (long long)per_sm * sm_count());
-            SSD_CHECK_CUDA(launch_pdl(256, ks, dim3(grid), dim3((SCW + 1) * 32), smem_stream, st, fl, conf, B, P, ipi_a, w.cand, capI, T));
-            SSD_CHECK_CUDA(launch_pdl(32, kw, dim3(B), dim3(NT), smem_sweep, st, fl, conf, ipi_a, ipi_b, (const float4*)loc, (const float4*)pri_cxcywh,
+            ks<<<grid, (SCW + 1) * 32, smem_stream, st>>>(fl, conf, B, P, ipi_a, w.cand, capI, T);
+            SSD_LAUNCH_CHECK();
+            SSD_CHECK_CUDA(launch_pdl(kw, dim3(B), dim3(NT), smem_sweep, st, fl, conf, ipi_a, ipi_b, (const float4*)loc, (const float4*)pri_cxcywh,
                                       w.cand, w.scr_a, w.scr_b, img_wh, P, NF, T, capI, top_k, iou_thr,
                                       (float4*)out_boxes, out_prob, out_cls, out_prior, out_cnt));
         }
@@ -1658,17 +1660,17 @@ static int run_detect(const float* loc, const float* conf, const float* pri_cxcy
     const dim3 g1(T, B);
     if (dl) {
         SSD_CHECK_CUDA(cudaFuncSetAttribute(detect_nms_levels_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_nms));
-        SSD_CHECK_CUDA(launch_pdl(8, detect_score_levels_kernel<21>, g1, dim3(SC_T), 0, st,
+        SSD_CHECK_CUDA(launch_pdl(detect_score_levels_kernel<21>, g1, dim3(SC_T), 0, st,
                                   P, min_score, capI, w.cand, w.cand_cnt, w.dir, w.dir_base, w.overflow, w.flag_cnt, *dl));
-        SSD_CHECK_CUDA(launch_pdl(8, detect_nms_levels_kernel, dim3(B), dim3(NT), smem_nms, st,
+        SSD_CHECK_CUDA(launch_pdl(detect_nms_levels_kernel, dim3(B), dim3(NT), smem_nms, st,
                                   *dl, (const float4*)pri_cxcywh, w.cand, w.scr_a, w.scr_b, (const unsigned short*)w.dir,
                                   (const unsigned int*)w.dir_base, w.cand_cnt, w.overflow, img_wh, P, NF, T, capI, top_k, iou_thr,
                                   (float4*)out_boxes, out_prob, out_cls, out_prior, out_cnt));
     } else {
         SSD_CHECK_CUDA(cudaFuncSetAttribute(detect_nms_kernel<FROM_SCORES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_nms));
-        SSD_CHECK_CUDA(launch_pdl(8, detect_score_kernel<21, FROM_SCORES>, g1, dim3(SC_T), 0, st,
+        SSD_CHECK_CUDA(launch_pdl(detect_score_kernel<21, FROM_SCORES>, g1, dim3(SC_T), 0, st,
                                   conf, P, min_score, capI, w.cand, w.cand_cnt, w.dir, w.dir_base, w.overflow, w.flag_cnt));
-        SSD_CHECK_CUDA(launch_pdl(8, detect_nms_kernel<FROM_SCORES>, dim3(B), dim3(NT), smem_nms, st,
+        SSD_CHECK_CUDA(launch_pdl(detect_nms_kernel<FROM_SCORES>, dim3(B), dim3(NT), smem_nms, st,
                                   (const float4*)loc, (const float4*)pri_cxcywh, w.cand, w.scr_a, w.scr_b, (const unsigned short*)w.dir,
                                   (const unsigned int*)w.dir_base, w.cand_cnt, w.overflow, img_wh, P, NF, T, capI, top_k, iou_thr,
                                   (float4*)out_boxes, out_prob, out_cls, out_prior, out_cnt));

@@ -19,6 +19,8 @@
 using namespace ssdhead;
 
 namespace ssdhead {
+size_t loss_ws_header_bytes(int maxB);     // loss.cu
+
 // Util.py:93-96 on the host for the one-off prior table (same fp32 operations as the device helper)
 static void priors_xyxy_host(const float* cxcywh, float* xyxy, int P)
 {
@@ -232,7 +234,7 @@ static const float* mapped_host_alias(const float* host)
 static int ctx_loss_ws_for(ssdhead_ctx* c, int B, cudaStream_t st)
 {
     if (c->last_loss_B == B) return 0;
-    const size_t head = 16 + (size_t)c->maxB * 16 + 256;
+    const size_t head = loss_ws_header_bytes(c->maxB);
     for (size_t off = 0; off + head <= c->ws_loss_total; off += c->ws_loss_bytes)
         SSD_CHECK_CUDA(cudaMemsetAsync((char*)c->ws_loss + off, 0, std::min(head, c->ws_loss_bytes), st));
     c->last_loss_B = B;
@@ -424,8 +426,7 @@ int ssdhead_ctx_multibox_loss_end(ssdhead_ctx* c, const float* loc, const float*
                         c->ws_loss, c->ws_loss_bytes, (cudaStream_t)stream);
 }
 
-// One training-head step on DEVICE tensors: the match runs on the context's auxiliary stream beside the CE
-// streaming kernel (which does not depend on it); both join before the mining kernel.  Asynchronous on `stream`.
+// One training-head step on DEVICE tensors: ssdhead_multibox_step, or the sharded step - two kernels on `stream`.
 int ssdhead_ctx_multibox_loss_dev(ssdhead_ctx* c, const float* loc, const float* conf,
                                   const float* gt_xyxy, const float* gt_cls, const int32_t* gt_off, int B, int sumG,
                                   int neg_ratio, float pos_iou,
@@ -588,9 +589,8 @@ static int loss_host_impl(ssdhead_ctx* c, const float* loc_h, const float* conf_
     // page-locked, the dense zero background never crosses PCIe.  Host threads zero the buffers chunk by chunk while the
     // inputs stream in, the streaming kernel runs without its zero-fill, and the mining kernel stores its few hundred
     // rows per image straight into the host buffers through their UVA aliases.  Same bits in the caller's buffers.
-    static const int sparse_ok = getenv("SSDHEAD_E2E_SPARSE") ? atoi(getenv("SSDHEAD_E2E_SPARSE")) : 1;
-    float* gl_alias = (grads && sparse_ok) ? const_cast<float*>(mapped_host_alias(grad_loc_h)) : nullptr;
-    float* gc_alias = (grads && sparse_ok) ? const_cast<float*>(mapped_host_alias(grad_conf_h)) : nullptr;
+    float* gl_alias = grads ? const_cast<float*>(mapped_host_alias(grad_loc_h)) : nullptr;
+    float* gc_alias = grads ? const_cast<float*>(mapped_host_alias(grad_conf_h)) : nullptr;
     const bool sparse = gl_alias && gc_alias;
     int T = 0;
     if (sparse) {

@@ -39,6 +39,8 @@
 // HBM traffic per image: conf in once (733 KB) + CE out/in (2 x 35 KB, L2-resident between the two
 // kernels) + dense gradients out once (873 KB) + ~4*npos sparse rows: the algorithmic minimum.
 #include <algorithm>
+#include <tuple>
+#include <type_traits>
 #include "common.cuh"
 
 namespace ssdhead {
@@ -1387,14 +1389,35 @@ scale_grads_kernel(float4* __restrict__ gl, size_t n4_loc, float* __restrict__ g
 
 static size_t mine_smem_bytes(int P) { return (size_t)P * 4 + MN_BINS * 4 + (size_t)((P + 7) & ~7) * 2 + round_up((size_t)P, 16); }
 
-// workspace: [0,16) done counter | partials double[2B] | CE float[B*P] (when the caller passes no ce buffer)
+// Loss workspace (16-byte aligned): done counter [0,16) | partials double[2B] | CE float[B*P] (when the caller passes no
+// ce buffer) | best-gt map u16[B*P] of the steps | seeds float[SEED_CAP] of the fused match's cull.  The counter and the
+// partials are kept zero between calls.
+struct LossWs {
+    unsigned int* done_counter;
+    double* partials;
+    float* ce;
+    unsigned short* obj;
+    float* seed;
+};
+static LossWs loss_ws(void* ws, int B, int P)
+{
+    uintptr_t w = (uintptr_t)ws;
+    LossWs l;
+    l.done_counter = (unsigned int*)w;            w += 16;
+    l.partials = (double*)w;                      w += round_up((size_t)B * 2 * sizeof(double), 16);
+    l.ce = (float*)w;                             w += round_up((size_t)B * P * sizeof(float), 16);
+    l.obj = (unsigned short*)w;                   w += round_up((size_t)B * P * sizeof(unsigned short), 16);
+    l.seed = (float*)w;
+    return l;
+}
 size_t loss_workspace_bytes(int B, int P, int C)
 {
     if (mine_smem_bytes(P) > 220 * 1024 || P >= 65536) return 0;   // P <= ~31 000 priors
-    return 16 + round_up((size_t)B * 2 * sizeof(double), 16) + round_up((size_t)B * P * sizeof(float), 16) +
-           round_up((size_t)B * P * sizeof(unsigned short), 16) +     // CE, then the best-gt map of large-G batches,
-           (size_t)SEED_CAP * sizeof(float);                           // then the seeds of the fused match's cull
+    return (uintptr_t)loss_ws(nullptr, B, P).seed + (size_t)SEED_CAP * sizeof(float);
 }
+// Bytes from the start of a loss workspace that hold the done counter and the partials of any batch of up to maxB
+// images, plus 256 bytes that no field needs (they reach into the CE rows, which every call rewrites).
+size_t loss_ws_header_bytes(int maxB) { return (uintptr_t)loss_ws(nullptr, maxB, 0).ce + 256; }
 
 // rows workspace of the resident-gradient step: one record per image, the same for every batch size - int32 rows,
 // int32 positives, uint16 [P] row indices (P < 65536)
@@ -1416,16 +1439,14 @@ static int num_sms()
     return g_num_sms;
 }
 
+// The streaming CE kernel over [B*P] rows (lv == nullptr) or over the per-level tensors of lv
 template <int C, bool GRADS, bool MATCH>
 static int launch_ce_stream(const float* conf, float* ce, float* grad_conf, float* grad_loc, long long rows,
-                            const FusedMatch& fm, cudaStream_t st)
+                            const FusedMatch& fm, const LevelTab* lv, cudaStream_t st)
 {
     constexpr size_t tile = (size_t)CE_ROWS * C * 4;
     const size_t smem_ce = tile * CE_STAGES + (GRADS ? (size_t)CE_ZERO_ROWS * C * 4 : 0);
-    auto kce = ce_stream_kernel<C, GRADS, MATCH>;
-    SSD_CHECK_CUDA(cudaFuncSetAttribute(kce, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ce));
-    const int use_tma = (aligned16(conf) && (!GRADS || (aligned16(grad_conf) && aligned16(grad_loc)))) ? 1 : 0;
-    const long long tiles = (rows + CE_ROWS - 1) / CE_ROWS;
+    const long long tiles = (rows + CE_ROWS - 1) / CE_ROWS + (lv ? lv->n : 0);
     const int grid_ce = (int)std::min<long long>(tiles, (long long)CE_CTAS * num_sms());
     if (MATCH && fm.seed_lb) {
         const int stride = std::max(SEED_STRIDE, (fm.P + SEED_MAX - 1) / SEED_MAX);
@@ -1437,81 +1458,65 @@ static int launch_ce_stream(const float* conf, float* ce, float* grad_conf, floa
         SSD_LAUNCH_CHECK();
         count_launch();
     }
-    SSD_CHECK_CUDA(launch_pdl(1, kce, dim3(grid_ce), dim3(CE_THREADS), smem_ce, st, conf, ce, grad_conf, grad_loc, rows, use_tma, fm));
+    if (MATCH && lv) {
+        auto kce = ce_stream_levels_kernel<C, GRADS>;
+        SSD_CHECK_CUDA(cudaFuncSetAttribute(kce, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ce));
+        // stride ~ 0.618 T, coprime with T: consecutive visits land in different levels in proportion to their sizes
+        LevelTab lt = *lv;
+        const long long T = lt.tile0[lt.n];
+        auto gcd = [](long long a, long long b) { while (b) { const long long c = a % b; a = b; b = c; } return a; };
+        long long S = std::max<long long>(1, (long long)(0.6180339887 * (double)T));
+        while (S > 1 && gcd(S, T) != 1) --S;
+        lt.perm_stride = (int)S;
+        lt.perm_inc = T > 0 ? (int)(((long long)grid_ce * S) % T) : 0;
+        SSD_CHECK_CUDA(launch_pdl(kce, dim3(grid_ce), dim3(CE_THREADS), smem_ce, st, ce, rows, fm, lt));
+    } else {
+        auto kce = ce_stream_kernel<C, GRADS, MATCH>;
+        SSD_CHECK_CUDA(cudaFuncSetAttribute(kce, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ce));
+        const int use_tma = (aligned16(conf) && (!GRADS || (aligned16(grad_conf) && aligned16(grad_loc)))) ? 1 : 0;
+        SSD_CHECK_CUDA(launch_pdl(kce, dim3(grid_ce), dim3(CE_THREADS), smem_ce, st, conf, ce, grad_conf, grad_loc, rows, use_tma, fm));
+    }
     count_launch();
     return 0;
 }
 
-template <int C, bool GRADS>
-static int launch_mine(const MineParams& prm, cudaStream_t st)
+// A mining kernel on one CTA per image.  FIN: the forced-match finaliser is fused in, so every CTA must be co-resident
+// (they exchange the batch positive count through a counter) - a cooperative launch, which returns 1 (not an error)
+// when the grid does not fit.
+template <bool FIN, typename... KArgs, typename... Args>
+static int launch_mine(void (*kmn)(KArgs...), int B, int P, cudaStream_t st, Args... args)
 {
-    auto kmn = mine_kernel<C, GRADS, false>;
-    const size_t smem_mn = mine_smem_bytes(prm.P);
+    const size_t smem_mn = mine_smem_bytes(P);
     SSD_CHECK_CUDA(cudaFuncSetAttribute(kmn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_mn));
-    SSD_CHECK_CUDA(launch_pdl(4, kmn, dim3(prm.B), dim3(MN_T), smem_mn, st, prm));
-    count_launch();
-    return 0;
-}
-
-template <int C>
-static int launch_mine_sparse(const MineParams& prm, cudaStream_t st)
-{
-    auto kmn = mine_sparse_kernel<C>;
-    const size_t smem_mn = mine_smem_bytes(prm.P);
-    SSD_CHECK_CUDA(cudaFuncSetAttribute(kmn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_mn));
-    SSD_CHECK_CUDA(launch_pdl(4, kmn, dim3(prm.B), dim3(MN_T), smem_mn, st, prm));
-    count_launch();
-    return 0;
-}
-
-// mine_kernel with the forced-match finaliser fused in needs every CTA co-resident (they exchange the batch positive
-// count through a counter): cooperative launch; returns 1 (not an error) when the grid does not fit, so the caller
-// falls back to match_finalize_kernel + the ordinary mining kernel.
-template <int C, bool GRADS>
-static int launch_mine_fin(MineParams prm, cudaStream_t st)
-{
-    auto kmn = mine_kernel<C, GRADS, true>;
-    const size_t smem_mn = mine_smem_bytes(prm.P);
-    SSD_CHECK_CUDA(cudaFuncSetAttribute(kmn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_mn));
+    if (!FIN) {
+        SSD_CHECK_CUDA(launch_pdl(kmn, dim3(B), dim3(MN_T), smem_mn, st, args...));
+        count_launch();
+        return 0;
+    }
     int per_sm = 0;
     SSD_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kmn, MN_T, smem_mn));
-    if ((long long)per_sm * num_sms() < prm.B) return 1;
+    if ((long long)per_sm * num_sms() < B) return 1;
     // cooperative (co-residency guaranteed) AND programmatic stream serialization (the grid may become resident while
     // the streaming kernel drains; it waits in pdl_wait()).  Runtimes that refuse the combination get the plain
     // cooperative launch.
-    static int combo = getenv("SSDHEAD_COOP_PDL") ? atoi(getenv("SSDHEAD_COOP_PDL")) : 1;
-    if (combo) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(prm.B);
-        cfg.blockDim = dim3(MN_T);
-        cfg.dynamicSmemBytes = smem_mn;
-        cfg.stream = st;
-        cudaLaunchAttribute attr[2];
-        attr[0].id = cudaLaunchAttributeCooperative;
-        attr[0].val.cooperative = 1;
-        attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[1].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 2;
-        const cudaError_t e = cudaLaunchKernelEx(&cfg, kmn, prm);
-        if (e == cudaSuccess) { count_launch(); return 0; }
+    static bool with_pdl = true;
+    if (with_pdl) {
+        if (launch_pdl<true>(kmn, dim3(B), dim3(MN_T), smem_mn, st, args...) == cudaSuccess) { count_launch(); return 0; }
         (void)cudaGetLastError();
-        combo = 0;
+        with_pdl = false;
     }
-    void* args[] = {&prm};
-    SSD_CHECK_CUDA(cudaLaunchCooperativeKernel((const void*)kmn, dim3(prm.B), dim3(MN_T), args, smem_mn, st));
+    static_assert(std::is_same<std::tuple<std::decay_t<Args>...>, std::tuple<std::decay_t<KArgs>...>>::value,
+                  "the cooperative launch passes the arguments by address: they must have the kernel's parameter types");
+    void* ptrs[] = {(void*)&args...};
+    SSD_CHECK_CUDA(cudaLaunchCooperativeKernel((const void*)kmn, dim3(B), dim3(MN_T), ptrs, smem_mn, st));
     count_launch();
     return 0;
 }
 
-static float* ws_ce(void* ws, int B) { return (float*)((char*)ws + 16 + round_up((size_t)B * 2 * sizeof(double), 16)); }
-static float* ws_seed(void* ws, int B, int P) { return (float*)((char*)ws_ce(ws, B) + round_up((size_t)B * P * sizeof(float), 16) + round_up((size_t)B * P * sizeof(unsigned short), 16)); }
-static unsigned short* ws_obj(void* ws, int B, int P) { return (unsigned short*)((char*)ws_ce(ws, B) + round_up((size_t)B * P * sizeof(float), 16)); }
 // The walk over an image's gts in the mining kernel costs G x ~25 instructions per positive row, on the latency chain
 // of the step's last kernel; the streaming kernel can record the best gt of every prior instead (2 bytes per row, +1 %
 // of its traffic) and the walk disappears.  Measured at 1-10 gts per image: 112.4 -> 111.5 us per step at B=256 with the
-// map, 671 -> 565 us at 100 gts per image - so the map is used whenever a gt index fits its 16 bits
-// (SSDHEAD_OBJ_MAP_MIN=<average gts per image> restores a threshold for experiments).
+// map, 671 -> 565 us at 100 gts per image - so the steps use the map whenever a gt index fits its 16 bits.
 // The seeded cull of the fused match pays from a few dozen gts per image (the stress shape has 100); the ordinary
 // batches (<= 10 gts per image) keep the plain loop.  SSDHEAD_MATCH_CULL_MIN overrides the average gt count it starts at.
 static bool match_cull_enabled(int B, int sumG)
@@ -1521,10 +1526,216 @@ static bool match_cull_enabled(int B, int sumG)
     return B > 0 && sumG >= (long long)min_avg * B && sumG <= SEED_CAP;
 }
 
-static bool use_obj_map(int B, int sumG)
+// The arguments of the loss entry points, in the order they take them; an entry point leaves what it does not take null.
+struct StepArgs {
+    const float *loc, *conf, *gt_xyxy, *gt_cls;
+    const int32_t* gt_off;
+    const float *pri_xyxy, *pri_cxcywh;
+    int B, P, C, sumG, neg_ratio;
+    float pos_iou;
+    double* sums;
+    float *losses, *grad_loc, *grad_conf;
+    uint8_t* cls_u8;
+    int32_t *best_prior, *npos;
+    uint32_t* mined_mask;
+    float* ce;
+    void* ws_loss; size_t ws_loss_bytes;
+    void* ws_match; size_t ws_match_bytes;
+    void* stream;
+};
+
+// The peer exchange of a batch sharded by image over R GPUs
+struct Xchg { int R, rank; unsigned seq; void* const* peers; void* local; int32_t* err_flag; };
+
+static int check_xchg(const Xchg& x, bool seq_required)
 {
-    static const int min_avg = getenv("SSDHEAD_OBJ_MAP_MIN") ? atoi(getenv("SSDHEAD_OBJ_MAP_MIN")) : 0;
-    return sumG >= min_avg * B && sumG <= 65535;
+    if (x.R < 1 || x.R > XCHG_MAX_R || x.rank < 0 || x.rank >= x.R || (seq_required && x.seq == 0u)) return SSDHEAD_E_BADARG;
+    if (x.R > 1 && (!x.peers || !x.local || !x.err_flag)) return SSDHEAD_E_BADARG;
+    return 0;
+}
+
+// What the mining kernel reads beyond the match; `flat`: the head tensors loc and conf (the per-level steps take a table).
+// Their alignment is checked by the caller, where a batch of B = 0 has always been checked for it or not.
+static int check_mine(const StepArgs& a, bool flat)
+{
+    if ((flat && (!a.loc || !a.conf)) || !a.pri_cxcywh || !a.sums || !a.losses || a.neg_ratio < 0) return SSDHEAD_E_BADARG;
+    return 0;
+}
+
+// What every loss entry point needs: the sizes, the class count, the gradient pair and the loss workspace.  A batch of
+// B = 0 passes before the alignment and workspace checks: it has nothing to do.
+static int check_loss(int B, int P, int C, const float* grad_loc, const float* grad_conf, const void* ws, size_t ws_bytes)
+{
+    if (B < 0 || P <= 0 || !ws || (grad_loc == nullptr) != (grad_conf == nullptr)) return SSDHEAD_E_BADARG;
+    if (C != 21) return SSDHEAD_E_UNSUPPORTED;          // VOC head of the reference (Losses.py:184 hard-codes 21)
+    if (B == 0) return 0;
+    if ((grad_loc && !aligned16(grad_loc)) || !aligned16(ws)) return SSDHEAD_E_ALIGN;
+    const size_t need = loss_workspace_bytes(B, P, C);
+    if (need == 0) return SSDHEAD_E_UNSUPPORTED;
+    return ws_bytes < need ? SSDHEAD_E_WORKSPACE : 0;
+}
+
+// ... and what the fused match needs (every step)
+static int check_match(const StepArgs& a)
+{
+    if (a.sumG < 0 || !a.gt_off || !a.pri_xyxy || !a.cls_u8 || !a.npos || !a.ws_match) return SSDHEAD_E_BADARG;
+    if (a.sumG > 0 && (!a.gt_xyxy || !a.gt_cls || !a.best_prior)) return SSDHEAD_E_BADARG;
+    const int rc = check_loss(a.B, a.P, a.C, a.grad_loc, a.grad_conf, a.ws_loss, a.ws_loss_bytes);
+    if (rc || a.B == 0) return rc;
+    if ((long long)a.B * a.P >= (1ll << 31)) return SSDHEAD_E_UNSUPPORTED;
+    if (!aligned16(a.ws_match) || !aligned16(a.pri_xyxy) || (a.sumG > 0 && !aligned16(a.gt_xyxy))) return SSDHEAD_E_ALIGN;
+    return a.ws_match_bytes < match_ws_bytes(a.B, a.sumG) ? SSDHEAD_E_WORKSPACE : 0;
+}
+
+static int check_resident(const StepArgs& a, const void* ws_rows, size_t ws_rows_bytes)
+{
+    if (!ws_rows || !a.grad_loc || !a.grad_conf || a.B < 0 || a.P <= 0 || a.P >= 65536) return SSDHEAD_E_BADARG;
+    if (!aligned16(ws_rows) || !aligned16(a.grad_loc)) return SSDHEAD_E_ALIGN;
+    if (ws_rows_bytes < resident_rows_bytes(a.B, a.P)) return SSDHEAD_E_WORKSPACE;
+    return 0;
+}
+
+// The level table as the kernels index it: the levels partition the P priors, all or none of them carry gradients.
+// With B = 0 only the table's size is checked: an empty batch may pass levels without tensors.
+static int check_levels(const ssdhead_levels* levels, int B, int P, LevelTab* lv)
+{
+    if (!levels || levels->num_levels < 1 || levels->num_levels > MAX_LEVELS) return SSDHEAD_E_BADARG;
+    if (B == 0) return 0;
+    lv->n = levels->num_levels;
+    int sum = 0, with_grads = 0;
+    int t0 = 0;
+    for (int l = 0; l < lv->n; ++l) {
+        const int n = levels->count[l];
+        if (n <= 0 || !levels->conf[l] || !levels->loc[l]) return SSDHEAD_E_BADARG;
+        if (!aligned16(levels->loc[l])) return SSDHEAD_E_ALIGN;                        // float4 rows
+        const bool g = levels->grad_conf[l] != nullptr;
+        if (g != (levels->grad_loc[l] != nullptr)) return SSDHEAD_E_BADARG;
+        if (g && !aligned16(levels->grad_loc[l])) return SSDHEAD_E_ALIGN;
+        // conf / grad_conf rows are 84 bytes: a level whose pointers are not 16-byte aligned (e.g. a view into a larger
+        // tensor) cannot ride the TMA pipeline and goes through the plain-load path entirely
+        const bool tma_ok = aligned16(levels->conf[l]) && (!g || aligned16(levels->grad_conf[l]));
+        with_grads += g ? 1 : 0;
+        lv->cnt[l] = n; lv->start[l] = sum; lv->tile0[l] = t0;
+        lv->conf[l] = levels->conf[l]; lv->loc[l] = levels->loc[l]; lv->gconf[l] = levels->grad_conf[l]; lv->gloc[l] = levels->grad_loc[l];
+        sum += n;
+        const long long rows_l = (long long)B * n;
+        lv->rows[l] = (int)rows_l;
+        // the partial last tile of a level rides the TMA pipeline too when its byte counts are multiples of 16
+        if (tma_ok) t0 += (int)(rows_l / CE_ROWS) + ((rows_l % CE_ROWS) != 0 && (rows_l % 4) == 0 ? 1 : 0);
+    }
+    for (int l = lv->n; l <= MAX_LEVELS; ++l) { lv->start[l] = sum; lv->tile0[l] = t0; }
+    if (sum != P) return SSDHEAD_E_BADARG;
+    if (with_grads != 0 && with_grads != lv->n) return SSDHEAD_E_BADARG;
+    return 0;
+}
+
+// The natural match that rides in the streaming kernel
+static FusedMatch bind_match(const StepArgs& a, const MatchWs& mw, unsigned short* obj_u16, const float* seed_lb)
+{
+    FusedMatch fm = {};
+    fm.gt_xyxy = (const float4*)a.gt_xyxy; fm.gt_cls = a.gt_cls; fm.gt_off = a.gt_off; fm.pri_xyxy = (const float4*)a.pri_xyxy;
+    fm.P = a.P; fm.bg_class = a.C - 1; fm.pos_iou = a.pos_iou; fm.cls_u8 = a.cls_u8; fm.best_key = mw.best_key; fm.npos_acc = mw.npos_acc;
+    fm.obj_u16 = obj_u16; fm.sumG = a.sumG; fm.seed_lb = seed_lb;
+    return fm;
+}
+
+// The mining kernel's parameters; `mw` (the steps): the forced-match finaliser fused in, writing the match outputs
+static MineParams bind_mine(const StepArgs& a, const LossWs& lw, const int32_t* npos_norm, const MatchWs* mw)
+{
+    MineParams prm = {};
+    prm.loc = a.loc; prm.conf = a.conf; prm.cls_u8 = a.cls_u8;
+    prm.gt_xyxy = (const float4*)a.gt_xyxy; prm.gt_cls = a.gt_cls; prm.gt_off = a.gt_off;
+    prm.pri_xyxy = (const float4*)a.pri_xyxy; prm.pri_cxcywh = (const float4*)a.pri_cxcywh;
+    prm.best_prior = a.best_prior; prm.npos = a.npos; prm.npos_norm = npos_norm;
+    prm.B = a.B; prm.P = a.P; prm.neg_ratio = a.neg_ratio; prm.bg_class = a.C - 1; prm.pos_iou = a.pos_iou;
+    prm.sums = a.sums; prm.losses = a.losses; prm.grad_loc = a.grad_loc; prm.grad_conf = a.grad_conf;
+    prm.mined_mask = a.mined_mask;
+    prm.done_counter = lw.done_counter;
+    prm.partials = lw.partials;
+    prm.ce = a.ce ? a.ce : lw.ce;
+    prm.ce_tap = a.ce;
+    if (mw) {
+        prm.cls_rw = a.cls_u8; prm.best_prior_w = a.best_prior; prm.npos_w = a.npos;
+        prm.best_key = mw->best_key; prm.npos_acc = mw->npos_acc; prm.arrive_total = mw->arrive_total;
+    }
+    return prm;
+}
+
+// The forced-match finaliser on its own: one CTA per image after the streaming kernel's natural match
+static int launch_finalize(const StepArgs& a, const MatchWs& mw, cudaStream_t st)
+{
+    match_finalize_kernel<<<a.B, 64, 0, st>>>(a.gt_cls, a.gt_off, a.B, a.P, a.C - 1, a.best_prior, a.npos, a.cls_u8,
+                                              mw.best_key, mw.npos_acc, mw.image_counter);
+    SSD_LAUNCH_CHECK();
+    count_launch();
+    return 0;
+}
+
+// The mining kernel of a step, with the finaliser fused in; a batch that does not fit co-resident (B > 2 CTAs x SMs)
+// gets the finaliser and the ordinary mining kernel instead, except a sharded one: its peer exchange needs the
+// co-resident grid.
+template <bool GRADS>
+static int launch_mine_step(const StepArgs& a, const MineParams& prm, const LevelTab* lv, const MatchWs& mw, cudaStream_t st)
+{
+    int rc = lv ? launch_mine<true>(mine_levels_kernel<21, GRADS, true>, a.B, a.P, st, prm, *lv)
+                : launch_mine<true>(mine_kernel<21, GRADS, true>, a.B, a.P, st, prm);
+    if (rc != 1) return rc;
+    if (prm.xchg_R > 1) return SSDHEAD_E_UNSUPPORTED;
+    rc = launch_finalize(a, mw, st);
+    if (rc) return rc;
+    return lv ? launch_mine<false>(mine_levels_kernel<21, GRADS, false>, a.B, a.P, st, prm, *lv)
+              : launch_mine<false>(mine_kernel<21, GRADS, false>, a.B, a.P, st, prm);
+}
+
+// The whole training-head step of one GPU in two kernels, on checked arguments with B > 0: the streaming CE kernel
+// with the fused natural match over [B*P] rows (lv == nullptr) or the per-level tensors of lv, then the mining kernel
+// with the forced-match finaliser fused in.  ws_rows: resident gradient tensors - the streaming kernel writes no zero
+// background (it runs forward-only), the mining kernel retracts the previous step's rows and writes this step's.
+static int step_impl(const StepArgs& a, const LevelTab* lv, const Xchg& x, void* ws_rows)
+{
+    cudaStream_t st = (cudaStream_t)a.stream;
+    const LossWs lw = loss_ws(a.ws_loss, a.B, a.P);
+    const MatchWs mw = match_ws(a.ws_match, a.B, a.sumG);
+    unsigned short* obj = a.sumG <= 65535 ? lw.obj : nullptr;
+    const FusedMatch fm = bind_match(a, mw, obj, !lv && match_cull_enabled(a.B, a.sumG) ? lw.seed : nullptr);
+    MineParams prm = bind_mine(a, lw, a.npos + a.B, &mw);
+    prm.obj_u16 = obj;
+    prm.xchg_R = x.R; prm.xchg_rank = x.rank; prm.xchg_seq = x.seq;
+    prm.xchg_peers = (unsigned long long* const*)x.peers; prm.xchg_local = (unsigned long long*)x.local; prm.err_flag = x.err_flag;
+    if (ws_rows) {
+        prm.res_base = (unsigned char*)ws_rows;
+        prm.res_stride = resident_row_stride(a.P);
+    }
+    if (lv) prm.ce_w = lw.ce;
+    const bool grads = lv ? lv->gconf[0] != nullptr : a.grad_loc != nullptr;
+    const bool ce_grads = grads && !ws_rows;
+    const long long rows = (long long)a.B * a.P;
+    float* ce = a.ce ? a.ce : lw.ce;
+    int rc = ce_grads ? launch_ce_stream<21, true, true>(a.conf, ce, a.grad_conf, a.grad_loc, rows, fm, lv, st)
+                      : launch_ce_stream<21, false, true>(a.conf, ce, nullptr, nullptr, rows, fm, lv, st);
+    if (rc) return rc;
+    if (a.mined_mask) SSD_CHECK_CUDA(cudaMemsetAsync(a.mined_mask, 0, (size_t)a.B * ((a.P + 31) / 32) * sizeof(uint32_t), st));
+    return grads ? launch_mine_step<true>(a, prm, lv, mw, st) : launch_mine_step<false>(a, prm, lv, mw, st);
+}
+
+static int step_flat(const StepArgs& a, const Xchg& x, void* ws_rows)
+{
+    int rc = check_mine(a, true);
+    if (!rc && (!aligned16(a.loc) || !aligned16(a.pri_cxcywh))) rc = SSDHEAD_E_ALIGN;
+    if (!rc) rc = check_match(a);
+    if (rc || a.B == 0) return rc;
+    return step_impl(a, nullptr, x, ws_rows);
+}
+
+static int step_levels(const ssdhead_levels* levels, const StepArgs& a, const Xchg& x)
+{
+    LevelTab lv = {};
+    int rc = check_mine(a, false);
+    if (!rc) rc = check_match(a);
+    if (!rc) rc = check_levels(levels, a.B, a.P, &lv);
+    if (rc || a.B == 0) return rc;
+    if (!aligned16(a.pri_cxcywh)) return SSDHEAD_E_ALIGN;
+    return step_impl(a, &lv, x, nullptr);
 }
 
 }  // namespace ssdhead
@@ -1536,66 +1747,19 @@ extern "C" {
 int ssdhead_ce_stream(const float* conf, int B, int P, int C, float* ce, float* grad_loc, float* grad_conf,
                       void* ws, size_t ws_bytes, void* stream)
 {
-    if (B < 0 || P <= 0 || !conf || !ws) return SSDHEAD_E_BADARG;
-    if ((grad_loc == nullptr) != (grad_conf == nullptr)) return SSDHEAD_E_BADARG;
-    if (C != 21) return SSDHEAD_E_UNSUPPORTED;          // VOC head of the reference (Losses.py:184 hard-codes 21)
-    if (B == 0) return 0;
-    if ((grad_loc && !aligned16(grad_loc)) || !aligned16(ws)) return SSDHEAD_E_ALIGN;
-    const size_t need = loss_workspace_bytes(B, P, C);
-    if (need == 0) return SSDHEAD_E_UNSUPPORTED;
-    if (ws_bytes < need) return SSDHEAD_E_WORKSPACE;
-    float* ce_buf = ce ? ce : ws_ce(ws, B);
+    if (!conf) return SSDHEAD_E_BADARG;
+    const int rc = check_loss(B, P, C, grad_loc, grad_conf, ws, ws_bytes);
+    if (rc || B == 0) return rc;
+    float* ce_buf = ce ? ce : loss_ws(ws, B, P).ce;
     const long long rows = (long long)B * P;
     FusedMatch none = {};
-    return grad_loc ? launch_ce_stream<21, true, false>(conf, ce_buf, grad_conf, grad_loc, rows, none, (cudaStream_t)stream)
-                    : launch_ce_stream<21, false, false>(conf, ce_buf, nullptr, nullptr, rows, none, (cudaStream_t)stream);
+    return grad_loc ? launch_ce_stream<21, true, false>(conf, ce_buf, grad_conf, grad_loc, rows, none, nullptr, (cudaStream_t)stream)
+                    : launch_ce_stream<21, false, false>(conf, ce_buf, nullptr, nullptr, rows, none, nullptr, (cudaStream_t)stream);
 }
 
 // ssdhead_ce_stream with the natural match fused in, followed by the per-image forced-match finaliser: produces
 // everything ssdhead_match produces for the loss (cls_u8, best_prior, npos) without a separate pass over the priors.
-static int ce_match_stream_impl(const float* conf, const float* gt_xyxy, const float* gt_cls, const int32_t* gt_off,
-                            const float* pri_xyxy, int B, int P, int C, int sumG, float pos_iou,
-                            float* ce, float* grad_loc, float* grad_conf,
-                            uint8_t* cls_u8, int32_t* best_prior, int32_t* npos,
-                            void* ws_loss, size_t ws_loss_bytes, void* ws_match, size_t ws_match_bytes, void* stream,
-                            bool run_finalizer, unsigned short* obj_u16 = nullptr)
-{
-    if (B < 0 || P <= 0 || sumG < 0 || !conf || !gt_off || !pri_xyxy || !cls_u8 || !npos || !ws_loss || !ws_match) return SSDHEAD_E_BADARG;
-    if (sumG > 0 && (!gt_xyxy || !gt_cls || !best_prior)) return SSDHEAD_E_BADARG;
-    if ((grad_loc == nullptr) != (grad_conf == nullptr)) return SSDHEAD_E_BADARG;
-    if (C != 21) return SSDHEAD_E_UNSUPPORTED;
-    if (B == 0) return 0;
-    if ((long long)B * P >= (1ll << 31)) return SSDHEAD_E_UNSUPPORTED;
-    if ((grad_loc && !aligned16(grad_loc)) || !aligned16(ws_loss) || !aligned16(ws_match) || !aligned16(pri_xyxy) ||
-        (sumG > 0 && !aligned16(gt_xyxy)))
-        return SSDHEAD_E_ALIGN;
-    const size_t need = loss_workspace_bytes(B, P, C);
-    if (need == 0) return SSDHEAD_E_UNSUPPORTED;
-    if (ws_loss_bytes < need) return SSDHEAD_E_WORKSPACE;
-    if (ws_match_bytes < ssdhead_workspace_bytes(SSDHEAD_WS_MATCH, B, P, C, sumG)) return SSDHEAD_E_WORKSPACE;
-    cudaStream_t st = (cudaStream_t)stream;
-    // match workspace layout (zero on entry, zero on exit): best_key[sumG] u64 | tile_counter[B] | npos_acc[B] | image_counter
-    char* w = (char*)ws_match;
-    unsigned long long* best_key = (unsigned long long*)w;            w += round_up((size_t)sumG * 8, 16);
-    w += round_up((size_t)B * 4, 16);
-    int* npos_acc = (int*)w;                                          w += round_up((size_t)B * 4, 16);
-    unsigned int* image_counter = (unsigned int*)w;
-    FusedMatch fm;
-    fm.gt_xyxy = (const float4*)gt_xyxy; fm.gt_cls = gt_cls; fm.gt_off = gt_off; fm.pri_xyxy = (const float4*)pri_xyxy;
-    fm.P = P; fm.bg_class = C - 1; fm.pos_iou = pos_iou; fm.cls_u8 = cls_u8; fm.best_key = best_key; fm.npos_acc = npos_acc; fm.obj_u16 = obj_u16;
-    fm.sumG = sumG; fm.seed_lb = match_cull_enabled(B, sumG) ? ws_seed(ws_loss, B, P) : nullptr;
-    float* ce_buf = ce ? ce : ws_ce(ws_loss, B);
-    const long long rows = (long long)B * P;
-    const int rc = grad_loc ? launch_ce_stream<21, true, true>(conf, ce_buf, grad_conf, grad_loc, rows, fm, st)
-                            : launch_ce_stream<21, false, true>(conf, ce_buf, nullptr, nullptr, rows, fm, st);
-    if (rc) return rc;
-    if (!run_finalizer) return 0;
-    SSD_CHECK_CUDA(launch_pdl(2, match_finalize_kernel, dim3(B), dim3(64), 0, st, gt_cls, gt_off, B, P, C - 1, best_prior, npos, cls_u8,
-                              best_key, npos_acc, image_counter));
-    count_launch();
-    return 0;
-}
-
+// It records no best-gt map: ssdhead_mine walks the gts.
 int ssdhead_ce_match_stream(const float* conf, const float* gt_xyxy, const float* gt_cls, const int32_t* gt_off,
                             const float* pri_xyxy, int B, int P, int C, int sumG, float pos_iou,
                             float* ce, float* grad_loc, float* grad_conf,
@@ -1603,22 +1767,29 @@ int ssdhead_ce_match_stream(const float* conf, const float* gt_xyxy, const float
                             void* ws_loss, size_t ws_loss_bytes, void* ws_match, size_t ws_match_bytes,
                             int run_finalizer, void* stream)
 {
-    return ce_match_stream_impl(conf, gt_xyxy, gt_cls, gt_off, pri_xyxy, B, P, C, sumG, pos_iou, ce, grad_loc, grad_conf,
-                                cls_u8, best_prior, npos, ws_loss, ws_loss_bytes, ws_match, ws_match_bytes, stream,
-                                run_finalizer != 0);
+    const StepArgs a = {.conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off, .pri_xyxy = pri_xyxy,
+                        .B = B, .P = P, .C = C, .sumG = sumG, .pos_iou = pos_iou, .grad_loc = grad_loc,
+                        .grad_conf = grad_conf, .cls_u8 = cls_u8, .best_prior = best_prior, .npos = npos, .ce = ce,
+                        .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes, .ws_match = ws_match,
+                        .ws_match_bytes = ws_match_bytes, .stream = stream};
+    if (!conf) return SSDHEAD_E_BADARG;
+    int rc = check_match(a);
+    if (rc || B == 0) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    const LossWs lw = loss_ws(ws_loss, B, P);
+    const MatchWs mw = match_ws(ws_match, B, sumG);
+    const FusedMatch fm = bind_match(a, mw, nullptr, match_cull_enabled(B, sumG) ? lw.seed : nullptr);
+    float* ce_buf = ce ? ce : lw.ce;
+    const long long rows = (long long)B * P;
+    rc = grad_loc ? launch_ce_stream<21, true, true>(conf, ce_buf, grad_conf, grad_loc, rows, fm, nullptr, st)
+                  : launch_ce_stream<21, false, true>(conf, ce_buf, nullptr, nullptr, rows, fm, nullptr, st);
+    if (rc || !run_finalizer) return rc;
+    return launch_finalize(a, mw, st);
 }
 
-static int multibox_step_impl(const float* loc, const float* conf,
-                          const float* gt_xyxy, const float* gt_cls, const int32_t* gt_off,
-                          const float* pri_xyxy, const float* pri_cxcywh,
-                          int B, int P, int C, int sumG, int neg_ratio, float pos_iou,
-                          double* sums, float* losses, float* grad_loc, float* grad_conf,
-                          uint8_t* cls_u8, int32_t* best_prior, int32_t* npos,
-                          uint32_t* mined_mask, float* ce,
-                          void* ws_loss, size_t ws_loss_bytes, void* ws_match, size_t ws_match_bytes, void* stream,
-                          int R, int rank, unsigned seq, void* const* peers_dev, void* xchg_local, int* err_flag,
-                          void* ws_rows = nullptr, size_t ws_rows_bytes = 0);
-
+// The whole training-head step of ONE GPU in two kernels: the streaming CE kernel with the fused natural match,
+// then the mining kernel with the forced-match finaliser fused in (cooperative launch).  When the batch does not fit
+// co-resident (B > 2 CTAs x SMs) the finaliser and the ordinary mining kernel run separately (three kernels).
 int ssdhead_multibox_step(const float* loc, const float* conf,
                           const float* gt_xyxy, const float* gt_cls, const int32_t* gt_off,
                           const float* pri_xyxy, const float* pri_cxcywh,
@@ -1628,9 +1799,14 @@ int ssdhead_multibox_step(const float* loc, const float* conf,
                           uint32_t* mined_mask, float* ce,
                           void* ws_loss, size_t ws_loss_bytes, void* ws_match, size_t ws_match_bytes, void* stream)
 {
-    return multibox_step_impl(loc, conf, gt_xyxy, gt_cls, gt_off, pri_xyxy, pri_cxcywh, B, P, C, sumG, neg_ratio, pos_iou,
-                              sums, losses, grad_loc, grad_conf, cls_u8, best_prior, npos, mined_mask, ce,
-                              ws_loss, ws_loss_bytes, ws_match, ws_match_bytes, stream, 0, 0, 0u, nullptr, nullptr, nullptr);
+    const StepArgs a = {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off,
+                        .pri_xyxy = pri_xyxy, .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG,
+                        .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses,
+                        .grad_loc = grad_loc, .grad_conf = grad_conf, .cls_u8 = cls_u8, .best_prior = best_prior,
+                        .npos = npos, .mined_mask = mined_mask, .ce = ce, .ws_loss = ws_loss,
+                        .ws_loss_bytes = ws_loss_bytes, .ws_match = ws_match, .ws_match_bytes = ws_match_bytes,
+                        .stream = stream};
+    return step_flat(a, Xchg{}, nullptr);
 }
 
 // The same two kernels for a batch sharded by image over R GPUs: the mining kernel exchanges the positive count (before
@@ -1647,12 +1823,15 @@ int ssdhead_multibox_step_sharded(const float* loc, const float* conf,
                           int R, int rank, unsigned int seq, void* const* peers_dev, void* xchg_local_dev, int32_t* err_flag_dev,
                           void* stream)
 {
-    if (R < 1 || R > XCHG_MAX_R || rank < 0 || rank >= R || seq == 0u) return SSDHEAD_E_BADARG;
-    if (R > 1 && (!peers_dev || !xchg_local_dev || !err_flag_dev)) return SSDHEAD_E_BADARG;
-    return multibox_step_impl(loc, conf, gt_xyxy, gt_cls, gt_off, pri_xyxy, pri_cxcywh, B, P, C, sumG, neg_ratio, pos_iou,
-                              sums, losses, grad_loc, grad_conf, cls_u8, best_prior, npos, nullptr, nullptr,
-                              ws_loss, ws_loss_bytes, ws_match, ws_match_bytes, stream, R, rank, seq, peers_dev, xchg_local_dev,
-                              err_flag_dev);
+    const StepArgs a = {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off,
+                        .pri_xyxy = pri_xyxy, .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG,
+                        .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses,
+                        .grad_loc = grad_loc, .grad_conf = grad_conf, .cls_u8 = cls_u8, .best_prior = best_prior,
+                        .npos = npos, .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes, .ws_match = ws_match,
+                        .ws_match_bytes = ws_match_bytes, .stream = stream};
+    const Xchg x = {R, rank, seq, peers_dev, xchg_local_dev, err_flag_dev};
+    const int rc = check_xchg(x, true);
+    return rc ? rc : step_flat(a, x, nullptr);
 }
 
 // ssdhead_multibox_step with RESIDENT gradient tensors: grad_loc / grad_conf are all-zero when first handed over (together
@@ -1672,149 +1851,21 @@ int ssdhead_multibox_step_resident(const float* loc, const float* conf,
                           int R, int rank, unsigned int seq, void* const* peers_dev, void* xchg_local_dev, int32_t* err_flag_dev,
                           void* stream)
 {
-    if (!ws_rows || !grad_loc || !grad_conf) return SSDHEAD_E_BADARG;
-    if (R < 1 || R > XCHG_MAX_R || rank < 0 || rank >= R || (R > 1 && seq == 0u)) return SSDHEAD_E_BADARG;
-    if (R > 1 && (!peers_dev || !xchg_local_dev || !err_flag_dev)) return SSDHEAD_E_BADARG;
-    return multibox_step_impl(loc, conf, gt_xyxy, gt_cls, gt_off, pri_xyxy, pri_cxcywh, B, P, C, sumG, neg_ratio, pos_iou,
-                              sums, losses, grad_loc, grad_conf, cls_u8, best_prior, npos, nullptr, nullptr,
-                              ws_loss, ws_loss_bytes, ws_match, ws_match_bytes, stream,
-                              R > 1 ? R : 0, rank, seq, peers_dev, xchg_local_dev, err_flag_dev, ws_rows, ws_rows_bytes);
+    const StepArgs a = {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off,
+                        .pri_xyxy = pri_xyxy, .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG,
+                        .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses,
+                        .grad_loc = grad_loc, .grad_conf = grad_conf, .cls_u8 = cls_u8, .best_prior = best_prior,
+                        .npos = npos, .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes, .ws_match = ws_match,
+                        .ws_match_bytes = ws_match_bytes, .stream = stream};
+    Xchg x = {R, rank, seq, peers_dev, xchg_local_dev, err_flag_dev};
+    int rc = check_resident(a, ws_rows, ws_rows_bytes);
+    if (!rc) rc = check_xchg(x, R > 1);
+    if (rc) return rc;
+    if (R == 1) x.R = 0;                                 // one GPU: no exchange
+    return step_flat(a, x, ws_rows);
 }
 
 // ssdhead_multibox_step on per-level head tensors (SURVEY.md 8(f) #3, Model.py:212-235 without the permute/cat copies)
-extern "C++" {
-template <bool GRADS>
-static int multibox_step_levels_impl(const LevelTab& lv, const FusedMatch& fm, MineParams prm, int B, int P,
-                                     unsigned int* image_counter, cudaStream_t st)
-{
-    constexpr int C = 21;
-    constexpr size_t tile = (size_t)CE_ROWS * C * 4;
-    const size_t smem_ce = tile * CE_STAGES + (GRADS ? (size_t)CE_ZERO_ROWS * C * 4 : 0);
-    auto kce = ce_stream_levels_kernel<C, GRADS>;
-    SSD_CHECK_CUDA(cudaFuncSetAttribute(kce, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ce));
-    const long long rows = (long long)B * P;
-    const long long tiles = (rows + CE_ROWS - 1) / CE_ROWS + lv.n;
-    const int grid_ce = (int)std::min<long long>(tiles, (long long)CE_CTAS * num_sms());
-    LevelTab lt = lv;
-    {
-        // stride ~ 0.618 T, coprime with T: consecutive visits land in different levels in proportion to their sizes
-        const long long T = lv.tile0[lv.n];
-        auto gcd = [](long long a, long long b) { while (b) { const long long c = a % b; a = b; b = c; } return a; };
-        long long S = std::max<long long>(1, (long long)(0.6180339887 * (double)T));
-        while (S > 1 && gcd(S, T) != 1) --S;
-        lt.perm_stride = (int)S;
-        lt.perm_inc = T > 0 ? (int)(((long long)grid_ce * S) % T) : 0;
-    }
-    SSD_CHECK_CUDA(launch_pdl(1, kce, dim3(grid_ce), dim3(CE_THREADS), smem_ce, st, prm.ce_w, rows, fm, lt));
-    count_launch();
-
-    const size_t smem_mn = mine_smem_bytes(P);
-    auto kfin = mine_levels_kernel<C, GRADS, true>;
-    SSD_CHECK_CUDA(cudaFuncSetAttribute(kfin, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_mn));
-    int per_sm = 0;
-    SSD_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kfin, MN_T, smem_mn));
-    if ((long long)per_sm * num_sms() >= B) {
-        void* args[] = {&prm, (void*)&lv};
-        SSD_CHECK_CUDA(cudaLaunchCooperativeKernel((const void*)kfin, dim3(B), dim3(MN_T), args, smem_mn, st));
-        count_launch();
-        return 0;
-    }
-    if (prm.xchg_R > 1) return SSDHEAD_E_UNSUPPORTED;    // the peer exchange needs the co-resident grid
-    // does not fit co-resident: separate finaliser, ordinary mining kernel
-    SSD_CHECK_CUDA(launch_pdl(2, match_finalize_kernel, dim3(B), dim3(64), 0, st, fm.gt_cls, fm.gt_off, B, P, C - 1,
-                              prm.best_prior_w, prm.npos_w, prm.cls_rw, prm.best_key, prm.npos_acc, image_counter));
-    count_launch();
-    prm.best_prior = prm.best_prior_w; prm.npos = prm.npos_w; prm.npos_norm = prm.npos_w + B;
-    auto kmn = mine_levels_kernel<C, GRADS, false>;
-    SSD_CHECK_CUDA(cudaFuncSetAttribute(kmn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_mn));
-    SSD_CHECK_CUDA(launch_pdl(4, kmn, dim3(B), dim3(MN_T), smem_mn, st, prm, lv));
-    count_launch();
-    return 0;
-}
-}  // extern "C++"
-
-static int step_levels_common(const ssdhead_levels* levels,
-                              const float* gt_xyxy, const float* gt_cls, const int32_t* gt_off,
-                              const float* pri_xyxy, const float* pri_cxcywh,
-                              int B, int P, int C, int sumG, int neg_ratio, float pos_iou,
-                              double* sums, float* losses,
-                              uint8_t* cls_u8, int32_t* best_prior, int32_t* npos,
-                              void* ws_loss, size_t ws_loss_bytes, void* ws_match, size_t ws_match_bytes, void* stream,
-                              int R, int rank, unsigned seq, void* const* peers_dev, void* xchg_local, int* err_flag)
-{
-    if (!levels || B < 0 || P <= 0 || sumG < 0 || neg_ratio < 0) return SSDHEAD_E_BADARG;
-    if (!gt_off || !pri_xyxy || !pri_cxcywh || !sums || !losses || !cls_u8 || !npos || !ws_loss || !ws_match) return SSDHEAD_E_BADARG;
-    if (sumG > 0 && (!gt_xyxy || !gt_cls || !best_prior)) return SSDHEAD_E_BADARG;
-    if (levels->num_levels < 1 || levels->num_levels > MAX_LEVELS) return SSDHEAD_E_BADARG;
-    if (C != 21) return SSDHEAD_E_UNSUPPORTED;
-    if (B == 0) return 0;
-    if ((long long)B * P >= (1ll << 31)) return SSDHEAD_E_UNSUPPORTED;
-    if (!aligned16(ws_loss) || !aligned16(ws_match) || !aligned16(pri_xyxy) || !aligned16(pri_cxcywh) || (sumG > 0 && !aligned16(gt_xyxy)))
-        return SSDHEAD_E_ALIGN;
-    LevelTab lv = {};
-    lv.n = levels->num_levels;
-    int sum = 0, with_grads = 0;
-    int t0 = 0;
-    for (int l = 0; l < lv.n; ++l) {
-        const int n = levels->count[l];
-        if (n <= 0 || !levels->conf[l] || !levels->loc[l]) return SSDHEAD_E_BADARG;
-        if (!aligned16(levels->loc[l])) return SSDHEAD_E_ALIGN;                        // float4 rows
-        const bool g = levels->grad_conf[l] != nullptr;
-        if (g != (levels->grad_loc[l] != nullptr)) return SSDHEAD_E_BADARG;
-        if (g && !aligned16(levels->grad_loc[l])) return SSDHEAD_E_ALIGN;
-        // conf / grad_conf rows are 84 bytes: a level whose pointers are not 16-byte aligned (e.g. a view into a larger
-        // tensor) cannot ride the TMA pipeline and goes through the plain-load path entirely
-        const bool tma_ok = aligned16(levels->conf[l]) && (!g || aligned16(levels->grad_conf[l]));
-        with_grads += g ? 1 : 0;
-        lv.cnt[l] = n; lv.start[l] = sum; lv.tile0[l] = t0;
-        lv.conf[l] = levels->conf[l]; lv.loc[l] = levels->loc[l]; lv.gconf[l] = levels->grad_conf[l]; lv.gloc[l] = levels->grad_loc[l];
-        sum += n;
-        const long long rows_l = (long long)B * n;
-        lv.rows[l] = (int)rows_l;
-        // the partial last tile of a level rides the TMA pipeline too when its byte counts are multiples of 16
-        if (tma_ok) t0 += (int)(rows_l / CE_ROWS) + ((rows_l % CE_ROWS) != 0 && (rows_l % 4) == 0 ? 1 : 0);
-    }
-    for (int l = lv.n; l <= MAX_LEVELS; ++l) { lv.start[l] = sum; lv.tile0[l] = t0; }
-    if (sum != P) return SSDHEAD_E_BADARG;
-    if (with_grads != 0 && with_grads != lv.n) return SSDHEAD_E_BADARG;
-    const size_t need = loss_workspace_bytes(B, P, C);
-    if (need == 0) return SSDHEAD_E_UNSUPPORTED;
-    if (ws_loss_bytes < need) return SSDHEAD_E_WORKSPACE;
-    if (ws_match_bytes < ssdhead_workspace_bytes(SSDHEAD_WS_MATCH, B, P, C, sumG)) return SSDHEAD_E_WORKSPACE;
-    cudaStream_t st = (cudaStream_t)stream;
-    char* w = (char*)ws_match;
-    unsigned long long* best_key = (unsigned long long*)w;            w += round_up((size_t)sumG * 8, 16);
-    w += round_up((size_t)B * 4, 16);
-    int* npos_acc = (int*)w;                                          w += round_up((size_t)B * 4, 16);
-    unsigned int* image_counter = (unsigned int*)w;
-    FusedMatch fm;
-    fm.gt_xyxy = (const float4*)gt_xyxy; fm.gt_cls = gt_cls; fm.gt_off = gt_off; fm.pri_xyxy = (const float4*)pri_xyxy;
-    fm.P = P; fm.bg_class = C - 1; fm.pos_iou = pos_iou; fm.cls_u8 = cls_u8; fm.best_key = best_key; fm.npos_acc = npos_acc; fm.obj_u16 = use_obj_map(B, sumG) ? ws_obj(ws_loss, B, P) : nullptr;
-    fm.sumG = sumG; fm.seed_lb = nullptr;                    // (per-level layout: not seeded)
-
-    MineParams prm = {};
-    prm.loc = nullptr; prm.conf = nullptr; prm.cls_u8 = cls_u8;
-    prm.gt_xyxy = (const float4*)gt_xyxy; prm.gt_cls = gt_cls; prm.gt_off = gt_off;
-    prm.pri_xyxy = (const float4*)pri_xyxy; prm.pri_cxcywh = (const float4*)pri_cxcywh;
-    prm.best_prior = best_prior; prm.npos = npos; prm.npos_norm = npos + B;
-    prm.B = B; prm.P = P; prm.neg_ratio = neg_ratio; prm.bg_class = C - 1; prm.pos_iou = pos_iou;
-    prm.sums = sums; prm.losses = losses; prm.grad_loc = nullptr; prm.grad_conf = nullptr;
-    prm.mined_mask = nullptr;
-    prm.done_counter = (unsigned int*)ws_loss;
-    prm.partials = (double*)((char*)ws_loss + 16);
-    prm.ce_w = ws_ce(ws_loss, B);
-    prm.ce = prm.ce_w;
-    prm.ce_tap = nullptr;
-    prm.obj_u16 = fm.obj_u16;
-    prm.cls_rw = cls_u8; prm.best_prior_w = best_prior; prm.npos_w = npos;
-    prm.best_key = best_key; prm.npos_acc = npos_acc;
-    prm.arrive_total = (unsigned long long*)(image_counter + 2);
-    prm.xchg_R = R; prm.xchg_rank = rank; prm.xchg_seq = seq;
-    prm.xchg_peers = (unsigned long long* const*)peers_dev; prm.xchg_local = (unsigned long long*)xchg_local; prm.err_flag = err_flag;
-    return with_grads ? multibox_step_levels_impl<true>(lv, fm, prm, B, P, image_counter, st)
-                      : multibox_step_levels_impl<false>(lv, fm, prm, B, P, image_counter, st);
-}
-
 int ssdhead_multibox_step_levels(const ssdhead_levels* levels,
                                  const float* gt_xyxy, const float* gt_cls, const int32_t* gt_off,
                                  const float* pri_xyxy, const float* pri_cxcywh,
@@ -1823,9 +1874,12 @@ int ssdhead_multibox_step_levels(const ssdhead_levels* levels,
                                  uint8_t* cls_u8, int32_t* best_prior, int32_t* npos,
                                  void* ws_loss, size_t ws_loss_bytes, void* ws_match, size_t ws_match_bytes, void* stream)
 {
-    return step_levels_common(levels, gt_xyxy, gt_cls, gt_off, pri_xyxy, pri_cxcywh, B, P, C, sumG, neg_ratio, pos_iou,
-                              sums, losses, cls_u8, best_prior, npos, ws_loss, ws_loss_bytes, ws_match, ws_match_bytes, stream,
-                              0, 0, 0u, nullptr, nullptr, nullptr);
+    const StepArgs a = {.gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off, .pri_xyxy = pri_xyxy,
+                        .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG, .neg_ratio = neg_ratio,
+                        .pos_iou = pos_iou, .sums = sums, .losses = losses, .cls_u8 = cls_u8,
+                        .best_prior = best_prior, .npos = npos, .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes,
+                        .ws_match = ws_match, .ws_match_bytes = ws_match_bytes, .stream = stream};
+    return step_levels(levels, a, Xchg{});
 }
 
 // the per-level step of a batch sharded by image over R GPUs (peer-memory exchange inside the mining kernel, as in
@@ -1840,59 +1894,41 @@ int ssdhead_multibox_step_levels_sharded(const ssdhead_levels* levels,
                                  int R, int rank, unsigned int seq, void* const* peers_dev, void* xchg_local_dev, int32_t* err_flag_dev,
                                  void* stream)
 {
-    if (R < 1 || R > XCHG_MAX_R || rank < 0 || rank >= R || seq == 0u) return SSDHEAD_E_BADARG;
-    if (R > 1 && (!peers_dev || !xchg_local_dev || !err_flag_dev)) return SSDHEAD_E_BADARG;
-    return step_levels_common(levels, gt_xyxy, gt_cls, gt_off, pri_xyxy, pri_cxcywh, B, P, C, sumG, neg_ratio, pos_iou,
-                              sums, losses, cls_u8, best_prior, npos, ws_loss, ws_loss_bytes, ws_match, ws_match_bytes, stream,
-                              R, rank, seq, peers_dev, xchg_local_dev, err_flag_dev);
+    const StepArgs a = {.gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off, .pri_xyxy = pri_xyxy,
+                        .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG, .neg_ratio = neg_ratio,
+                        .pos_iou = pos_iou, .sums = sums, .losses = losses, .cls_u8 = cls_u8,
+                        .best_prior = best_prior, .npos = npos, .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes,
+                        .ws_match = ws_match, .ws_match_bytes = ws_match_bytes, .stream = stream};
+    const Xchg x = {R, rank, seq, peers_dev, xchg_local_dev, err_flag_dev};
+    const int rc = check_xchg(x, true);
+    return rc ? rc : step_levels(levels, a, x);
 }
 
 size_t ssdhead_xchg_bytes(void) { return (size_t)XCHG_WORDS * 8; }
 
-static int mine_impl(const float* loc, const float* conf,
-                 const float* gt_xyxy, const float* gt_cls, const int32_t* gt_off,
-                 const float* pri_xyxy, const float* pri_cxcywh,
-                 const int32_t* best_prior, const int32_t* npos, const int32_t* npos_norm, const uint8_t* cls_u8,
-                 int B, int P, int C, int neg_ratio, float pos_iou,
-                 double* sums, float* losses, float* grad_loc, float* grad_conf,
-                 uint32_t* mined_mask, float* ce,
-                 void* ws, size_t ws_bytes, void* stream,
-                 int sp_cap, int32_t* sp_cnt, int32_t* sp_idx, float* sp_conf, float* sp_loc)
+// The mining kernel alone, on the match of an earlier call; sp_cnt != nullptr: the gradient returns as packed rows
+static int mine_impl(const StepArgs& a, const int32_t* npos_norm,
+                     int sp_cap, int32_t* sp_cnt, int32_t* sp_idx, float* sp_conf, float* sp_loc)
 {
-    if (B < 0 || P <= 0 || neg_ratio < 0) return SSDHEAD_E_BADARG;
-    if (!loc || !conf || !gt_off || !pri_xyxy || !pri_cxcywh || !npos || !npos_norm || !cls_u8 || !sums || !losses || !ws)
-        return SSDHEAD_E_BADARG;
-    if ((grad_loc == nullptr) != (grad_conf == nullptr)) return SSDHEAD_E_BADARG;
+    if (!a.gt_off || !a.pri_xyxy || !a.npos || !npos_norm || !a.cls_u8) return SSDHEAD_E_BADARG;
     const bool sparse = sp_cnt != nullptr;
-    if (sparse && (sp_cap <= 0 || !sp_idx || !sp_conf || !sp_loc || grad_loc)) return SSDHEAD_E_BADARG;
-    if (C != 21) return SSDHEAD_E_UNSUPPORTED;
-    if (B == 0) return 0;
-    if (!aligned16(loc) || !aligned16(pri_xyxy) || !aligned16(pri_cxcywh) || (gt_xyxy && !aligned16(gt_xyxy)) ||
-        (grad_loc && !aligned16(grad_loc)) || !aligned16(ws) || (sparse && !aligned16(sp_loc)))
+    if (sparse && (sp_cap <= 0 || !sp_idx || !sp_conf || !sp_loc || a.grad_loc)) return SSDHEAD_E_BADARG;
+    int rc = check_mine(a, true);
+    if (!rc) rc = check_loss(a.B, a.P, a.C, a.grad_loc, a.grad_conf, a.ws_loss, a.ws_loss_bytes);
+    if (rc || a.B == 0) return rc;
+    if (!aligned16(a.loc) || !aligned16(a.pri_xyxy) || !aligned16(a.pri_cxcywh) || (a.gt_xyxy && !aligned16(a.gt_xyxy)) ||
+        (sparse && !aligned16(sp_loc)))
         return SSDHEAD_E_ALIGN;
-    const size_t need = loss_workspace_bytes(B, P, C);
-    if (need == 0) return SSDHEAD_E_UNSUPPORTED;
-    if (ws_bytes < need) return SSDHEAD_E_WORKSPACE;
-    cudaStream_t st = (cudaStream_t)stream;
-
-    MineParams prm = {};
-    prm.loc = loc; prm.conf = conf; prm.cls_u8 = cls_u8;
-    prm.gt_xyxy = (const float4*)gt_xyxy; prm.gt_cls = gt_cls; prm.gt_off = gt_off;
-    prm.pri_xyxy = (const float4*)pri_xyxy; prm.pri_cxcywh = (const float4*)pri_cxcywh;
-    prm.best_prior = best_prior; prm.npos = npos; prm.npos_norm = npos_norm;
-    prm.B = B; prm.P = P; prm.neg_ratio = neg_ratio; prm.bg_class = C - 1; prm.pos_iou = pos_iou;
-    prm.sums = sums; prm.losses = losses; prm.grad_loc = grad_loc; prm.grad_conf = grad_conf;
-    prm.mined_mask = mined_mask;
-    prm.done_counter = (unsigned int*)ws;
-    prm.partials = (double*)((char*)ws + 16);
-    prm.ce = ce ? ce : ws_ce(ws, B);
-    prm.ce_tap = ce;
+    cudaStream_t st = (cudaStream_t)a.stream;
+    MineParams prm = bind_mine(a, loss_ws(a.ws_loss, a.B, a.P), npos_norm, nullptr);
     prm.sp_cap = sp_cap; prm.sp_cnt = sp_cnt; prm.sp_idx = sp_idx; prm.sp_conf = sp_conf; prm.sp_loc = sp_loc;
-    if (mined_mask) SSD_CHECK_CUDA(cudaMemsetAsync(mined_mask, 0, (size_t)B * ((P + 31) / 32) * sizeof(uint32_t), st));
-    if (sparse) return launch_mine_sparse<21>(prm, st);
-    return grad_loc ? launch_mine<21, true>(prm, st) : launch_mine<21, false>(prm, st);
+    if (a.mined_mask) SSD_CHECK_CUDA(cudaMemsetAsync(a.mined_mask, 0, (size_t)a.B * ((a.P + 31) / 32) * sizeof(uint32_t), st));
+    if (sparse) return launch_mine<false>(mine_sparse_kernel<21>, a.B, a.P, st, prm);
+    return a.grad_loc ? launch_mine<false>(mine_kernel<21, true, false>, a.B, a.P, st, prm)
+                      : launch_mine<false>(mine_kernel<21, false, false>, a.B, a.P, st, prm);
 }
 
+// (the match outputs in StepArgs are writable for the steps that produce them; the mining kernel only reads them)
 int ssdhead_mine(const float* loc, const float* conf,
                  const float* gt_xyxy, const float* gt_cls, const int32_t* gt_off,
                  const float* pri_xyxy, const float* pri_cxcywh,
@@ -1902,9 +1938,14 @@ int ssdhead_mine(const float* loc, const float* conf,
                  uint32_t* mined_mask, float* ce,
                  void* ws, size_t ws_bytes, void* stream)
 {
-    return mine_impl(loc, conf, gt_xyxy, gt_cls, gt_off, pri_xyxy, pri_cxcywh, best_prior, npos, npos_norm, cls_u8,
-                     B, P, C, neg_ratio, pos_iou, sums, losses, grad_loc, grad_conf, mined_mask, ce, ws, ws_bytes, stream,
-                     0, nullptr, nullptr, nullptr, nullptr);
+    const StepArgs a = {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off,
+                        .pri_xyxy = pri_xyxy, .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C,
+                        .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses,
+                        .grad_loc = grad_loc, .grad_conf = grad_conf, .cls_u8 = const_cast<uint8_t*>(cls_u8),
+                        .best_prior = const_cast<int32_t*>(best_prior), .npos = const_cast<int32_t*>(npos),
+                        .mined_mask = mined_mask, .ce = ce, .ws_loss = ws, .ws_loss_bytes = ws_bytes,
+                        .stream = stream};
+    return mine_impl(a, npos_norm, 0, nullptr, nullptr, nullptr, nullptr);
 }
 
 int ssdhead_mine_sparse(const float* loc, const float* conf,
@@ -1917,80 +1958,13 @@ int ssdhead_mine_sparse(const float* loc, const float* conf,
                  void* ws, size_t ws_bytes, void* stream)
 {
     if (!row_cnt) return SSDHEAD_E_BADARG;
-    return mine_impl(loc, conf, gt_xyxy, gt_cls, gt_off, pri_xyxy, pri_cxcywh, best_prior, npos, npos_norm, cls_u8,
-                     B, P, C, neg_ratio, pos_iou, sums, losses, nullptr, nullptr, nullptr, nullptr, ws, ws_bytes, stream,
-                     row_cap, row_cnt, row_idx, grad_conf_rows, grad_loc_rows);
-}
-
-// The whole training-head step of ONE GPU in two kernels: the streaming CE kernel with the fused natural match,
-// then the mining kernel with the forced-match finaliser fused in (cooperative launch).  When the batch does not fit
-// co-resident (B > 2 CTAs x SMs) it falls back to ssdhead_ce_match_stream + ssdhead_mine (three kernels).
-static int multibox_step_impl(const float* loc, const float* conf,
-                          const float* gt_xyxy, const float* gt_cls, const int32_t* gt_off,
-                          const float* pri_xyxy, const float* pri_cxcywh,
-                          int B, int P, int C, int sumG, int neg_ratio, float pos_iou,
-                          double* sums, float* losses, float* grad_loc, float* grad_conf,
-                          uint8_t* cls_u8, int32_t* best_prior, int32_t* npos,
-                          uint32_t* mined_mask, float* ce,
-                          void* ws_loss, size_t ws_loss_bytes, void* ws_match, size_t ws_match_bytes, void* stream,
-                          int R, int rank, unsigned seq, void* const* peers_dev, void* xchg_local, int* err_flag,
-                          void* ws_rows, size_t ws_rows_bytes)
-{
-    if (!loc || !pri_cxcywh || !sums || !losses || neg_ratio < 0) return SSDHEAD_E_BADARG;
-    if (!aligned16(loc) || !aligned16(pri_cxcywh)) return SSDHEAD_E_ALIGN;
-    // resident gradient tensors: the streaming kernel writes no zero background (it runs forward-only), the mining
-    // kernel retracts the previous step's rows and writes this step's
-    const bool resident = ws_rows != nullptr;
-    if (resident) {
-        if (!grad_loc || !grad_conf || B < 0 || P <= 0 || P >= 65536) return SSDHEAD_E_BADARG;
-        if (!aligned16(ws_rows) || !aligned16(grad_loc)) return SSDHEAD_E_ALIGN;
-        if (ws_rows_bytes < resident_rows_bytes(B, P)) return SSDHEAD_E_WORKSPACE;
-    }
-    // (ws_loss is validated by the call below before anything is written through this pointer)
-    unsigned short* obj_map = (ws_loss && B > 0 && use_obj_map(B, sumG) && loss_workspace_bytes(B, P, C) && ws_loss_bytes >= loss_workspace_bytes(B, P, C))
-                                  ? ws_obj(ws_loss, B, P) : nullptr;
-    int rc = ce_match_stream_impl(conf, gt_xyxy, gt_cls, gt_off, pri_xyxy, B, P, C, sumG, pos_iou, ce,
-                                  resident ? nullptr : grad_loc, resident ? nullptr : grad_conf,
-                                  cls_u8, best_prior, npos, ws_loss, ws_loss_bytes, ws_match, ws_match_bytes, stream, false, obj_map);
-    if (rc || B == 0) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    char* w = (char*)ws_match;
-    unsigned long long* best_key = (unsigned long long*)w;            w += round_up((size_t)sumG * 8, 16);
-    w += round_up((size_t)B * 4, 16);
-    int* npos_acc = (int*)w;                                          w += round_up((size_t)B * 4, 16);
-    unsigned int* image_counter = (unsigned int*)w;
-
-    MineParams prm = {};
-    prm.loc = loc; prm.conf = conf; prm.cls_u8 = cls_u8;
-    prm.gt_xyxy = (const float4*)gt_xyxy; prm.gt_cls = gt_cls; prm.gt_off = gt_off;
-    prm.pri_xyxy = (const float4*)pri_xyxy; prm.pri_cxcywh = (const float4*)pri_cxcywh;
-    prm.best_prior = best_prior; prm.npos = npos; prm.npos_norm = npos + B;
-    prm.B = B; prm.P = P; prm.neg_ratio = neg_ratio; prm.bg_class = C - 1; prm.pos_iou = pos_iou;
-    prm.sums = sums; prm.losses = losses; prm.grad_loc = grad_loc; prm.grad_conf = grad_conf;
-    prm.mined_mask = mined_mask;
-    prm.done_counter = (unsigned int*)ws_loss;
-    prm.partials = (double*)((char*)ws_loss + 16);
-    prm.ce = ce ? ce : ws_ce(ws_loss, B);
-    prm.ce_tap = ce;
-    prm.obj_u16 = obj_map;
-    prm.cls_rw = cls_u8; prm.best_prior_w = best_prior; prm.npos_w = npos;
-    prm.best_key = best_key; prm.npos_acc = npos_acc;
-    prm.arrive_total = (unsigned long long*)(image_counter + 2);   // 8-byte aligned word of the 16-byte tail
-    prm.xchg_R = R; prm.xchg_rank = rank; prm.xchg_seq = seq;
-    prm.xchg_peers = (unsigned long long* const*)peers_dev; prm.xchg_local = (unsigned long long*)xchg_local; prm.err_flag = err_flag;
-    if (resident) {
-        prm.res_base = (unsigned char*)ws_rows;
-        prm.res_stride = resident_row_stride(P);
-    }
-    if (mined_mask) SSD_CHECK_CUDA(cudaMemsetAsync(mined_mask, 0, (size_t)B * ((P + 31) / 32) * sizeof(uint32_t), st));
-    rc = grad_loc ? launch_mine_fin<21, true>(prm, st) : launch_mine_fin<21, false>(prm, st);
-    if (rc != 1) return rc;
-    if (R > 1) return SSDHEAD_E_UNSUPPORTED;       // the peer exchange needs the co-resident grid: use the NCCL route
-    // does not fit co-resident: separate finaliser, ordinary mining kernel
-    SSD_CHECK_CUDA(launch_pdl(2, match_finalize_kernel, dim3(B), dim3(64), 0, st, gt_cls, gt_off, B, P, C - 1, best_prior, npos, cls_u8,
-                              best_key, npos_acc, image_counter));
-    count_launch();
-    return grad_loc ? launch_mine<21, true>(prm, st) : launch_mine<21, false>(prm, st);
+    const StepArgs a = {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off,
+                        .pri_xyxy = pri_xyxy, .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C,
+                        .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses,
+                        .cls_u8 = const_cast<uint8_t*>(cls_u8), .best_prior = const_cast<int32_t*>(best_prior),
+                        .npos = const_cast<int32_t*>(npos), .ws_loss = ws, .ws_loss_bytes = ws_bytes,
+                        .stream = stream};
+    return mine_impl(a, npos_norm, row_cap, row_cnt, row_idx, grad_conf_rows, grad_loc_rows);
 }
 
 int ssdhead_multibox_loss(const float* loc, const float* conf,

@@ -424,21 +424,15 @@ int ssdhead_match(const float* gt_xyxy, const float* gt_cls, const int32_t* gt_o
     if (sumG > 0 && (!gt_xyxy || !gt_cls || !best_prior)) return SSDHEAD_E_BADARG;
     if (B > 65535) return SSDHEAD_E_UNSUPPORTED;
     if (!aligned16(pri_xyxy) || (sumG > 0 && !aligned16(gt_xyxy)) || !aligned16(ws)) return SSDHEAD_E_ALIGN;
-    const size_t need = ssdhead_workspace_bytes(SSDHEAD_WS_MATCH, B, P, C, sumG);
-    if (ws_bytes < need) return SSDHEAD_E_WORKSPACE;
+    if (ws_bytes < match_ws_bytes(B, sumG)) return SSDHEAD_E_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
-    // workspace (zero on entry, zero on exit): best_key[sumG] u64 | tile_counter[B] | npos_acc[B] | image_counter
-    char* w = (char*)ws;
-    unsigned long long* best_key = (unsigned long long*)w;            w += round_up((size_t)sumG * 8, 16);
-    unsigned int* tile_counter = (unsigned int*)w;                    w += round_up((size_t)B * 4, 16);
-    int* npos_acc = (int*)w;                                          w += round_up((size_t)B * 4, 16);
-    unsigned int* image_counter = (unsigned int*)w;
+    const MatchWs mw = match_ws(ws, B, sumG);
     // enough CTAs per image to fill the machine about once (5 CTAs/SM), never more than the image has tiles
     const int ntiles = (P + MTILE - 1) / MTILE;
     const int per_image = std::max(1, std::min(ntiles, (5 * 148) / B));
     dim3 grid(per_image, B);
     match_kernel<<<grid, MT, 0, st>>>((const float4*)gt_xyxy, gt_cls, gt_off, (const float4*)pri_xyxy, B, P, C - 1, pos_iou,
-                                      best_prior, npos, cls_u8, obj_idx, cls, best_key, tile_counter, npos_acc, image_counter);
+                                      best_prior, npos, cls_u8, obj_idx, cls, mw.best_key, mw.tile_counter, mw.npos_acc, mw.image_counter);
     count_launch();
     SSD_LAUNCH_CHECK();
     return 0;

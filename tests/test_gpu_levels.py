@@ -24,16 +24,25 @@ def _split(t, counts):
     return out
 
 
-@pytest.mark.parametrize("B", [3, 32, 256])
+@pytest.mark.parametrize("B", [3, 32, 256, 300])
 def test_loss_levels_equals_concatenated(B):
+    """B = 300 is more images than the 2 CTAs x 148 SMs of a B200 the mining kernel can hold co-resident: both routes
+    take the separate finaliser and the ordinary mining kernel (three launches instead of two)."""
+    from objectdetection_ssd_b200 import _lib
     from objectdetection_ssd_b200.head import PackedGT
     pri = H.priors()
     loc, conf, tb, tc = H.train_inputs(51, B, pri.shape[0])
     head = _head(pri)
     gt = PackedGT(tb, tc, head.dev)
     ref = head.loss(loc.cuda(), conf.cuda(), gt, with_grads=True)
-    lv = head.loss_levels(_split(loc.cuda(), SSD300_LEVELS), _split(conf.cuda(), SSD300_LEVELS), gt, with_grads=True)
+    loc_lv, conf_lv = _split(loc.cuda(), SSD300_LEVELS), _split(conf.cuda(), SSD300_LEVELS)
+    n0 = _lib.launch_count()
+    lv = head.loss_levels(loc_lv, conf_lv, gt, with_grads=True)
+    launches = _lib.launch_count() - n0
     torch.cuda.synchronize()
+    if B >= 256:
+        coresident = 2 * torch.cuda.get_device_properties(0).multi_processor_count   # 2 mining CTAs per SM
+        assert launches == (3 if B > coresident else 2), launches
     assert torch.equal(lv["losses"], ref["losses"]) and torch.equal(lv["sums"], ref["sums"])
     assert torch.equal(lv["npos"], ref["npos"]) and torch.equal(lv["cls_u8"], ref["cls_u8"])
     assert torch.equal(lv["best_prior"], ref["best_prior"])
