@@ -873,7 +873,11 @@ __device__ __forceinline__ void mine_body(const MineParams& p, const LevelTab* _
                 extra += (c_new != p.bg_class ? 1 : 0) - (c_nat != p.bg_class ? 1 : 0);
                 p.cls_rw[row0 + bp] = (uint8_t)c_new;
                 s_cls[bp] = (uint8_t)c_new;                  // a prior has one winner: no two threads patch the same entry
-                s_key[bp] = c_new != p.bg_class ? 0u : (__float_as_uint(p.ce[row0 + bp]) & 0x7fffffffu);
+                const uint32_t key = c_new != p.bg_class ? 0u : (__float_as_uint(p.ce[row0 + bp]) & 0x7fffffffu);
+                s_key[bp] = key;
+                // a gt labelled with the background class turns a positive into a negative: its key rises from 0 to
+                // its CE, which the histogram range (s_max) must cover - a NaN / inf key sends the image to the radix path
+                if (c_new == p.bg_class) atomicMax(&s_max, key);
                 if (p.obj_u16) p.obj_u16[row0 + bp] = (unsigned short)g;
             }
         }
@@ -904,8 +908,8 @@ __device__ __forceinline__ void mine_body(const MineParams& p, const LevelTab* _
     }
     const int* bprior = FIN ? p.best_prior_w : p.best_prior;
     __syncthreads();
-    kmax = s_max;                                            // (may be the key of a prior a forced match made positive:
-    LPHASE(2);                                               //  it only scales the histogram bins)
+    kmax = s_max;                                            // covers every key: the override folded in the keys it raised;
+    LPHASE(2);                                               // a key it lowered to 0 (made positive) only widens the bins
 
     // ---- 2. the k largest keys, ties to the lower prior index (T4): mark them with bit 31 ----
     const long long kk = (long long)p.neg_ratio * (long long)npos_b;
