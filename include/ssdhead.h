@@ -21,6 +21,12 @@
  *   - gt layout: boxes packed [sumG,4] fractional xyxy, classes [sumG] fp32 (Dataset.py:26),
  *     offsets int32 [B+1] (the cumsum of Losses.py:130).  Background class id = C-1
  *     (Losses.py:171).  Prior tables [P,4]: `pri_xyxy` and `pri_cxcywh` (Losses.py:6-7).
+ *   - `sumG` is a CAPACITY: the number of gt rows the packed arrays, best_prior and the match workspace have room
+ *     for.  It must be at least gt_off[B]; the rows past gt_off[B] are never read, and best_prior past gt_off[B] is
+ *     never written.  Every kernel finds an image's gts through gt_off only, read on the device, so a caller with
+ *     fixed buffers (a captured CUDA graph, or a context created with max_sumG) passes the capacity and lets the
+ *     count change from call to call.  Results do not depend on the capacity; it selects routes that give the same
+ *     bits (above 65 535 the steps do not record each prior's best gt, which costs time).
  *   - tie rules T1-T8 of SURVEY.md section 8.1 (repeated in DESIGN.md) are implemented exactly.
  */
 #ifndef SSDHEAD_H_

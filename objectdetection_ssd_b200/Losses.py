@@ -22,8 +22,8 @@ from . import Util as _U
 from .Util import (class_to_label, label_to_class, create_priors_ssd300, xywh_to_xyxy, xyxy_to_xywh,       # noqa: F401
                    gcxgcy_to_cxcy, get_offsets_coords, find_intersection, get_jaccard_tensor1,
                    get_jaccard_tensor11, map_prior_to_bb, subsampling)
-from .head import (MultiboxHead, PackedGT, multibox_loss, detect as _detect, multibox_loss_levels,
-                   detect_levels as _detect_levels)
+from .head import (MultiboxHead, PackedGT, StaticHead, multibox_loss, detect as _detect, multibox_loss_levels,  # noqa: F401
+                   detect_levels as _detect_levels, refuse_capture as _refuse_capture)
 from .priors import cxcywh_to_xyxy_host
 
 ancs_xywh = create_priors_ssd300()
@@ -57,7 +57,9 @@ def _dev_of(t):
 
 def ssd(outputs, tr_classes, tr_bboxs):
     """Batch multibox loss.  ``outputs`` = (loc [B,P,4], conf [B,P,21]); ``tr_classes`` / ``tr_bboxs`` = lists of
-    B tensors ([n_i] class ids, [n_i,4] fractional xyxy).  Returns (loc_loss, conf_loss)."""
+    B tensors ([n_i] class ids, [n_i,4] fractional xyxy).  Returns (loc_loss, conf_loss).  Not capturable into a CUDA
+    graph (it raises under capture): ``StaticHead`` is."""
+    _refuse_capture("ssd()")
     loc, conf = outputs
     head = _head(_dev_of(loc))
     _last.clear()
@@ -106,6 +108,7 @@ def ssd_levels(outputs, tr_classes, tr_bboxs):
     """``ssd`` on per-level head tensors (SURVEY.md 8(f) #3): ``outputs`` = (list of loc [B, n_l, 4], list of conf
     [B, n_l, 21]) - e.g. from ``head_levels`` - in the prior order of ``create_priors_ssd300``.  Same value and
     gradients as ``ssd(torch.cat(...))``, bit for bit, without ever building the concatenated tensors."""
+    _refuse_capture("ssd_levels()")
     locs, confs = outputs
     head = _head(_dev_of(confs[0]))
     _last.clear()
@@ -116,13 +119,16 @@ def ssd_levels(outputs, tr_classes, tr_bboxs):
 def inference_batch_levels(loc_levels, conf_levels, top_k=200, min_score=0.2, iou_threshold=0.45, img_wh=None,
                            max_candidates=0):
     """``inference_batch`` on per-level head tensors."""
+    _refuse_capture("inference_batch_levels()")
     return _detect_levels(_head(_dev_of(conf_levels[0])), list(loc_levels), list(conf_levels), min_score, iou_threshold,
                           top_k, img_wh, max_candidates)
 
 
 def inference_batch(loc, conf, top_k=200, min_score=0.2, iou_threshold=0.45, img_wh=None, max_candidates=0):
     """Batched detect front end (SURVEY.md 8(f) #2): loc [B,P,4], conf [B,P,21] -> dict of padded
-    [B,top_k,...] tensors + counts; ``img_wh`` [B,2] scales the boxes to pixels (Losses.py:87-89)."""
+    [B,top_k,...] tensors + counts; ``img_wh`` [B,2] scales the boxes to pixels (Losses.py:87-89).  Under CUDA graph
+    capture use ``StaticHead.detect``."""
+    _refuse_capture("inference_batch()")
     return _detect(_head(_dev_of(loc)), loc, conf, min_score, iou_threshold, top_k, img_wh, max_candidates)
 
 
@@ -142,6 +148,7 @@ def inference(l_, c_, index, top_k=200, phase='train', toDraw=True, min_score=0.
     """Single-image detect.  ``l_`` [P,4] predicted offsets, ``c_`` [P,21] logits.  Returns
     (pred_bboxes [K,4] pixel xyxy, classes int64 [K], probs [K]) with K <= top_k, or ([], [], []) when
     nothing passes ``min_score`` (Losses.py:62-63)."""
+    _refuse_capture("inference()")
     w, h = _image_size(phase, index)
     out = _detect(_head(_dev_of(l_)), l_.unsqueeze(0), c_.unsqueeze(0), min_score, iou_threshold, top_k,
                   torch.tensor([[float(w), float(h)]]), 0)

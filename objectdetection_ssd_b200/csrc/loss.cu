@@ -104,7 +104,7 @@ struct FusedMatch {
     int* npos_acc;
     unsigned short* obj_u16;     // nullable: natural best gt (local index) of every prior, for batches with many gts per image
     const float* seed_lb;        // batches with many gts per image (else nullptr): a lower bound of every gt's best IoU
-    int sumG;                    // (match_seed_kernel); a warp skips the gts that can neither make one of its priors positive
+    int sumG;                    // capacity of the gt arrays (match_seed_kernel's grid); a warp skips the gts that can neither make one of its priors positive
 };                               // nor be best matched by one of them
 
 // Everything the match of one row needs from global memory, fetched ONE TILE AHEAD so the two dependent L2 round trips
@@ -287,20 +287,22 @@ __device__ __forceinline__ void fused_match_rows(const FusedMatch& m, unsigned r
 // Batches with many gts per image: a lower bound of every gt's best IoU - its best IoU over every SEED_STRIDE-th prior.
 // One warp per gt.  The fused match then skips, per warp, the gts whose IoU with its priors cannot reach that bound.
 // The sampled priors are staged in shared memory once per CTA (every warp of the grid walks all of them); a warp then
-// takes gts in turn.
+// takes gts in turn.  The packed gt arrays may be longer than the batch (`sumG` is their capacity): the warps stop at
+// gt_off[B], read here, so a captured graph replays with whatever count the offsets hold.
 constexpr int SEED_STRIDE = 16;                              // (stress shape: stride 8 / 16 / 32 leaves 8.0 / 8.6 / 10.3 of 23.2 gts per warp to visit)
 constexpr int SEED_CAP = 65536;                              // gts of a batch the cull has seeds for (a fixed tail of the loss workspace:
                                                              // written before it is read, so it needs no cleaning)
 constexpr int SEED_MAX = 8192;                               // sampled priors held in shared memory (128 KB)
 __global__ void __launch_bounds__(256)
-match_seed_kernel(const float4* __restrict__ gt_xyxy, const float4* __restrict__ pri_xyxy, int sumG, int nsamp, int stride,
-                  float* __restrict__ seed_lb)
+match_seed_kernel(const float4* __restrict__ gt_xyxy, const int* __restrict__ gt_off, int B, const float4* __restrict__ pri_xyxy,
+                  int nsamp, int stride, float* __restrict__ seed_lb)
 {
     extern __shared__ __align__(16) float4 s_pri[];
     const int t = threadIdx.x, lane = t & 31;
+    const int n = gt_off[B];
     for (int i = t; i < nsamp; i += 256) s_pri[i] = pri_xyxy[(size_t)i * stride];
     __syncthreads();
-    for (int g = blockIdx.x * 8 + (t >> 5); g < sumG; g += gridDim.x * 8) {
+    for (int g = blockIdx.x * 8 + (t >> 5); g < n; g += gridDim.x * 8) {
         const float4 gb = gt_xyxy[g];
         const float ga = box_area(gb);
         float best = 0.0f;
@@ -1457,8 +1459,10 @@ static int launch_ce_stream(const float* conf, float* ce, float* grad_conf, floa
         const int nsamp = (fm.P + stride - 1) / stride;
         const size_t smem_seed = (size_t)nsamp * 16;
         SSD_CHECK_CUDA(cudaFuncSetAttribute(match_seed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_seed));
-        const int grid_seed = std::min((fm.sumG + 7) / 8, 2 * num_sms());
-        match_seed_kernel<<<grid_seed, 256, smem_seed, st>>>(fm.gt_xyxy, fm.pri_xyxy, fm.sumG, nsamp, stride, const_cast<float*>(fm.seed_lb));
+        const int grid_seed = std::min((fm.sumG + 7) / 8, 2 * num_sms());      // sized by the capacity
+        const int B = (int)(rows / fm.P);                                       // rows = B * P in every caller
+        match_seed_kernel<<<grid_seed, 256, smem_seed, st>>>(fm.gt_xyxy, fm.gt_off, B, fm.pri_xyxy, nsamp, stride,
+                                                             const_cast<float*>(fm.seed_lb));
         SSD_LAUNCH_CHECK();
         count_launch();
     }
@@ -1484,6 +1488,18 @@ static int launch_ce_stream(const float* conf, float* ce, float* grad_conf, floa
     return 0;
 }
 
+// Whether `st` is capturing into a graph (a failed query counts as capturing: the caller then takes the launch that
+// cannot be refused).
+static bool stream_capturing(cudaStream_t st)
+{
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    if (cudaStreamIsCapturing(st, &cs) != cudaSuccess) {
+        (void)cudaGetLastError();
+        return true;
+    }
+    return cs != cudaStreamCaptureStatusNone;
+}
+
 // A mining kernel on one CTA per image.  FIN: the forced-match finaliser is fused in, so every CTA must be co-resident
 // (they exchange the batch positive count through a counter) - a cooperative launch, which returns 1 (not an error)
 // when the grid does not fit.
@@ -1502,12 +1518,16 @@ static int launch_mine(void (*kmn)(KArgs...), int B, int P, cudaStream_t st, Arg
     if ((long long)per_sm * num_sms() < B) return 1;
     // cooperative (co-residency guaranteed) AND programmatic stream serialization (the grid may become resident while
     // the streaming kernel drains; it waits in pdl_wait()).  Runtimes that refuse the combination get the plain
-    // cooperative launch.
-    static bool with_pdl = true;
-    if (with_pdl) {
-        if (launch_pdl<true>(kmn, dim3(B), dim3(MN_T), smem_mn, st, args...) == cudaSuccess) { count_launch(); return 0; }
+    // cooperative launch.  The combination is first tried on an eager launch: a refused launch inside a stream capture
+    // would invalidate the capture, so a capture takes it only once an eager launch has shown it is accepted.
+    static int with_pdl = 0;                                 // 0: not tried yet, 1: accepted, -1: refused
+    const bool capturing = with_pdl >= 0 && stream_capturing(st);
+    if (with_pdl == 1 || (with_pdl == 0 && !capturing)) {
+        const cudaError_t e = launch_pdl<true>(kmn, dim3(B), dim3(MN_T), smem_mn, st, args...);
+        if (e == cudaSuccess) { with_pdl = 1; count_launch(); return 0; }
+        if (capturing) return (int)e;
         (void)cudaGetLastError();
-        with_pdl = false;
+        with_pdl = -1;
     }
     static_assert(std::is_same<std::tuple<std::decay_t<Args>...>, std::tuple<std::decay_t<KArgs>...>>::value,
                   "the cooperative launch passes the arguments by address: they must have the kernel's parameter types");

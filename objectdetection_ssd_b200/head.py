@@ -44,6 +44,15 @@ def require_cuda(dev) -> torch.device:
 _staging_pool = None     # pinned.StagingPool, created with the first host-list batch
 
 
+def refuse_capture(what: str) -> None:
+    """Raise if the current stream is capturing a CUDA graph: ``what`` packs its gts from host values and shares
+    workspaces between calls, so a graph of it would replay stale gts or write into freed memory."""
+    if torch.cuda.is_available() and torch.cuda.is_current_stream_capturing():
+        raise RuntimeError(f"{what} cannot be captured into a CUDA graph (it reads its gt count on the host and shares "
+                           "its workspaces); use objectdetection_ssd_b200.Losses.StaticHead: load() the gts before "
+                           "each replay, capture StaticHead.loss / loss_levels / detect")
+
+
 class PackedGT:
     """Ragged gt lists packed once: boxes [sumG,4] f32, classes [sumG] f32, offsets int32 [B+1]
     (host-side equivalent of Losses.py:129-130; no per-image synchronisation).
@@ -53,6 +62,7 @@ class PackedGT:
     page-locked block that then crosses to the device in one copy, offsets included."""
 
     def __init__(self, boxes: Sequence[torch.Tensor], classes: Sequence[torch.Tensor], dev: torch.device):
+        refuse_capture("PackedGT")
         try:
             counts = [b.shape[0] for b in boxes]
         except IndexError:                       # a 0-dim entry: no box
@@ -120,17 +130,22 @@ class PackedGT:
         return self._off_np.tolist()
 
     def _fill_staging(self, st, boxes, classes):
-        if getattr(st, "boxes_t", None) is None:                    # torch views of the pinned arrays, made once per block
-            st.boxes_t = torch.from_numpy(st.boxes)
-            st.classes_t = torch.from_numpy(st.classes)
-            st.offsets_t = torch.from_numpy(st.offsets)
-            st.raw_t = torch.from_numpy(st.raw)
+        _staging_views(st)
         n = self.sumG
         # one concatenation per list, then one small copy into the block (copy_ converts int64 class ids and checks the
         # shapes: [n,4] boxes, [n] classes)
         st.boxes_t[:n].copy_(self._cat(boxes, 4))
         st.classes_t[:n].copy_(self._cat(classes, 0))
         st.offsets[:] = self._off_np
+
+
+def _staging_views(st):
+    """torch views of a staging block's pinned arrays, made once per block."""
+    if getattr(st, "boxes_t", None) is None:
+        st.boxes_t = torch.from_numpy(st.boxes)
+        st.classes_t = torch.from_numpy(st.classes)
+        st.offsets_t = torch.from_numpy(st.offsets)
+        st.raw_t = torch.from_numpy(st.raw)
 
 
 class MultiboxHead:
@@ -503,3 +518,181 @@ def detect_levels(head: MultiboxHead, loc_levels, conf_levels, min_score=0.2, io
         _ptr(ws), ws.numel(), _stream(dev)), "ssdhead_detect_levels")
     return out
 
+
+
+# ---------------------------------------------------------------------------------------------- CUDA graph capture
+class _FixedWorkspaces(MultiboxHead):
+    """A MultiboxHead whose workspaces are allocated and zero-filled by the first call that needs each of them, outside
+    any capture, and then never resized, moved or re-zeroed: a captured graph keeps pointing at them, and the kernels
+    leave every counter zeroed again.  Its callers keep the batch size and the gt capacity fixed, so each workspace has
+    one size."""
+
+    def _workspace(self, which: int, B: int, n: int) -> torch.Tensor:
+        cur = self._ws.get(which)
+        if cur is None:
+            if torch.cuda.is_current_stream_capturing():
+                raise RuntimeError("StaticHead: the first loss / loss_levels / detect call allocates and zero-fills its "
+                                   "workspace and cannot be captured; make one eager call of it first (a warm-up step)")
+            need = int(self.lib.ssdhead_workspace_bytes(which, B, self.P, self.C, n))
+            if need == 0:
+                raise RuntimeError(f"ssdhead: unsupported shape for this entry point (B={B}, P={self.P}, C={self.C})")
+            cur = torch.zeros(need, dtype=torch.uint8, device=self.dev)
+            self._ws[which] = cur
+        return cur
+
+
+class _StaticGT:
+    """Device gt buffers of fixed capacity in the ``pinned.gt_layout`` layout; ``sumG`` is the capacity (the kernels
+    read the count from ``off[B]``)."""
+
+    def __init__(self, B: int, capacity: int, dev: torch.device):
+        from .pinned import gt_layout
+        o0, o1, o2, total = gt_layout(capacity, B)
+        self.B, self.sumG = B, capacity
+        self.block = torch.zeros(total, dtype=torch.uint8, device=dev)
+        self.boxes = self.block[o0:o0 + capacity * 16].view(torch.float32).view(capacity, 4)
+        self.classes = self.block[o1:o1 + capacity * 4].view(torch.float32)
+        self.off = self.block[o2:o2 + (B + 1) * 4].view(torch.int32)
+
+
+class StaticHead:
+    """The training-head step and detect of one fixed batch size, in a form that can be captured into a CUDA graph.
+
+    It owns its device gt buffers (room for ``max_gt`` gts of ``batch`` images) and its workspaces, so a graph captured
+    around ``loss`` / ``loss_levels`` (with ``backward()``) or ``detect`` stays valid: the kernels read the gt count
+    from the offsets on the device.  Before each replay, ``load`` or ``load_packed`` writes the next batch's gts into
+    the buffers, in stream order on the current stream; both refuse to run under capture.  The first call of
+    ``loss`` / ``loss_levels`` / ``detect`` allocates its workspace and must be eager (a warm-up step).  One graph per
+    object: two graphs of one object would share its gt buffers and workspaces.
+
+        sh = StaticHead(priors, batch=32, max_gt=32 * 64, device="cuda")
+        sh.load(boxes, classes); l, c = sh.loss(loc, conf); (l + c).backward()      # warm-up, eager
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
+            l, c = sh.loss(loc, conf); (l + c).backward()
+        for boxes, classes in batches:
+            sh.load(boxes, classes)            # or sh.load_packed(*collate.collate_gt(...))
+            loc.copy_(...); conf.copy_(...); g.replay()
+    """
+
+    def __init__(self, priors: torch.Tensor, batch: int, max_gt: int, device=None, num_classes: int = 21):
+        if torch.cuda.is_available() and torch.cuda.is_current_stream_capturing():
+            raise RuntimeError("StaticHead: create it before capturing (it allocates its buffers)")
+        self.B, self.max_gt = int(batch), int(max_gt)
+        if self.B < 1 or self.max_gt < self.B:
+            raise ValueError(f"StaticHead: batch must be >= 1 and max_gt >= batch (every image has a gt), got "
+                             f"batch={batch}, max_gt={max_gt}")
+        self.head = _FixedWorkspaces(priors, device, num_classes)
+        self.dev = self.head.dev
+        self.gt = _StaticGT(self.B, self.max_gt, self.dev)
+        from .pinned import StagingPool
+        self._pool = StagingPool()
+        self._loaded = False
+
+    # ------------------------------------------------------------------ gts, outside the graph
+    def _refuse_capture(self, what: str) -> None:
+        if torch.cuda.is_current_stream_capturing():
+            raise RuntimeError(f"StaticHead.{what}() cannot be captured: call it before each replay, outside the graph")
+
+    def _offsets(self, counts) -> np.ndarray:
+        if len(counts) != self.B:
+            raise ValueError(f"StaticHead holds {self.B} images, got {len(counts)}")
+        bad = [i for i, n in enumerate(counts) if n <= 0]
+        if bad:
+            # the reference fails the same way on an image without objects (Losses.py:153, max over an empty dim)
+            raise IndexError(f"image {bad[0]} has no ground-truth box: max() over an empty dimension")
+        offs = np.zeros(self.B + 1, dtype=np.int32)
+        np.cumsum(counts, out=offs[1:])
+        if int(offs[-1]) > self.max_gt:
+            raise ValueError(f"StaticHead: {int(offs[-1])} gts, more than max_gt = {self.max_gt}")
+        return offs
+
+    def _upload(self, st) -> None:
+        """One copy of the whole staging block into the device buffers; the block returns to the pool behind an event."""
+        cur = torch.cuda.current_stream(self.dev)
+        self.gt.block.copy_(st.raw_t, non_blocking=True)
+        if st.event is None:
+            st.event = torch.cuda.Event()
+        st.event.record(cur)
+        self._pool.release(st, st.event)
+        self._loaded = True
+
+    def load(self, boxes: Sequence[torch.Tensor], classes: Sequence[torch.Tensor]) -> None:
+        """Ragged gt lists (``ssd()``'s ``tr_bboxs`` / ``tr_classes``: B tensors of [n_i, 4] fractional xyxy and [n_i]
+        class ids), on the host or on the device, into the device buffers."""
+        self._refuse_capture("load")
+        if len(classes) != len(boxes):
+            raise ValueError(f"{len(boxes)} box lists but {len(classes)} class lists")
+        offs = self._offsets([b.shape[0] if b.dim() > 0 else 0 for b in boxes])
+        n = int(offs[-1])
+        bx, cl = PackedGT._cat(boxes, 4), PackedGT._cat(classes, 0)
+        if tuple(bx.shape) != (n, 4) or tuple(cl.shape) != (n,):
+            raise ValueError(f"gt lists disagree: boxes {tuple(bx.shape)}, classes {tuple(cl.shape)}, {n} gts expected")
+        if bx.device.type == "cpu" and cl.device.type == "cpu":
+            st = self._pool.acquire(self.max_gt, self.B, exact=True)
+            _staging_views(st)
+            st.boxes_t[:n].copy_(bx)
+            st.classes_t[:n].copy_(cl)
+            st.offsets[:] = offs
+            self._upload(st)
+            return
+        self.gt.boxes[:n].copy_(bx, non_blocking=True)
+        self.gt.classes[:n].copy_(cl, non_blocking=True)
+        self.gt.off.copy_(torch.from_numpy(offs).pin_memory(), non_blocking=True)
+        self._loaded = True
+
+    def load_packed(self, gt_xyxy, gt_cls, gt_off) -> None:
+        """The packed layout of ``collate.collate_gt`` (boxes [n,4], classes [n], offsets int32 [B+1]): numpy arrays or
+        tensors, on the host or on the device (device offsets are read back to check them: one synchronisation)."""
+        self._refuse_capture("load_packed")
+        off = gt_off.detach().cpu().numpy() if isinstance(gt_off, torch.Tensor) else np.asarray(gt_off)
+        off = off.astype(np.int64).reshape(-1)
+        if off.shape[0] != self.B + 1 or off[0] != 0:
+            raise ValueError(f"StaticHead: expected {self.B + 1} offsets starting at 0, got {off.shape[0]}")
+        offs = self._offsets(np.diff(off))
+        n = int(offs[-1])
+        if gt_xyxy.shape[0] < n or gt_cls.shape[0] < n:
+            raise ValueError(f"StaticHead: the offsets list {n} gts, the arrays hold {gt_xyxy.shape[0]} boxes and "
+                             f"{gt_cls.shape[0]} classes")
+        if not any(isinstance(t, torch.Tensor) and t.is_cuda for t in (gt_xyxy, gt_cls)):
+            st = self._pool.acquire(self.max_gt, self.B, exact=True)
+            _staging_views(st)
+            as_np = lambda a: a.detach().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+            st.boxes[:n] = as_np(gt_xyxy)[:n].reshape(n, 4)
+            st.classes[:n] = as_np(gt_cls)[:n].reshape(n)
+            st.offsets[:] = offs
+            self._upload(st)
+            return
+        as_t = lambda a: a if isinstance(a, torch.Tensor) else torch.from_numpy(np.asarray(a))
+        self.gt.boxes[:n].copy_(as_t(gt_xyxy)[:n].reshape(n, 4), non_blocking=True)
+        self.gt.classes[:n].copy_(as_t(gt_cls)[:n].reshape(n), non_blocking=True)
+        self.gt.off.copy_(torch.from_numpy(offs).pin_memory(), non_blocking=True)
+        self._loaded = True
+
+    # ------------------------------------------------------------------ capturable calls
+    def _require_loaded(self) -> None:
+        if not self._loaded:
+            raise RuntimeError("StaticHead: load() or load_packed() the gts before the first loss call")
+
+    def loss(self, loc: torch.Tensor, conf: torch.Tensor, neg_ratio: int = NEG_RATIO, pos_iou: float = POS_IOU):
+        """(loc_loss, conf_loss) as 0-dim tensors with grad_fn, as ``ssd()`` returns them, on the loaded gts."""
+        self._require_loaded()
+        need = torch.is_grad_enabled() and (loc.requires_grad or conf.requires_grad)
+        return _MultiboxLossFn.apply(loc, conf, self.head, self.gt, neg_ratio, pos_iou, None, need)
+
+    def loss_levels(self, loc_levels, conf_levels, neg_ratio: int = NEG_RATIO, pos_iou: float = POS_IOU):
+        """``loss`` on per-level head tensors, as ``ssd_levels()``."""
+        self._require_loaded()
+        L = len(conf_levels)
+        need = torch.is_grad_enabled() and any(t.requires_grad for t in list(loc_levels) + list(conf_levels))
+        return _MultiboxLossLevelsFn.apply(self.head, self.gt, neg_ratio, pos_iou, L, need, *loc_levels, *conf_levels)
+
+    def detect(self, loc: torch.Tensor, conf: torch.Tensor, min_score: float = 0.2, iou_thr: float = 0.45,
+               top_k: int = 200, img_wh: Optional[torch.Tensor] = None):
+        """The ``inference_batch`` dict (boxes, prob, cls, prior, cnt).  ``img_wh`` [B,2], if given, must already be on
+        this device: a host copy cannot be captured."""
+        if int(loc.shape[0]) != self.B:
+            raise ValueError(f"StaticHead holds {self.B} images, got a batch of {int(loc.shape[0])}")
+        if img_wh is not None and (not isinstance(img_wh, torch.Tensor) or img_wh.device != self.dev):
+            raise ValueError(f"StaticHead.detect: img_wh must be a tensor on {self.dev} (a host copy cannot be captured)")
+        return _detect(self.head, loc, conf, min_score, iou_thr, top_k, img_wh, 0, False)

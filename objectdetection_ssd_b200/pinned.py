@@ -87,20 +87,24 @@ class StagingPool:
         self.free: List[Staging] = []
         self.max_free = max_free
 
-    def acquire(self, capacity: int, B: int) -> Staging:
+    def acquire(self, capacity: int, B: int, exact: bool = False) -> Staging:
+        """A block for ``capacity`` gts of ``B`` images.  ``exact``: exactly that capacity, so the block has the layout
+        of a device buffer made with ``gt_layout(capacity, B)`` and goes up in one copy."""
+        def fits(s):
+            return s.B == B and (s.capacity == capacity if exact else s.capacity >= capacity)
         best: Optional[int] = None
         for i, s in enumerate(self.free):
-            if s.capacity >= capacity and s.B == B and (s.event is None or s.event.query()):
+            if fits(s) and (s.event is None or s.event.query()):
                 if best is None or s.capacity < self.free[best].capacity:
                     best = i
         if best is not None:
             return self.free.pop(best)
         for i, s in enumerate(self.free):      # everything of this shape is still in flight: wait for the oldest
-            if s.capacity >= capacity and s.B == B and len(self.free) >= self.max_free:
+            if fits(s) and len(self.free) >= self.max_free:
                 s = self.free.pop(i)
                 s.event.synchronize()
                 return s
-        cap = max(64, 1 << (max(capacity, 1) - 1).bit_length())       # round up: ragged batches reuse one block
+        cap = capacity if exact else max(64, 1 << (max(capacity, 1) - 1).bit_length())   # round up: ragged batches reuse one block
         return Staging(cap, B)
 
     def release(self, s: Staging, event) -> None:
