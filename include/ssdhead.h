@@ -283,7 +283,9 @@ int ssdhead_detect(const float* loc_dev, const float* conf_dev, const float* pri
                    int32_t* out_cnt_dev, void* ws_dev, size_t ws_bytes, void* stream);
 
 /* Stage-isolated twin of ssdhead_detect taking decoded boxes [B,P,4] (cxcywh) and class
- * probabilities [B,P,C] as given (the oracle's), so keep lists can be compared bit-exactly. */
+ * probabilities [B,P,C] as given (the oracle's), so keep lists can be compared bit-exactly.
+ * Any finite or infinite score ranks as the reference's descending sort ranks it: -0.0 ties with
+ * +0.0 (and is reported as +0.0), negative scores rank below zero, scores above 1 above 1.0. */
 int ssdhead_detect_from_scores(const float* boxes_cxcywh_dev, const float* probs_dev,
                                int B, int P, int C, float min_score, float iou_thr, int top_k,
                                const float* img_wh_dev, int max_candidates,

@@ -111,10 +111,10 @@ size_t detect_workspace_bytes(int B, int P, int C, int n)
     return detect_ws_layout(B, P, C, n, nullptr, nullptr);
 }
 
-// key = prob bits << 32 | ~(class << 24 | prior): descending key order = descending prob, then lower class, then
-// lower prior (T5, T7)
-__device__ __forceinline__ unsigned long long make_key(float prob, int cls, int prior) {
-    return ((unsigned long long)__float_as_uint(prob) << 32) | (unsigned long long)(0xffffffffu - (((unsigned)cls << 24) | (unsigned)prior));
+// key = score word << 32 | ~(class << 24 | prior): descending key order = descending prob, then lower class, then
+// lower prior (T5, T7).  The score word is the probability's bits (score_word below).
+__device__ __forceinline__ unsigned long long make_key(unsigned word, int cls, int prior) {
+    return ((unsigned long long)word << 32) | (unsigned long long)(0xffffffffu - (((unsigned)cls << 24) | (unsigned)prior));
 }
 __device__ __forceinline__ int key_cls(unsigned long long key) { return (int)((0xffffffffu - (unsigned)(key & 0xffffffffull)) >> 24); }
 __device__ __forceinline__ unsigned key_prior(unsigned long long key) { return (0xffffffffu - (unsigned)(key & 0xffffffffull)) & 0xffffffu; }
@@ -123,6 +123,21 @@ __device__ __forceinline__ unsigned key_prior(unsigned long long key) { return (
 __device__ __forceinline__ int coarse_rank(unsigned pbits) {
     const int d = (int)(0x3f800000u >> 18) - (int)(pbits >> 18);
     return min(CBINS - 1, max(0, d));
+}
+// The score word of a key (its upper 32 bits).  A softmax probability is >= +0, so its bits already order it.  The scores
+// given to ssdhead_detect_from_scores can be anything: -0.0 must tie with +0.0 and a negative score rank below both (as in
+// the reference's descending sort), so there the word is the order-preserving map of common.cuh (-0 -> +0, non-negative
+// scores -> bits | 2^31, negative ones -> ~bits).  SCORE_TOP is what the word of 0x3f800000 (1.0) becomes.
+template <bool FROM_SCORES> __device__ __forceinline__ unsigned score_word(float p) {
+    return FROM_SCORES ? float_order_key(p) : __float_as_uint(p);
+}
+template <bool FROM_SCORES> __device__ __forceinline__ float word_score(unsigned w) {
+    return __uint_as_float(!FROM_SCORES ? w : (w & 0x80000000u) ? (w ^ 0x80000000u) : ~w);
+}
+template <bool FROM_SCORES> constexpr unsigned SCORE_TOP = FROM_SCORES ? 0x80000000u : 0u;
+// coarse rank bin of a score word; negative given scores fall into the last bin
+template <bool FROM_SCORES> __device__ __forceinline__ int coarse_rank_w(unsigned w) {
+    return !FROM_SCORES ? coarse_rank(w) : (w & 0x80000000u) ? coarse_rank(w ^ 0x80000000u) : CBINS - 1;
 }
 
 // Head outputs given per pyramid level (ssdhead_detect_levels; see ssdhead.h): level l holds cnt[l] priors per image,
@@ -296,7 +311,7 @@ detect_score_body(const int b, const int tile, const int T, uint64_t* s_bar_p, c
     for (unsigned j = lane; j < wtotal; j += 32) {
         const unsigned lq = st_q[j];
         const float pj = wrow[(lq >> 5) * C + (lq & 31u)];
-        atomicAdd(&s_ch[coarse_rank(__float_as_uint(pj))], 1u);
+        atomicAdd(&s_ch[coarse_rank_w<FROM_SCORES>(score_word<FROM_SCORES>(pj))], 1u);
     }
     __syncthreads();
     // exclusive prefix sums over the 256 rank bins: the chunk is written ordered by bin, highest probabilities first,
@@ -333,8 +348,9 @@ detect_score_body(const int b, const int tile, const int T, uint64_t* s_bar_p, c
         for (unsigned j = lane; j < wtotal; j += 32) {
             const unsigned lq = st_q[j];
             const float pj = wrow[(lq >> 5) * C + (lq & 31u)];
-            const int rb = coarse_rank(__float_as_uint(pj));
-            seg[s_ch[rb] + atomicAdd(&s_fill[rb], 1u)] = make_key(pj, (int)(lq & 31u), r0 + warp * 32 + (int)(lq >> 5));
+            const unsigned w = score_word<FROM_SCORES>(pj);
+            const int rb = coarse_rank_w<FROM_SCORES>(w);
+            seg[s_ch[rb] + atomicAdd(&s_fill[rb], 1u)] = make_key(w, (int)(lq & 31u), r0 + warp * 32 + (int)(lq >> 5));
         }
     }
 }
@@ -469,7 +485,7 @@ sample_floor(const int b, const float* __restrict__ conf, int P, float min_score
 #pragma unroll
             for (int q = 0; q < NF; ++q) {
                 const float p = FROM_SCORES ? e[q] : __fmul_rn(e[q], inv);
-                if (p >= min_score) atomicAdd(&s_h[coarse_rank(__float_as_uint(p))], 1u);
+                if (p >= min_score) atomicAdd(&s_h[coarse_rank_w<FROM_SCORES>(score_word<FROM_SCORES>(p))], 1u);
             }
         }
     }
@@ -1066,7 +1082,7 @@ detect_nms_body(const int b, const FloorArgs fl, const ItemLayout il,
 #pragma unroll
             for (int u = 0; u < 4; ++u)
                 if (f0 + u * NT + t < fl_n) {
-                    atomicAdd(&s_col[coarse_rank((unsigned)(kk[u] >> 32))], 1u);
+                    atomicAdd(&s_col[coarse_rank_w<FROM_SCORES>((unsigned)(kk[u] >> 32))], 1u);
                     if (fl_parked) s_buf_b[f0 + u * NT + t] = kk[u];     // the first slice is picked out of shared memory
                 }
         }
@@ -1141,9 +1157,10 @@ detect_nms_body(const int b, const FloorArgs fl, const ItemLayout il,
         // key bounds of the slice from its coarse bins (the open-ended last bin has none: the sort measures them)
         const bool pre = rc1 < CBINS;
         const unsigned top18 = 0x3f800000u >> 18;
-        const unsigned long long kmax0 = rc0 == 0 ? (0x3f800000ull << 32 | 0xffffffffull)
-                                                  : ((unsigned long long)((top18 - rc0 + 1) << 18) << 32) - 1ull;
-        const unsigned long long kmin0 = pre ? (unsigned long long)((top18 - (rc1 - 1)) << 18) << 32 : 0ull;
+        constexpr unsigned long long top = SCORE_TOP<FROM_SCORES>;
+        const unsigned long long kmax0 = rc0 == 0 ? ((0x3f800000ull + top) << 32 | 0xffffffffull)
+                                                  : (((unsigned long long)((top18 - rc0 + 1) << 18) + top) << 32) - 1ull;
+        const unsigned long long kmin0 = pre ? ((unsigned long long)((top18 - (rc1 - 1)) << 18) + top) << 32 : 0ull;
         const BinMap bin0(kmin0, kmax0);
         if (pre) for (int i = t; i < FBINS; i += NT) s_cnt[i] = 0u;
         if (FLOOR) {
@@ -1153,7 +1170,7 @@ detect_nms_body(const int b, const FloorArgs fl, const ItemLayout il,
             if (fl_parked) {
                 for (int f = t; f < fl_n; f += NT) {
                     const unsigned long long k = s_buf_b[f];
-                    const int r = coarse_rank((unsigned)(k >> 32));
+                    const int r = coarse_rank_w<FROM_SCORES>((unsigned)(k >> 32));
                     if (r >= rc0 && r < rc1) {
                         X[atomicAdd(&s_gcnt, 1u)] = k;
                         if (pre) atomicAdd(&s_cnt[bin0(k)], 1u);
@@ -1178,7 +1195,7 @@ detect_nms_body(const int b, const FloorArgs fl, const ItemLayout il,
 #pragma unroll
                 for (int u = 0; u < 4; ++u) {
                     if (f0 + u * NT + t >= fl_n) continue;
-                    const int r = coarse_rank((unsigned)(kk[u] >> 32));
+                    const int r = coarse_rank_w<FROM_SCORES>((unsigned)(kk[u] >> 32));
                     if (r >= rc0 && r < rc1) {
                         X[atomicAdd(&s_gcnt, 1u)] = kk[u];
                         if (pre) atomicAdd(&s_cnt[bin0(kk[u])], 1u);
@@ -1242,7 +1259,7 @@ detect_nms_body(const int b, const FloorArgs fl, const ItemLayout il,
         const unsigned long long key = s_kkey[i];
         const float4 v = s_kbox[i];
         ob[slot] = img_wh ? make_float4(__fmul_rn(v.x, sx), __fmul_rn(v.y, sy), __fmul_rn(v.z, sx), __fmul_rn(v.w, sy)) : v;   // Losses.py:89
-        op[slot] = __uint_as_float((unsigned)(key >> 32));
+        op[slot] = word_score<FROM_SCORES>((unsigned)(key >> 32));
         oc[slot] = key_cls(key);
         if (oi) oi[slot] = (int)key_prior(key);
     };
@@ -1345,7 +1362,7 @@ score_rows(Ptr x, const bool valid, const float F, const int prior, unsigned int
         do {
             const int q = __ffs(cmask) - 1;
             cmask &= cmask - 1u;
-            *seg++ = make_key(prob_again<FROM_SCORES>(x, q, m, inv), q, prior);
+            *seg++ = make_key(score_word<FROM_SCORES>(prob_again<FROM_SCORES>(x, q, m, inv)), q, prior);
         } while (cmask);
     }
 }
