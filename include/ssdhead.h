@@ -169,8 +169,9 @@ int ssdhead_multibox_step(const float* loc_dev, const float* conf_dev,
  * `peers_dev`: device table of R pointers to the ranks' exchange buffers (ssdhead_xchg_bytes() each, zero-filled
  * once, mapped into this process with cudaIpcOpenMemHandle; entry `rank` is xchg_local_dev).  `seq` >= 1 is a step
  * counter every rank advances in lock step.  sums/losses come back GLOBAL, npos[B] is this rank's own count,
- * *err_flag_dev is set if a (10 s bounded) wait for a peer expired.  B must fit co-resident (else E_UNSUPPORTED:
- * use ssdhead_ce_match_stream + an all-reduce + ssdhead_mine). */
+ * *err_flag_dev is set if a (10 s bounded) wait for a peer expired.  B must fit co-resident (else E_UNSUPPORTED,
+ * returned before anything is launched, the workspaces and gradients untouched: use ssdhead_ce_match_stream + an
+ * all-reduce + ssdhead_mine).  The same holds for the per-level and resident steps with R > 1. */
 int ssdhead_multibox_step_sharded(const float* loc_dev, const float* conf_dev,
                           const float* gt_xyxy_dev, const float* gt_cls_dev, const int32_t* gt_off_dev,
                           const float* pri_xyxy_dev, const float* pri_cxcywh_dev,

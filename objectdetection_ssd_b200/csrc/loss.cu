@@ -1500,6 +1500,19 @@ static bool stream_capturing(cudaStream_t st)
     return cs != cudaStreamCaptureStatusNone;
 }
 
+// Whether a grid of B CTAs of the mining kernel kmn can be co-resident (*fits); the kernel's dynamic shared memory limit
+// is raised first, as its launch needs and the occupancy query reads it.
+template <typename... KArgs>
+static int mine_fits_coresident(void (*kmn)(KArgs...), int B, int P, bool* fits)
+{
+    const size_t smem_mn = mine_smem_bytes(P);
+    SSD_CHECK_CUDA(cudaFuncSetAttribute(kmn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_mn));
+    int per_sm = 0;
+    SSD_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kmn, MN_T, smem_mn));
+    *fits = (long long)per_sm * num_sms() >= B;
+    return 0;
+}
+
 // A mining kernel on one CTA per image.  FIN: the forced-match finaliser is fused in, so every CTA must be co-resident
 // (they exchange the batch positive count through a counter) - a cooperative launch, which returns 1 (not an error)
 // when the grid does not fit.
@@ -1507,15 +1520,15 @@ template <bool FIN, typename... KArgs, typename... Args>
 static int launch_mine(void (*kmn)(KArgs...), int B, int P, cudaStream_t st, Args... args)
 {
     const size_t smem_mn = mine_smem_bytes(P);
-    SSD_CHECK_CUDA(cudaFuncSetAttribute(kmn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_mn));
     if (!FIN) {
+        SSD_CHECK_CUDA(cudaFuncSetAttribute(kmn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_mn));
         SSD_CHECK_CUDA(launch_pdl(kmn, dim3(B), dim3(MN_T), smem_mn, st, args...));
         count_launch();
         return 0;
     }
-    int per_sm = 0;
-    SSD_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kmn, MN_T, smem_mn));
-    if ((long long)per_sm * num_sms() < B) return 1;
+    bool fits = false;
+    const int rc = mine_fits_coresident(kmn, B, P, &fits);
+    if (rc || !fits) return rc ? rc : 1;
     // cooperative (co-residency guaranteed) AND programmatic stream serialization (the grid may become resident while
     // the streaming kernel drains; it waits in pdl_wait()).  Runtimes that refuse the combination get the plain
     // cooperative launch.  The combination is first tried on an eager launch: a refused launch inside a stream capture
@@ -1732,6 +1745,17 @@ static int step_impl(const StepArgs& a, const LevelTab* lv, const Xchg& x, void*
     }
     if (lv) prm.ce_w = lw.ce;
     const bool grads = lv ? lv->gconf[0] != nullptr : a.grad_loc != nullptr;
+    if (x.R > 1) {
+        // a sharded batch has no three-kernel fallback (its peer exchange needs the co-resident grid): one that does not
+        // fit is refused here, before the streaming kernel adds into the match workspace or writes any gradient
+        bool fits = false;
+        const int frc = lv ? (grads ? mine_fits_coresident(mine_levels_kernel<21, true, true>, a.B, a.P, &fits)
+                                    : mine_fits_coresident(mine_levels_kernel<21, false, true>, a.B, a.P, &fits))
+                           : (grads ? mine_fits_coresident(mine_kernel<21, true, true>, a.B, a.P, &fits)
+                                    : mine_fits_coresident(mine_kernel<21, false, true>, a.B, a.P, &fits));
+        if (frc) return frc;
+        if (!fits) return SSDHEAD_E_UNSUPPORTED;
+    }
     const bool ce_grads = grads && !ws_rows;
     const long long rows = (long long)a.B * a.P;
     float* ce = a.ce ? a.ce : lw.ce;

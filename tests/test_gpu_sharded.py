@@ -76,6 +76,34 @@ def _worker(rank, world, port, q):
         assert not ctx.xchg_error()
         assert torch.equal(losses_lv, losses) and torch.equal(sums_lv, sums), (losses_lv, losses)
         assert torch.equal(torch.cat([k[2] for k in keep], 1), gl) and torch.equal(torch.cat([k[3] for k in keep], 1), gcf)
+        # --- the host-buffer steps on the same exchange (xchg_npos_kernel, sum_chunks_xchg_kernel): dense gradients
+        # into page-locked and into pageable buffers, then packed rows scattered back to dense
+        from objectdetection_ssd_b200.ctx import SparseRows
+        from objectdetection_ssd_b200.pinned import pinned_empty
+        host = {}
+        for pinned in (True, False):
+            alloc = pinned_empty if pinned else (lambda shape, dt=np.float32: np.empty(shape, dt))
+            hl, hc = alloc(tl.shape), alloc(tc.shape)
+            hl[...] = loc[lo:hi]
+            hc[...] = conf[lo:hi]
+            hgl, hgc = alloc(tl.shape), alloc(tc.shape)
+            lh = ctx.loss_host(hl, hc, gx, gcl, off, hgl, hgc)
+            host["pinned" if pinned else "pageable"] = (np.array(lh, np.float32), hgl.copy(), hgc.copy())
+        rows = SparseRows(B, cap=4096)
+        ls = ctx.loss_host_sparse(np.ascontiguousarray(loc[lo:hi]), np.ascontiguousarray(conf[lo:hi]), gx, gcl, off, rows)
+        sgl, sgc = rows.scatter(P)
+        host["sparse"] = (np.array(ls, np.float32), sgl, sgc)
+        assert not ctx.xchg_error()
+        # --- three steps with resident gradient tensors, the first one fresh
+        rgl, rgc = torch.empty_like(tl), torch.empty_like(tc)
+        sums_res, losses_res = torch.empty(2, dtype=torch.float64, device=dev), torch.empty(2, device=dev)
+        for i in range(3):
+            ctx.loss_dev_resident(tl.data_ptr(), tc.data_ptr(), tgx.data_ptr(), tgc.data_ptr(), toff.data_ptr(), B,
+                                  int(off[-1]), sums_res.data_ptr(), losses_res.data_ptr(), rgl.data_ptr(), rgc.data_ptr(), st,
+                                  fresh=(i == 0))
+        torch.cuda.synchronize()
+        assert not ctx.xchg_error()
+        host["resident"] = (losses_res.cpu().numpy(), rgl.cpu().numpy(), rgc.cpu().numpy())
         # --- NCCL route through the drop-in surface
         head = MultiboxHead(pri, dev)
         l2 = tl.clone().requires_grad_(True)
@@ -85,7 +113,7 @@ def _worker(rank, world, port, q):
         (a + b).backward()
         torch.cuda.synchronize()
         q.put((rank, lo, hi, losses.cpu().numpy(), sums.cpu().numpy(), gl.cpu().numpy(), gcf.cpu().numpy(),
-               np.array([a.item(), b.item()]), l2.grad.cpu().numpy(), c2.grad.cpu().numpy()))
+               np.array([a.item(), b.item()]), l2.grad.cpu().numpy(), c2.grad.cpu().numpy(), host))
         ctx.close()
     finally:
         dist.destroy_process_group()
@@ -117,11 +145,18 @@ def test_two_gpu_sharded_step_equals_full_batch():
     ref = O.multibox_loss(torch.from_numpy(loc), torch.from_numpy(conf), tb, tc, pri)
     fl = full["losses"].cpu().numpy()
     assert abs(fl[0] - ref["loc_loss"].item()) <= 1e-5 * ref["loc_loss"].item()
-    for rank, lo, hi, losses, sums, gl, gcf, nccl_losses, ngl, ngc in res:
+    for rank, lo, hi, losses, sums, gl, gcf, nccl_losses, ngl, ngc, host in res:
         assert np.allclose(losses, fl, rtol=1e-6), (rank, losses, fl)                     # global losses on every rank
         assert np.allclose(sums, full["sums"].cpu().numpy(), rtol=1e-9)
         assert np.array_equal(gcf, full["grad_conf"][lo:hi].cpu().numpy())                # exact gradient slices
         assert np.array_equal(gl, full["grad_loc"][lo:hi].cpu().numpy())
         assert np.allclose(nccl_losses, fl, rtol=1e-6)
         assert np.array_equal(ngc, gcf) and np.array_equal(ngl, gl)
+        # host-buffer and resident steps after xchg_import: exact gradient slices; the host path sums per chunk, so its
+        # losses agree with the full batch's to rounding
+        for name, (hl, hgl, hgc) in host.items():
+            assert np.array_equal(hgl, gl) and np.array_equal(hgc, gcf), (rank, name)
+            assert np.allclose(hl, fl, rtol=1e-6, atol=0), (rank, name, hl, fl)
     assert np.array_equal(res[0][3], res[1][3]), "both ranks must hold bit-identical global losses"
+    for name in res[0][10]:                             # sum_chunks_xchg_kernel folds in rank order on every rank
+        assert np.array_equal(res[0][10][name][0], res[1][10][name][0]), name
