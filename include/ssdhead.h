@@ -374,7 +374,14 @@ int ssdhead_pack_gt(const float* const* boxes_host, const float* const* classes_
 
 /* ---- host-buffer front end (pinned staging + streams owned by the context) -----------
  * The same path for callers whose tensors live in host memory (what the reference's CPU
- * path sees).  Copies are pipelined against the kernels in image chunks. */
+ * path sees).  Copies are pipelined against the kernels in image chunks.
+ * Ordering: the device entry points of a context (loss_dev, _dev_resident, _levels_dev, begin/end) and its host loss
+ * entry points (loss_host, _host_sparse) share the context's match outputs and loss workspace.  Every host call
+ * (detect_host too, although it shares no buffer with the device steps) waits for the context's last eager device
+ * call, so a device step may be followed by a host call without a synchronize (the host call returns once both are
+ * done).  That wait does not reach work replayed from a captured CUDA
+ * graph: a caller that replays captured context steps orders the replay with the host calls itself (e.g. synchronizes
+ * the replay stream first).  Device calls of one context on different streams are ordered by the caller as well. */
 typedef struct ssdhead_ctx ssdhead_ctx;
 int  ssdhead_ctx_create(ssdhead_ctx** out, int device, int maxB, int P, int C, int max_sumG, int top_k,
                         const float* pri_cxcywh_host);

@@ -241,6 +241,33 @@ static int ctx_loss_ws_for(ssdhead_ctx* c, int B, cudaStream_t st)
     return 0;
 }
 
+// The device entry points run asynchronously on the caller's stream and use the context's match outputs, match
+// workspace and loss-workspace slot 0; the host entry points use the same buffers from the context's own streams.
+// Each device call records ev_done behind its work, and every host call makes s_aux and s_main wait on it before its
+// first copy, so a host call never overlaps the device step queued before it.  Not while the stream is capturing: an
+// event recorded inside a capture cannot be waited on from outside it, so the caller orders graph replays of captured
+// context steps with the host calls itself.
+static int ctx_device_done(ssdhead_ctx* c, cudaStream_t st, int rc)
+{
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    const cudaError_t q = cudaStreamIsCapturing(st, &cap);
+    if (q != cudaSuccess) {                  // the legacy stream while another stream captures: nothing to record
+        if (q == cudaErrorStreamCaptureImplicit) (void)cudaGetLastError();
+        return rc;
+    }
+    if (cap == cudaStreamCaptureStatusNone) {
+        const cudaError_t e = cudaEventRecord(c->ev_done, st);
+        if (e != cudaSuccess && rc == 0) rc = (int)e;
+    }
+    return rc;
+}
+static int ctx_host_after_device(ssdhead_ctx* c)
+{
+    SSD_CHECK_CUDA(cudaStreamWaitEvent(c->s_aux, c->ev_done, 0));
+    SSD_CHECK_CUDA(cudaStreamWaitEvent(c->s_main, c->ev_done, 0));
+    return 0;
+}
+
 #define CTX_CUDA(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) { rc = (int)_e; goto fail; } } while (0)
 
 static const int kMaxChunks = 16;
@@ -407,9 +434,8 @@ int ssdhead_ctx_multibox_loss_begin(ssdhead_ctx* c, const float* conf,
     const int rc = ssdhead_ce_match_stream(conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, B, c->P, c->C, sumG, pos_iou,
                                            nullptr, grad_loc, grad_conf, c->cls_u8, c->best_prior, c->npos,
                                            c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes, 1, st);
-    if (rc) return rc;
-    if (npos_total_dev) *npos_total_dev = c->npos + B;
-    return 0;
+    if (rc == 0 && npos_total_dev) *npos_total_dev = c->npos + B;
+    return ctx_device_done(c, st, rc);
 }
 
 // end: the mining kernel, normalised by *npos_norm_dev (null = this rank's own count).
@@ -420,10 +446,11 @@ int ssdhead_ctx_multibox_loss_end(ssdhead_ctx* c, const float* loc, const float*
 {
     if (!c) return SSDHEAD_E_BADARG;
     if (B <= 0 || B > c->maxB) return SSDHEAD_E_STATE;
-    return ssdhead_mine(loc, conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, c->best_prior, c->npos,
-                        npos_norm_dev ? npos_norm_dev : c->npos + B,
-                        c->cls_u8, B, c->P, c->C, neg_ratio, pos_iou, sums, losses, grad_loc, grad_conf, nullptr, nullptr,
-                        c->ws_loss, c->ws_loss_bytes, (cudaStream_t)stream);
+    const int rc = ssdhead_mine(loc, conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, c->best_prior, c->npos,
+                                npos_norm_dev ? npos_norm_dev : c->npos + B,
+                                c->cls_u8, B, c->P, c->C, neg_ratio, pos_iou, sums, losses, grad_loc, grad_conf, nullptr, nullptr,
+                                c->ws_loss, c->ws_loss_bytes, (cudaStream_t)stream);
+    return ctx_device_done(c, (cudaStream_t)stream, rc);
 }
 
 // One training-head step on DEVICE tensors: ssdhead_multibox_step, or the sharded step - two kernels on `stream`.
@@ -435,14 +462,17 @@ int ssdhead_ctx_multibox_loss_dev(ssdhead_ctx* c, const float* loc, const float*
     if (!c) return SSDHEAD_E_BADARG;
     if (B <= 0 || B > c->maxB || sumG < 0 || sumG > c->max_sumG) return SSDHEAD_E_STATE;
     { const int zr = ctx_loss_ws_for(c, B, (cudaStream_t)stream); if (zr) return zr; }
+    int rc;
     if (c->xchg_R > 1)
-        return ssdhead_multibox_step_sharded(loc, conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
-                                             neg_ratio, pos_iou, sums, losses, grad_loc, grad_conf, c->cls_u8, c->best_prior, c->npos,
-                                             c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes,
-                                             c->xchg_R, c->xchg_rank, ++c->xchg_seq, c->xchg_peers_dev, c->xchg_local, c->err_flag, stream);
-    return ssdhead_multibox_step(loc, conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
-                                 neg_ratio, pos_iou, sums, losses, grad_loc, grad_conf, c->cls_u8, c->best_prior, c->npos,
-                                 nullptr, nullptr, c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes, stream);
+        rc = ssdhead_multibox_step_sharded(loc, conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
+                                           neg_ratio, pos_iou, sums, losses, grad_loc, grad_conf, c->cls_u8, c->best_prior, c->npos,
+                                           c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes,
+                                           c->xchg_R, c->xchg_rank, ++c->xchg_seq, c->xchg_peers_dev, c->xchg_local, c->err_flag, stream);
+    else
+        rc = ssdhead_multibox_step(loc, conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
+                                   neg_ratio, pos_iou, sums, losses, grad_loc, grad_conf, c->cls_u8, c->best_prior, c->npos,
+                                   nullptr, nullptr, c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes, stream);
+    return ctx_device_done(c, (cudaStream_t)stream, rc);
 }
 
 int ssdhead_ctx_multibox_loss_dev_resident(ssdhead_ctx* c, const float* loc, const float* conf,
@@ -470,12 +500,13 @@ int ssdhead_ctx_multibox_loss_dev_resident(ssdhead_ctx* c, const float* loc, con
     }
     { const int zr = ctx_loss_ws_for(c, B, st); if (zr) return zr; }
     const bool sharded = c->xchg_R > 1;
-    return ssdhead_multibox_step_resident(loc, conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
+    const int rc = ssdhead_multibox_step_resident(loc, conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
                                           neg_ratio, pos_iou, sums, losses, grad_loc, grad_conf, c->cls_u8, c->best_prior, c->npos,
                                           c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes, c->ws_rows, c->ws_rows_bytes,
                                           sharded ? c->xchg_R : 1, sharded ? c->xchg_rank : 0, sharded ? ++c->xchg_seq : 0u,
                                           sharded ? c->xchg_peers_dev : nullptr, sharded ? c->xchg_local : nullptr,
                                           sharded ? c->err_flag : nullptr, stream);
+    return ctx_device_done(c, st, rc);
 }
 
 int ssdhead_ctx_multibox_loss_levels_dev(ssdhead_ctx* c, const ssdhead_levels* levels,
@@ -486,14 +517,17 @@ int ssdhead_ctx_multibox_loss_levels_dev(ssdhead_ctx* c, const ssdhead_levels* l
     if (!c || !levels) return SSDHEAD_E_BADARG;
     if (B <= 0 || B > c->maxB || sumG < 0 || sumG > c->max_sumG) return SSDHEAD_E_STATE;
     { const int zr = ctx_loss_ws_for(c, B, (cudaStream_t)stream); if (zr) return zr; }
+    int rc;
     if (c->xchg_R > 1)
-        return ssdhead_multibox_step_levels_sharded(levels, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
-                                                    neg_ratio, pos_iou, sums, losses, c->cls_u8, c->best_prior, c->npos,
-                                                    c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes,
-                                                    c->xchg_R, c->xchg_rank, ++c->xchg_seq, c->xchg_peers_dev, c->xchg_local, c->err_flag, stream);
-    return ssdhead_multibox_step_levels(levels, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
-                                        neg_ratio, pos_iou, sums, losses, c->cls_u8, c->best_prior, c->npos,
-                                        c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes, stream);
+        rc = ssdhead_multibox_step_levels_sharded(levels, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
+                                                  neg_ratio, pos_iou, sums, losses, c->cls_u8, c->best_prior, c->npos,
+                                                  c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes,
+                                                  c->xchg_R, c->xchg_rank, ++c->xchg_seq, c->xchg_peers_dev, c->xchg_local, c->err_flag, stream);
+    else
+        rc = ssdhead_multibox_step_levels(levels, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
+                                          neg_ratio, pos_iou, sums, losses, c->cls_u8, c->best_prior, c->npos,
+                                          c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes, stream);
+    return ctx_device_done(c, (cudaStream_t)stream, rc);
 }
 
 int ssdhead_ctx_xchg_export(ssdhead_ctx* c, void* handle64_out)
@@ -555,6 +589,7 @@ static int loss_host_impl(ssdhead_ctx* c, const float* loc_h, const float* conf_
     SSD_CHECK_CUDA(cudaSetDevice(c->device));
     const int P = c->P, C = c->C;
     const bool grads = grad_loc_h != nullptr;
+    { const int wr = ctx_host_after_device(c); if (wr) return wr; }
     { const int zr = ctx_loss_ws_for(c, -B, c->s_main); if (zr) return zr; }   // (-B: the chunked layout of batch B)
 
     // gt -> device, match on the auxiliary stream
@@ -730,6 +765,7 @@ int ssdhead_ctx_detect_host(ssdhead_ctx* c, const float* loc_h, const float* con
     if (B <= 0 || B > c->maxB || !c->ws_detect) return SSDHEAD_E_STATE;
     SSD_CHECK_CUDA(cudaSetDevice(c->device));
     const size_t nr = (size_t)B * c->P;
+    { const int wr = ctx_host_after_device(c); if (wr) return wr; }
     if (c->last_detect_B != B) {
         // the detect workspace keeps its counters zeroed, but their position depends on B: re-zero on a shape change
         SSD_CHECK_CUDA(cudaMemsetAsync(c->ws_detect, 0, c->ws_detect_bytes, c->s_main));
