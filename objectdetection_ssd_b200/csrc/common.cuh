@@ -251,6 +251,87 @@ constexpr int XCHG_MAX_R = 16;
 constexpr int XCHG_WORDS = 2 * 4 * XCHG_MAX_R;     // parity x {npos, sum_l1, sum_ce, sums_flag} x rank
 __host__ __device__ __forceinline__ int xchg_slot(unsigned seq, int what, int rank) { return ((int)(seq & 1u) * 4 + what) * XCHG_MAX_R + rank; }
 
+// The exchange of a batch sharded by image over R GPUs; R <= 1: no exchange.
+struct Xchg {
+    int R, rank;
+    unsigned int seq;                        // step sequence number (>= 1); slots are double-buffered by its parity
+    unsigned long long* const* peers;        // [R] device table: peer-mapped exchange buffers, indexed by rank
+    unsigned long long* local;               // this rank's buffer
+    int* err_flag;                           // set to 1 if a bounded wait expired
+};
+
+// This rank's positive count into the exchange buffer of every rank (own included): one 64-bit word seq << 32 | count
+// validates itself, so relaxed, pipelined stores suffice
+__device__ __forceinline__ void xchg_publish_count(const Xchg& x, unsigned count) {
+    const unsigned long long word = ((unsigned long long)x.seq << 32) | count;
+    for (int q = 0; q < x.R; ++q) st_relaxed_sys_u64(x.peers[q] + xchg_slot(x.seq, 0, x.rank), word);
+}
+// The global positive count: the words of all ranks in this rank's buffer.  The wait is bounded; when it expires,
+// err_flag reports it.
+__device__ __forceinline__ int xchg_gather_count(const Xchg& x) {
+    unsigned spins = 0;
+    int tot = 0;
+    for (int q = 0; q < x.R; ++q) {
+        unsigned long long w;
+        while ((unsigned)((w = ld_acquire_sys_u64(x.local + xchg_slot(x.seq, 0, q))) >> 32) != x.seq && ++spins < (1u << 27)) __nanosleep(64);
+        tot += (int)(unsigned)w;
+    }
+    if (spins >= (1u << 27)) *x.err_flag = 1;
+    return tot;
+}
+// All-reduce of the two loss sums: values first, one system fence, then the flags; the global sums are accumulated in
+// rank order on every rank -> identical bits everywhere.  Bounded wait as above.
+__device__ __forceinline__ void xchg_allreduce_sums(const Xchg& x, double& a, double& c) {
+    for (int q = 0; q < x.R; ++q) {
+        st_relaxed_sys_u64(x.peers[q] + xchg_slot(x.seq, 1, x.rank), (unsigned long long)__double_as_longlong(a));
+        st_relaxed_sys_u64(x.peers[q] + xchg_slot(x.seq, 2, x.rank), (unsigned long long)__double_as_longlong(c));
+    }
+    __threadfence_system();
+    for (int q = 0; q < x.R; ++q) st_relaxed_sys_u64(x.peers[q] + xchg_slot(x.seq, 3, x.rank), (unsigned long long)x.seq);
+    unsigned spins = 0;
+    a = 0.0; c = 0.0;
+    for (int q = 0; q < x.R; ++q) {
+        while ((unsigned)ld_acquire_sys_u64(x.local + xchg_slot(x.seq, 3, q)) != x.seq && ++spins < (1u << 27)) __nanosleep(64);
+        a += __longlong_as_double((long long)ld_relaxed_sys_u64(x.local + xchg_slot(x.seq, 1, q)));
+        c += __longlong_as_double((long long)ld_relaxed_sys_u64(x.local + xchg_slot(x.seq, 2, q)));
+    }
+    if (spins >= (1u << 27)) *x.err_flag = 1;
+}
+// Losses.py:182,197: the box loss over 4 N, the class loss over N
+__device__ __forceinline__ void losses_from_sums(float* losses, double sum_l1, double sum_ce, int npos) {
+    const double N = (double)npos;
+    losses[0] = (float)(sum_l1 / (4.0 * N));
+    losses[1] = (float)(sum_ce / N);
+}
+
+// The arguments of the loss entry points, in the order they take them; an entry point leaves what it does not take null.
+struct StepArgs {
+    const ssdhead_levels* levels;
+    const float *loc, *conf, *gt_xyxy, *gt_cls;
+    const int32_t* gt_off;
+    const float *pri_xyxy, *pri_cxcywh;
+    int B, P, C, sumG, neg_ratio;
+    float pos_iou;
+    double* sums;
+    float *losses, *grad_loc, *grad_conf;
+    uint8_t* cls_u8;
+    int32_t *best_prior, *npos;
+    uint32_t* mined_mask;
+    float* ce;
+    void* ws_loss; size_t ws_loss_bytes;
+    void* ws_match; size_t ws_match_bytes;
+    void* ws_rows; size_t ws_rows_bytes;
+    void* stream;
+};
+
+// The training-head step on the flat head tensors, on the per-level tensors of a.levels, or on resident gradient
+// tensors described by a.ws_rows (ssdhead_multibox_step_resident)
+enum class StepKind { flat, levels, resident };
+
+// The whole training-head step of one GPU with every argument check (loss.cu).  x: the exchange of a sharded batch,
+// or null for none.
+int run_step(StepKind kind, const StepArgs& a, const Xchg* x);
+
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(FULL, v, d);

@@ -36,61 +36,32 @@ __global__ void sum_chunks_kernel(const double* __restrict__ chunk_sums, int nch
     double a = 0.0, c = 0.0;
     for (int i = 0; i < nchunks; ++i) { a += chunk_sums[2 * i]; c += chunk_sums[2 * i + 1]; }
     sums[0] = a; sums[1] = c;
-    const double N = (double)(*npos_norm);
-    losses[0] = (float)(a / (4.0 * N));
-    losses[1] = (float)(c / N);
+    losses_from_sums(losses, a, c, *npos_norm);
 }
 
-// Sharded batches through the host-buffer entry points: the same exchange buffers the fused mining kernel uses
+// Sharded batches through the host-buffer entry points: the same exchange protocol the fused mining kernel uses
 // (common.cuh), driven by two single-thread kernels.  xchg_npos_kernel: this rank's positive count goes to every rank,
 // the global count comes back - before any chunk is mined (it scales the gradients, Losses.py:182,197).
-struct XchgArgs {
-    int R, rank;
-    unsigned int seq;
-    unsigned long long* const* peers;
-    unsigned long long* local;
-    int* err_flag;
-};
-__global__ void xchg_npos_kernel(const int* __restrict__ npos_local, int* __restrict__ npos_global, const XchgArgs x)
+__global__ void xchg_npos_kernel(const int* __restrict__ npos_local, int* __restrict__ npos_global, const Xchg x)
 {
-    const unsigned long long word = ((unsigned long long)x.seq << 32) | (unsigned)(*npos_local);
-    for (int q = 0; q < x.R; ++q) st_relaxed_sys_u64(x.peers[q] + xchg_slot(x.seq, 0, x.rank), word);   // self-validating word
-    unsigned spins = 0;
-    int tot = 0;
-    for (int q = 0; q < x.R; ++q) {
-        unsigned long long w;
-        while ((unsigned)((w = ld_acquire_sys_u64(x.local + xchg_slot(x.seq, 0, q))) >> 32) != x.seq && ++spins < (1u << 27)) __nanosleep(64);
-        tot += (int)(unsigned)w;
-    }
-    if (spins >= (1u << 27)) *x.err_flag = 1;
-    *npos_global = tot;
+    xchg_publish_count(x, (unsigned)(*npos_local));
+    *npos_global = xchg_gather_count(x);
 }
-// The chunk sums of this rank -> global sums (added in rank order on every rank: identical bits everywhere) -> losses.
+// The chunk sums of this rank -> global sums -> losses.
 __global__ void sum_chunks_xchg_kernel(const double* __restrict__ chunk_sums, int nchunks, const int* __restrict__ npos_norm,
-                                       double* __restrict__ sums, float* __restrict__ losses, const XchgArgs x)
+                                       double* __restrict__ sums, float* __restrict__ losses, const Xchg x)
 {
     double a = 0.0, c = 0.0;
     for (int i = 0; i < nchunks; ++i) { a += chunk_sums[2 * i]; c += chunk_sums[2 * i + 1]; }
-    for (int q = 0; q < x.R; ++q) {
-        st_relaxed_sys_u64(x.peers[q] + xchg_slot(x.seq, 1, x.rank), (unsigned long long)__double_as_longlong(a));
-        st_relaxed_sys_u64(x.peers[q] + xchg_slot(x.seq, 2, x.rank), (unsigned long long)__double_as_longlong(c));
-    }
-    __threadfence_system();                      // values before flags
-    for (int q = 0; q < x.R; ++q) st_relaxed_sys_u64(x.peers[q] + xchg_slot(x.seq, 3, x.rank), (unsigned long long)x.seq);
-    unsigned spins = 0;
-    a = 0.0; c = 0.0;
-    for (int q = 0; q < x.R; ++q) {
-        while ((unsigned)ld_acquire_sys_u64(x.local + xchg_slot(x.seq, 3, q)) != x.seq && ++spins < (1u << 27)) __nanosleep(64);
-        a += __longlong_as_double((long long)ld_relaxed_sys_u64(x.local + xchg_slot(x.seq, 1, q)));
-        c += __longlong_as_double((long long)ld_relaxed_sys_u64(x.local + xchg_slot(x.seq, 2, q)));
-    }
-    if (spins >= (1u << 27)) *x.err_flag = 1;
+    xchg_allreduce_sums(x, a, c);
     sums[0] = a; sums[1] = c;
-    const double N = (double)(*npos_norm);
-    losses[0] = (float)(a / (4.0 * N));
-    losses[1] = (float)(c / N);
+    losses_from_sums(losses, a, c, *npos_norm);
 }
 }  // namespace ssdhead
+
+// Image chunks of a host-buffer loss call (the formula in loss_host_impl caps them at 8): each has its own loss-workspace
+// slot, its own entry of chunk_sums and its own pair of copy events.
+static constexpr int kMaxChunks = 8;
 
 // A few host threads that live as long as the context: they zero the caller's DENSE gradient buffers while the inputs
 // of a host-buffer loss call stream in (spawning threads per call would cost ~0.1 ms of every call).  All waiting is
@@ -102,7 +73,7 @@ struct ZeroPool {
     std::function<void(int)> job;          // job(thread index); valid while a generation is running
     unsigned generation = 0;
     int finished = 0;
-    int chunk_done[16] = {};               // threads that finished chunk k of the current generation
+    int chunk_done[kMaxChunks] = {};       // threads that finished chunk k of the current generation
     bool stop = false;
 
     int size() const { return (int)threads.size(); }
@@ -171,19 +142,21 @@ static int zero_pool_threads()
     return (int)std::min(8u, std::max(1u, cores / (unsigned)ranks / 2u));
 }
 
+// What the loss-workspace slots were last laid out for: a device step of B images in slot 0, or the image chunks of a
+// host-buffer call of B images, one per slot
+struct LossLayout { int B; bool chunked; };
+
 struct ssdhead_ctx {
     ZeroPool pool;
-    int device, maxB, P, C, max_sumG, top_k, last_detect_B, last_loss_B;
-    // cross-GPU exchange (sharded batches)
-    int xchg_R, xchg_rank;
-    unsigned int xchg_seq;
-    void* xchg_local;
-    void** xchg_peers_dev;
-    void* xchg_opened[16];
-    int* err_flag;
+    int device, maxB, P, C, max_sumG, top_k, last_detect_B;
+    LossLayout loss_layout;
+    // cross-GPU exchange (sharded batches): R = 1 until ssdhead_ctx_xchg_import; the peer buffers it mapped
+    Xchg xchg;
+    void* xchg_opened[XCHG_MAX_R];
+    std::vector<void*> owned;                           // every device buffer of the context (alloc / release)
     cudaStream_t s_main, s_aux, s_h2d, s_d2h;
-    cudaEvent_t ev_fork, ev_join, ev_gt, ev_done;
-    std::vector<cudaEvent_t> ev_in, ev_out;            // per chunk
+    cudaEvent_t ev_join, ev_done;
+    cudaEvent_t ev_in[kMaxChunks], ev_out[kMaxChunks];  // per chunk
     // prior tables
     float *pri_cxcywh, *pri_xyxy;
     // gt + match outputs
@@ -201,7 +174,7 @@ struct ssdhead_ctx {
     size_t ws_rows_bytes;
     float *res_grad_loc, *res_grad_conf;
     int res_B;                              // images of the two tensors that were zero-filled at the hand-over
-    size_t ws_match_bytes, ws_loss_bytes, ws_loss_total, ws_detect_bytes;
+    size_t ws_match_bytes, ws_loss_bytes, ws_detect_bytes;
     // detect outputs (host-buffer path)
     float *det_boxes, *det_prob;
     int32_t *det_cls, *det_prior, *det_cnt;
@@ -213,6 +186,20 @@ struct ssdhead_ctx {
     int32_t *sp_cnt, *sp_idx;
     float *sp_conf, *sp_loc;
     size_t sp_rows;                                     // capacity of the staging in rows (B * row_cap)
+
+    // A device buffer of the context, zero-filled on request; ssdhead_ctx_destroy frees every one still held
+    template <typename T> cudaError_t alloc(T** p, size_t bytes, bool zero = false) {
+        const cudaError_t e = cudaMalloc((void**)p, bytes);
+        if (e != cudaSuccess) return e;
+        owned.push_back((void*)*p);
+        return zero ? cudaMemset((void*)*p, 0, bytes) : cudaSuccess;
+    }
+    template <typename T> void release(T*& p) {
+        if (!p) return;
+        owned.erase(std::find(owned.begin(), owned.end(), (void*)p));
+        cudaFree((void*)p);
+        p = nullptr;
+    }
 };
 
 // Device-visible alias of a page-locked host buffer (UVA maps cudaHostAlloc / cudaHostRegister memory), or null for
@@ -230,14 +217,14 @@ static const float* mapped_host_alias(const float* host)
 
 // The loss workspace keeps its counters and per-image partial sums zeroed between steps, but their extent depends on
 // the batch size (include/ssdhead.h: "re-zero a buffer before reusing it with another shape"): re-zero the headers of
-// all chunk workspaces when B changes.
-static int ctx_loss_ws_for(ssdhead_ctx* c, int B, cudaStream_t st)
+// all chunk workspaces when the layout changes.
+static int ctx_loss_ws_for(ssdhead_ctx* c, LossLayout l, cudaStream_t st)
 {
-    if (c->last_loss_B == B) return 0;
-    const size_t head = loss_ws_header_bytes(c->maxB);
-    for (size_t off = 0; off + head <= c->ws_loss_total; off += c->ws_loss_bytes)
+    if (c->loss_layout.B == l.B && c->loss_layout.chunked == l.chunked) return 0;
+    const size_t head = loss_ws_header_bytes(c->maxB), total = c->ws_loss_bytes * kMaxChunks;
+    for (size_t off = 0; off + head <= total; off += c->ws_loss_bytes)
         SSD_CHECK_CUDA(cudaMemsetAsync((char*)c->ws_loss + off, 0, std::min(head, c->ws_loss_bytes), st));
-    c->last_loss_B = B;
+    c->loss_layout = l;
     return 0;
 }
 
@@ -268,9 +255,26 @@ static int ctx_host_after_device(ssdhead_ctx* c)
     return 0;
 }
 
-#define CTX_CUDA(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) { rc = (int)_e; goto fail; } } while (0)
+// The exchange of the next step of a sharded batch (the step sequence number advances), or null on one GPU
+static const Xchg* ctx_next_xchg(ssdhead_ctx* c)
+{
+    if (c->xchg.R <= 1) return nullptr;
+    ++c->xchg.seq;
+    return &c->xchg;
+}
 
-static const int kMaxChunks = 16;
+// One step of the device entry points on the caller's stream, with the context's priors, match outputs and workspaces
+// (B and sumG are checked against the context by the caller)
+static int ctx_step(ssdhead_ctx* c, StepKind kind, StepArgs a)
+{
+    a.pri_xyxy = c->pri_xyxy; a.pri_cxcywh = c->pri_cxcywh; a.P = c->P; a.C = c->C;
+    a.cls_u8 = c->cls_u8; a.best_prior = c->best_prior; a.npos = c->npos;
+    a.ws_loss = c->ws_loss; a.ws_loss_bytes = c->ws_loss_bytes; a.ws_match = c->ws_match; a.ws_match_bytes = c->ws_match_bytes;
+    a.ws_rows = c->ws_rows; a.ws_rows_bytes = c->ws_rows_bytes;
+    cudaStream_t st = (cudaStream_t)a.stream;
+    { const int zr = ctx_loss_ws_for(c, {a.B, false}, st); if (zr) return zr; }
+    return ctx_device_done(c, st, run_step(kind, a, ctx_next_xchg(c)));
+}
 
 extern "C" {
 
@@ -319,24 +323,15 @@ void ssdhead_ctx_destroy(ssdhead_ctx* c)
     c->pool.shutdown();
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
-    void* bufs[] = {c->pri_cxcywh, c->pri_xyxy, c->gt_xyxy, c->gt_cls, c->gt_off, c->best_prior, c->npos, c->cls_u8,
-                    c->loc, c->conf, c->grad_loc, c->grad_conf, c->sums, c->chunk_sums, c->losses,
-                    c->ws_match, c->ws_loss, c->ws_detect, c->det_boxes, c->det_prob, c->det_cls, c->det_prior, c->det_cnt};
-    for (void* b : bufs) if (b) cudaFree(b);
+    for (void* b : c->owned) cudaFree(b);
     if (c->h_losses) cudaFreeHost(c->h_losses);
-    for (int q = 0; q < 16; ++q) if (c->xchg_opened[q]) cudaIpcCloseMemHandle(c->xchg_opened[q]);
-    if (c->xchg_local) cudaFree(c->xchg_local);
-    if (c->xchg_peers_dev) cudaFree(c->xchg_peers_dev);
-    if (c->err_flag) cudaFree(c->err_flag);
-    if (c->ws_rows) cudaFree(c->ws_rows);
-    void* more[] = {c->npos_global, c->sp_cnt, c->sp_idx, c->sp_conf, c->sp_loc};
-    for (void* b : more) if (b) cudaFree(b);
-    cudaStream_t st[] = {c->s_main, c->s_aux, c->s_h2d, c->s_d2h};
-    for (cudaStream_t s : st) if (s) cudaStreamDestroy(s);
-    cudaEvent_t ev[] = {c->ev_fork, c->ev_join, c->ev_gt, c->ev_done};
-    for (cudaEvent_t e : ev) if (e) cudaEventDestroy(e);
-    for (cudaEvent_t e : c->ev_in) if (e) cudaEventDestroy(e);
-    for (cudaEvent_t e : c->ev_out) if (e) cudaEventDestroy(e);
+    for (void* m : c->xchg_opened) if (m) cudaIpcCloseMemHandle(m);
+    for (cudaStream_t s : {c->s_main, c->s_aux, c->s_h2d, c->s_d2h}) if (s) cudaStreamDestroy(s);
+    for (cudaEvent_t e : {c->ev_join, c->ev_done}) if (e) cudaEventDestroy(e);
+    for (int k = 0; k < kMaxChunks; ++k) {
+        if (c->ev_in[k]) cudaEventDestroy(c->ev_in[k]);
+        if (c->ev_out[k]) cudaEventDestroy(c->ev_out[k]);
+    }
     delete c;
 }
 
@@ -344,79 +339,64 @@ int ssdhead_ctx_create(ssdhead_ctx** out, int device, int maxB, int P, int C, in
                        const float* pri_cxcywh_host)
 {
     if (!out || maxB <= 0 || P <= 0 || C < 2 || max_sumG < 0 || top_k <= 0 || !pri_cxcywh_host) return SSDHEAD_E_BADARG;
-    int rc = 0;
     ssdhead_ctx* c = new ssdhead_ctx();
     c->device = device; c->maxB = maxB; c->P = P; c->C = C; c->max_sumG = std::max(max_sumG, 1); c->top_k = top_k;
-    {
+    c->xchg.R = 1;
+    const int rc = [&]() -> int {
         const size_t nrow = (size_t)maxB * P;
         std::vector<float> xy((size_t)P * 4);
         priors_xyxy_host(pri_cxcywh_host, xy.data(), P);
-        CTX_CUDA(cudaSetDevice(device));
-        CTX_CUDA(cudaStreamCreateWithFlags(&c->s_main, cudaStreamNonBlocking));
-        CTX_CUDA(cudaStreamCreateWithFlags(&c->s_aux, cudaStreamNonBlocking));
-        CTX_CUDA(cudaStreamCreateWithFlags(&c->s_h2d, cudaStreamNonBlocking));
-        CTX_CUDA(cudaStreamCreateWithFlags(&c->s_d2h, cudaStreamNonBlocking));
-        CTX_CUDA(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
-        CTX_CUDA(cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));
-        CTX_CUDA(cudaEventCreateWithFlags(&c->ev_gt, cudaEventDisableTiming));
-        CTX_CUDA(cudaEventCreateWithFlags(&c->ev_done, cudaEventDisableTiming));
-        c->ev_in.assign(kMaxChunks, nullptr);
-        c->ev_out.assign(kMaxChunks, nullptr);
-        for (int i = 0; i < kMaxChunks; ++i) {
-            CTX_CUDA(cudaEventCreateWithFlags(&c->ev_in[i], cudaEventDisableTiming));
-            CTX_CUDA(cudaEventCreateWithFlags(&c->ev_out[i], cudaEventDisableTiming));
+        SSD_CHECK_CUDA(cudaSetDevice(device));
+        for (cudaStream_t* s : {&c->s_main, &c->s_aux, &c->s_h2d, &c->s_d2h})
+            SSD_CHECK_CUDA(cudaStreamCreateWithFlags(s, cudaStreamNonBlocking));
+        SSD_CHECK_CUDA(cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));
+        SSD_CHECK_CUDA(cudaEventCreateWithFlags(&c->ev_done, cudaEventDisableTiming));
+        for (int k = 0; k < kMaxChunks; ++k) {
+            SSD_CHECK_CUDA(cudaEventCreateWithFlags(&c->ev_in[k], cudaEventDisableTiming));
+            SSD_CHECK_CUDA(cudaEventCreateWithFlags(&c->ev_out[k], cudaEventDisableTiming));
         }
-        CTX_CUDA(cudaMalloc(&c->pri_cxcywh, (size_t)P * 16));
-        CTX_CUDA(cudaMalloc(&c->pri_xyxy, (size_t)P * 16));
-        CTX_CUDA(cudaMemcpy(c->pri_cxcywh, pri_cxcywh_host, (size_t)P * 16, cudaMemcpyHostToDevice));
-        CTX_CUDA(cudaMemcpy(c->pri_xyxy, xy.data(), (size_t)P * 16, cudaMemcpyHostToDevice));
-        CTX_CUDA(cudaMalloc(&c->gt_xyxy, (size_t)c->max_sumG * 16));
-        CTX_CUDA(cudaMalloc(&c->gt_cls, (size_t)c->max_sumG * 4));
-        CTX_CUDA(cudaMalloc(&c->gt_off, (size_t)(maxB + 1) * 4));
-        CTX_CUDA(cudaMalloc(&c->best_prior, (size_t)c->max_sumG * 4));
-        CTX_CUDA(cudaMalloc(&c->npos, (size_t)(maxB + 1) * 4));
-        CTX_CUDA(cudaMalloc(&c->cls_u8, round_up(nrow, 16)));
-        CTX_CUDA(cudaMalloc(&c->loc, nrow * 16));
-        CTX_CUDA(cudaMalloc(&c->conf, nrow * C * 4));
-        CTX_CUDA(cudaMalloc(&c->grad_loc, nrow * 16));
-        CTX_CUDA(cudaMalloc(&c->grad_conf, nrow * C * 4));
-        CTX_CUDA(cudaMalloc(&c->sums, 2 * sizeof(double)));
-        CTX_CUDA(cudaMalloc(&c->chunk_sums, 2 * kMaxChunks * sizeof(double)));
-        CTX_CUDA(cudaMalloc(&c->losses, 2 * sizeof(float)));
+        SSD_CHECK_CUDA(c->alloc(&c->pri_cxcywh, (size_t)P * 16));
+        SSD_CHECK_CUDA(c->alloc(&c->pri_xyxy, (size_t)P * 16));
+        SSD_CHECK_CUDA(cudaMemcpy(c->pri_cxcywh, pri_cxcywh_host, (size_t)P * 16, cudaMemcpyHostToDevice));
+        SSD_CHECK_CUDA(cudaMemcpy(c->pri_xyxy, xy.data(), (size_t)P * 16, cudaMemcpyHostToDevice));
+        SSD_CHECK_CUDA(c->alloc(&c->gt_xyxy, (size_t)c->max_sumG * 16));
+        SSD_CHECK_CUDA(c->alloc(&c->gt_cls, (size_t)c->max_sumG * 4));
+        SSD_CHECK_CUDA(c->alloc(&c->gt_off, (size_t)(maxB + 1) * 4));
+        SSD_CHECK_CUDA(c->alloc(&c->best_prior, (size_t)c->max_sumG * 4));
+        SSD_CHECK_CUDA(c->alloc(&c->npos, (size_t)(maxB + 1) * 4));
+        SSD_CHECK_CUDA(c->alloc(&c->cls_u8, round_up(nrow, 16)));
+        SSD_CHECK_CUDA(c->alloc(&c->loc, nrow * 16));
+        SSD_CHECK_CUDA(c->alloc(&c->conf, nrow * C * 4));
+        SSD_CHECK_CUDA(c->alloc(&c->grad_loc, nrow * 16));
+        SSD_CHECK_CUDA(c->alloc(&c->grad_conf, nrow * C * 4));
+        SSD_CHECK_CUDA(c->alloc(&c->sums, 2 * sizeof(double)));
+        SSD_CHECK_CUDA(c->alloc(&c->chunk_sums, 2 * kMaxChunks * sizeof(double)));
+        SSD_CHECK_CUDA(c->alloc(&c->losses, 2 * sizeof(float)));
         c->ws_match_bytes = ssdhead_workspace_bytes(SSDHEAD_WS_MATCH, maxB, P, C, c->max_sumG);
         c->ws_loss_bytes = ssdhead_workspace_bytes(SSDHEAD_WS_LOSS, maxB, P, C, 0);
         c->ws_detect_bytes = ssdhead_workspace_bytes(SSDHEAD_WS_DETECT, maxB, P, C, 0);
-        CTX_CUDA(cudaMalloc(&c->ws_match, c->ws_match_bytes));
-        CTX_CUDA(cudaMemset(c->ws_match, 0, c->ws_match_bytes));
-        if (c->ws_loss_bytes) {
-            // one workspace per chunk slot so chunk i+1 can stream while chunk i is being mined
-            c->ws_loss_total = c->ws_loss_bytes * kMaxChunks;
-            CTX_CUDA(cudaMalloc(&c->ws_loss, c->ws_loss_bytes * kMaxChunks));
-            CTX_CUDA(cudaMemset(c->ws_loss, 0, c->ws_loss_bytes * kMaxChunks));
-        }
-        if (c->ws_detect_bytes) {
-            CTX_CUDA(cudaMalloc(&c->ws_detect, c->ws_detect_bytes));
-            CTX_CUDA(cudaMemset(c->ws_detect, 0, c->ws_detect_bytes));
-        }
-        CTX_CUDA(cudaMalloc(&c->det_boxes, (size_t)maxB * top_k * 16));
-        CTX_CUDA(cudaMalloc(&c->det_prob, (size_t)maxB * top_k * 4));
-        CTX_CUDA(cudaMalloc(&c->det_cls, (size_t)maxB * top_k * 4));
-        CTX_CUDA(cudaMalloc(&c->det_prior, (size_t)maxB * top_k * 4));
-        CTX_CUDA(cudaMalloc(&c->det_cnt, (size_t)maxB * 4));
-        CTX_CUDA(cudaHostAlloc(&c->h_losses, 64, cudaHostAllocDefault));
-        CTX_CUDA(cudaMalloc(&c->xchg_local, ssdhead_xchg_bytes()));
-        CTX_CUDA(cudaMemset(c->xchg_local, 0, ssdhead_xchg_bytes()));
-        CTX_CUDA(cudaMalloc(&c->xchg_peers_dev, 16 * sizeof(void*)));
-        CTX_CUDA(cudaMalloc(&c->err_flag, sizeof(int)));
-        CTX_CUDA(cudaMemset(c->err_flag, 0, sizeof(int)));
-        CTX_CUDA(cudaMalloc(&c->npos_global, sizeof(int32_t)));
-        c->xchg_R = 1;
+        SSD_CHECK_CUDA(c->alloc(&c->ws_match, c->ws_match_bytes, true));
+        // one loss workspace per chunk slot so chunk i+1 can stream while chunk i is being mined
+        if (c->ws_loss_bytes) SSD_CHECK_CUDA(c->alloc(&c->ws_loss, c->ws_loss_bytes * kMaxChunks, true));
+        if (c->ws_detect_bytes) SSD_CHECK_CUDA(c->alloc(&c->ws_detect, c->ws_detect_bytes, true));
+        SSD_CHECK_CUDA(c->alloc(&c->det_boxes, (size_t)maxB * top_k * 16));
+        SSD_CHECK_CUDA(c->alloc(&c->det_prob, (size_t)maxB * top_k * 4));
+        SSD_CHECK_CUDA(c->alloc(&c->det_cls, (size_t)maxB * top_k * 4));
+        SSD_CHECK_CUDA(c->alloc(&c->det_prior, (size_t)maxB * top_k * 4));
+        SSD_CHECK_CUDA(c->alloc(&c->det_cnt, (size_t)maxB * 4));
+        SSD_CHECK_CUDA(cudaHostAlloc(&c->h_losses, 64, cudaHostAllocDefault));
+        SSD_CHECK_CUDA(c->alloc(&c->xchg.local, ssdhead_xchg_bytes(), true));
+        SSD_CHECK_CUDA(c->alloc(&c->xchg.peers, XCHG_MAX_R * sizeof(void*)));
+        SSD_CHECK_CUDA(c->alloc(&c->xchg.err_flag, sizeof(int), true));
+        SSD_CHECK_CUDA(c->alloc(&c->npos_global, sizeof(int32_t)));
+        return 0;
+    }();
+    if (rc) {
+        ssdhead_ctx_destroy(c);
+        return rc;
     }
     *out = c;
     return 0;
-fail:
-    ssdhead_ctx_destroy(c);
-    return rc;
 }
 
 // Sharded batches: the step in two halves around the all-reduce of the positive count (SURVEY.md 8(e)).
@@ -429,7 +409,7 @@ int ssdhead_ctx_multibox_loss_begin(ssdhead_ctx* c, const float* conf,
     if (!c) return SSDHEAD_E_BADARG;
     if (B <= 0 || B > c->maxB || sumG < 0 || sumG > c->max_sumG) return SSDHEAD_E_STATE;
     cudaStream_t st = (cudaStream_t)stream;
-    { const int zr = ctx_loss_ws_for(c, B, st); if (zr) return zr; }
+    { const int zr = ctx_loss_ws_for(c, {B, false}, st); if (zr) return zr; }
     // the natural match rides inside the CE streaming kernel; a small finaliser applies the forced-match override
     const int rc = ssdhead_ce_match_stream(conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, B, c->P, c->C, sumG, pos_iou,
                                            nullptr, grad_loc, grad_conf, c->cls_u8, c->best_prior, c->npos,
@@ -461,18 +441,10 @@ int ssdhead_ctx_multibox_loss_dev(ssdhead_ctx* c, const float* loc, const float*
 {
     if (!c) return SSDHEAD_E_BADARG;
     if (B <= 0 || B > c->maxB || sumG < 0 || sumG > c->max_sumG) return SSDHEAD_E_STATE;
-    { const int zr = ctx_loss_ws_for(c, B, (cudaStream_t)stream); if (zr) return zr; }
-    int rc;
-    if (c->xchg_R > 1)
-        rc = ssdhead_multibox_step_sharded(loc, conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
-                                           neg_ratio, pos_iou, sums, losses, grad_loc, grad_conf, c->cls_u8, c->best_prior, c->npos,
-                                           c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes,
-                                           c->xchg_R, c->xchg_rank, ++c->xchg_seq, c->xchg_peers_dev, c->xchg_local, c->err_flag, stream);
-    else
-        rc = ssdhead_multibox_step(loc, conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
-                                   neg_ratio, pos_iou, sums, losses, grad_loc, grad_conf, c->cls_u8, c->best_prior, c->npos,
-                                   nullptr, nullptr, c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes, stream);
-    return ctx_device_done(c, (cudaStream_t)stream, rc);
+    return ctx_step(c, StepKind::flat,
+                    {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off, .B = B, .sumG = sumG,
+                     .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses, .grad_loc = grad_loc,
+                     .grad_conf = grad_conf, .stream = stream});
 }
 
 int ssdhead_ctx_multibox_loss_dev_resident(ssdhead_ctx* c, const float* loc, const float* conf,
@@ -487,7 +459,7 @@ int ssdhead_ctx_multibox_loss_dev_resident(ssdhead_ctx* c, const float* loc, con
         SSD_CHECK_CUDA(cudaSetDevice(c->device));
         c->ws_rows_bytes = ssdhead_workspace_bytes(SSDHEAD_WS_ROWS, c->maxB, c->P, c->C, 0);
         if (c->ws_rows_bytes == 0) return SSDHEAD_E_UNSUPPORTED;
-        SSD_CHECK_CUDA(cudaMalloc(&c->ws_rows, c->ws_rows_bytes));
+        SSD_CHECK_CUDA(c->alloc(&c->ws_rows, c->ws_rows_bytes));
         fresh = 1;
     }
     if (fresh) {
@@ -498,15 +470,10 @@ int ssdhead_ctx_multibox_loss_dev_resident(ssdhead_ctx* c, const float* loc, con
     } else if (grad_loc != c->res_grad_loc || grad_conf != c->res_grad_conf || B > c->res_B) {
         return SSDHEAD_E_STATE;                          // not the tensors the rows workspace describes, or images beyond the clean part
     }
-    { const int zr = ctx_loss_ws_for(c, B, st); if (zr) return zr; }
-    const bool sharded = c->xchg_R > 1;
-    const int rc = ssdhead_multibox_step_resident(loc, conf, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
-                                          neg_ratio, pos_iou, sums, losses, grad_loc, grad_conf, c->cls_u8, c->best_prior, c->npos,
-                                          c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes, c->ws_rows, c->ws_rows_bytes,
-                                          sharded ? c->xchg_R : 1, sharded ? c->xchg_rank : 0, sharded ? ++c->xchg_seq : 0u,
-                                          sharded ? c->xchg_peers_dev : nullptr, sharded ? c->xchg_local : nullptr,
-                                          sharded ? c->err_flag : nullptr, stream);
-    return ctx_device_done(c, st, rc);
+    return ctx_step(c, StepKind::resident,
+                    {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off, .B = B, .sumG = sumG,
+                     .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses, .grad_loc = grad_loc,
+                     .grad_conf = grad_conf, .stream = stream});
 }
 
 int ssdhead_ctx_multibox_loss_levels_dev(ssdhead_ctx* c, const ssdhead_levels* levels,
@@ -516,18 +483,9 @@ int ssdhead_ctx_multibox_loss_levels_dev(ssdhead_ctx* c, const ssdhead_levels* l
 {
     if (!c || !levels) return SSDHEAD_E_BADARG;
     if (B <= 0 || B > c->maxB || sumG < 0 || sumG > c->max_sumG) return SSDHEAD_E_STATE;
-    { const int zr = ctx_loss_ws_for(c, B, (cudaStream_t)stream); if (zr) return zr; }
-    int rc;
-    if (c->xchg_R > 1)
-        rc = ssdhead_multibox_step_levels_sharded(levels, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
-                                                  neg_ratio, pos_iou, sums, losses, c->cls_u8, c->best_prior, c->npos,
-                                                  c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes,
-                                                  c->xchg_R, c->xchg_rank, ++c->xchg_seq, c->xchg_peers_dev, c->xchg_local, c->err_flag, stream);
-    else
-        rc = ssdhead_multibox_step_levels(levels, gt_xyxy, gt_cls, gt_off, c->pri_xyxy, c->pri_cxcywh, B, c->P, c->C, sumG,
-                                          neg_ratio, pos_iou, sums, losses, c->cls_u8, c->best_prior, c->npos,
-                                          c->ws_loss, c->ws_loss_bytes, c->ws_match, c->ws_match_bytes, stream);
-    return ctx_device_done(c, (cudaStream_t)stream, rc);
+    return ctx_step(c, StepKind::levels,
+                    {.levels = levels, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off, .B = B, .sumG = sumG,
+                     .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses, .stream = stream});
 }
 
 int ssdhead_ctx_xchg_export(ssdhead_ctx* c, void* handle64_out)
@@ -536,25 +494,25 @@ int ssdhead_ctx_xchg_export(ssdhead_ctx* c, void* handle64_out)
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
     SSD_CHECK_CUDA(cudaSetDevice(c->device));
     cudaIpcMemHandle_t h;
-    SSD_CHECK_CUDA(cudaIpcGetMemHandle(&h, c->xchg_local));
+    SSD_CHECK_CUDA(cudaIpcGetMemHandle(&h, c->xchg.local));
     std::memcpy(handle64_out, &h, 64);
     return 0;
 }
 
 int ssdhead_ctx_xchg_import(ssdhead_ctx* c, const void* handles, int R, int rank)
 {
-    if (!c || !handles || R < 1 || R > 16 || rank < 0 || rank >= R) return SSDHEAD_E_BADARG;
+    if (!c || !handles || R < 1 || R > XCHG_MAX_R || rank < 0 || rank >= R) return SSDHEAD_E_BADARG;
     SSD_CHECK_CUDA(cudaSetDevice(c->device));
-    void* table[16] = {};
+    void* table[XCHG_MAX_R] = {};
     for (int q = 0; q < R; ++q) {
-        if (q == rank) { table[q] = c->xchg_local; continue; }
+        if (q == rank) { table[q] = c->xchg.local; continue; }
         cudaIpcMemHandle_t h;
         std::memcpy(&h, (const char*)handles + 64 * q, 64);
         SSD_CHECK_CUDA(cudaIpcOpenMemHandle(&table[q], h, cudaIpcMemLazyEnablePeerAccess));
         c->xchg_opened[q] = table[q];
     }
-    SSD_CHECK_CUDA(cudaMemcpy(c->xchg_peers_dev, table, sizeof(table), cudaMemcpyHostToDevice));
-    c->xchg_R = R; c->xchg_rank = rank; c->xchg_seq = 0;
+    SSD_CHECK_CUDA(cudaMemcpy((void*)c->xchg.peers, table, sizeof(table), cudaMemcpyHostToDevice));
+    c->xchg.R = R; c->xchg.rank = rank; c->xchg.seq = 0;
     return 0;
 }
 
@@ -562,7 +520,7 @@ int ssdhead_ctx_xchg_error(ssdhead_ctx* c)
 {
     if (!c) return SSDHEAD_E_BADARG;
     int e = 0;
-    if (cudaMemcpy(&e, c->err_flag, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess) return 1;
+    if (cudaMemcpy(&e, c->xchg.err_flag, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess) return 1;
     return e;
 }
 
@@ -588,9 +546,46 @@ static int loss_host_impl(ssdhead_ctx* c, const float* loc_h, const float* conf_
     if (sumG < 0 || sumG > c->max_sumG || (sumG > 0 && (!gt_xyxy_h || !gt_cls_h))) return SSDHEAD_E_STATE;
     SSD_CHECK_CUDA(cudaSetDevice(c->device));
     const int P = c->P, C = c->C;
-    const bool grads = grad_loc_h != nullptr;
+
+    // The gradient return, and where the mining kernel writes it.
+    // DENSE.  The gradient is sparse (about 4 Npos of the B x P rows): when the caller's gradient buffers are
+    // page-locked, the dense zero background never crosses PCIe.  Host threads zero the buffers chunk by chunk while the
+    // inputs stream in, the streaming kernel runs without its zero-fill, and the mining kernel stores its few hundred
+    // rows per image straight into the host buffers through their UVA aliases.  Same bits in the caller's buffers.
+    // Pageable buffers get the dense gradient of the context's device buffers, copied back chunk by chunk.
+    // ROWS: packed rows; page-locked output buffers are written in place by the mining kernel, pageable ones through
+    // device staging copied back at the end.  No zero background exists on either side.
+    enum class Grads { none, dense_staged, dense_in_place, rows_in_place, rows_staged };
+    Grads ret = Grads::none;
+    float* gl_dev = nullptr; float* gc_dev = nullptr;
+    int32_t* rc_dev = nullptr; int32_t* ri_dev = nullptr; float* rgc_dev = nullptr; float* rgl_dev = nullptr;
+    if (grad_loc_h) {
+        gl_dev = const_cast<float*>(mapped_host_alias(grad_loc_h));
+        gc_dev = const_cast<float*>(mapped_host_alias(grad_conf_h));
+        ret = gl_dev && gc_dev ? Grads::dense_in_place : Grads::dense_staged;
+        if (ret == Grads::dense_staged) { gl_dev = c->grad_loc; gc_dev = c->grad_conf; }
+    } else if (rows) {
+        rc_dev = (int32_t*)mapped_host_alias((const float*)row_cnt_h);
+        ri_dev = (int32_t*)mapped_host_alias((const float*)row_idx_h);
+        rgc_dev = const_cast<float*>(mapped_host_alias(gconf_rows_h));
+        rgl_dev = const_cast<float*>(mapped_host_alias(gloc_rows_h));
+        ret = rc_dev && ri_dev && rgc_dev && rgl_dev ? Grads::rows_in_place : Grads::rows_staged;
+    }
+    if (ret == Grads::rows_staged) {
+        const size_t need_rows = (size_t)B * row_cap;
+        if (c->sp_rows < need_rows) {
+            c->release(c->sp_cnt); c->release(c->sp_idx); c->release(c->sp_conf); c->release(c->sp_loc);
+            c->sp_rows = 0;
+            SSD_CHECK_CUDA(c->alloc(&c->sp_cnt, (size_t)c->maxB * 2 * 4));
+            SSD_CHECK_CUDA(c->alloc(&c->sp_idx, need_rows * 4));
+            SSD_CHECK_CUDA(c->alloc(&c->sp_conf, need_rows * C * 4));
+            SSD_CHECK_CUDA(c->alloc(&c->sp_loc, need_rows * 16));
+            c->sp_rows = need_rows;
+        }
+        rc_dev = c->sp_cnt; ri_dev = c->sp_idx; rgc_dev = c->sp_conf; rgl_dev = c->sp_loc;
+    }
     { const int wr = ctx_host_after_device(c); if (wr) return wr; }
-    { const int zr = ctx_loss_ws_for(c, -B, c->s_main); if (zr) return zr; }   // (-B: the chunked layout of batch B)
+    { const int zr = ctx_loss_ws_for(c, {B, true}, c->s_main); if (zr) return zr; }
 
     // gt -> device, match on the auxiliary stream
     if (sumG > 0) {
@@ -601,13 +596,10 @@ static int loss_host_impl(ssdhead_ctx* c, const float* loc_h, const float* conf_
     int rc = ssdhead_match(c->gt_xyxy, c->gt_cls, c->gt_off, c->pri_xyxy, B, P, C, sumG, pos_iou,
                            c->best_prior, c->npos, c->cls_u8, nullptr, nullptr, c->ws_match, c->ws_match_bytes, c->s_aux);
     if (rc) return rc;
-    const bool sharded = c->xchg_R > 1;
-    XchgArgs xa = {};
+    const Xchg* x = ctx_next_xchg(c);
     const int32_t* npos_norm = c->npos + B;
-    if (sharded) {
-        xa.R = c->xchg_R; xa.rank = c->xchg_rank; xa.seq = ++c->xchg_seq;
-        xa.peers = (unsigned long long* const*)c->xchg_peers_dev; xa.local = (unsigned long long*)c->xchg_local; xa.err_flag = c->err_flag;
-        xchg_npos_kernel<<<1, 1, 0, c->s_aux>>>(c->npos + B, c->npos_global, xa);
+    if (x) {
+        xchg_npos_kernel<<<1, 1, 0, c->s_aux>>>(c->npos + B, c->npos_global, *x);
         count_launch();
         SSD_LAUNCH_CHECK();
         npos_norm = c->npos_global;
@@ -618,83 +610,52 @@ static int loss_host_impl(ssdhead_ctx* c, const float* loc_h, const float* conf_
     // >= 8 images per chunk, at most 8 chunks (measured on B200/PCIe5: 1 chunk 8.2 ms, 4: 5.8, 8: 5.6, 16: 6.3 at B=256)
     const int nchunks = std::min(8, std::max(1, B / 8));
     const int per = (B + nchunks - 1) / nchunks;
-    int used = 0;
+    struct Chunk { int b0, nb; size_t r0, nr; } chunk[kMaxChunks];      // first image, images, first row, rows
+    for (int k = 0, b0 = 0; b0 < B; ++k, b0 += per) {
+        const int nb = std::min(per, B - b0);
+        chunk[k] = {b0, nb, (size_t)b0 * P, (size_t)nb * P};
+    }
 
-    // DENSE return.  The gradient is sparse (about 4 Npos of the B x P rows): when the caller's gradient buffers are
-    // page-locked, the dense zero background never crosses PCIe.  Host threads zero the buffers chunk by chunk while the
-    // inputs stream in, the streaming kernel runs without its zero-fill, and the mining kernel stores its few hundred
-    // rows per image straight into the host buffers through their UVA aliases.  Same bits in the caller's buffers.
-    float* gl_alias = grads ? const_cast<float*>(mapped_host_alias(grad_loc_h)) : nullptr;
-    float* gc_alias = grads ? const_cast<float*>(mapped_host_alias(grad_conf_h)) : nullptr;
-    const bool sparse = gl_alias && gc_alias;
-    int T = 0;
-    if (sparse) {
+    // the pool's job writes into the caller's buffers: no return before it is done
+    struct JoinPool { ZeroPool* pool; ~JoinPool() { if (pool) pool->wait(); } } join = {nullptr};
+    if (ret == Grads::dense_in_place) {
         if (c->pool.size() == 0) c->pool.start(zero_pool_threads());
-        T = c->pool.size();
+        const int T = c->pool.size();
         ZeroPool* pool = &c->pool;
         c->pool.run([=](int ti) {
-            for (int k = 0, b0 = 0; b0 < B; ++k, b0 += per) {
-                const int nb = std::min(per, B - b0);
-                const size_t r0 = (size_t)b0 * P, nr = (size_t)nb * P;
+            for (int k = 0; k < nchunks; ++k) {
                 auto zero_part = [&](float* base, size_t floats) {
                     const size_t part = ((floats + T - 1) / T + 15) & ~(size_t)15;     // T parts cover everything
                     const size_t lo = std::min(floats, part * ti), hi = std::min(floats, lo + part);
                     if (hi > lo) std::memset(base + lo, 0, (hi - lo) * sizeof(float));
                 };
-                zero_part(grad_conf_h + r0 * C, nr * C);
-                zero_part(grad_loc_h + r0 * 4, nr * 4);
+                zero_part(grad_conf_h + chunk[k].r0 * C, chunk[k].nr * C);
+                zero_part(grad_loc_h + chunk[k].r0 * 4, chunk[k].nr * 4);
                 pool->mark_chunk(k);
             }
         });
+        join.pool = pool;
     }
-    // ROW return: packed rows; page-locked output buffers are written in place by the mining kernel, pageable ones
-    // through device staging copied back at the end.  No zero background exists on either side.
-    int32_t* rc_dev = nullptr; int32_t* ri_dev = nullptr; float* rgc_dev = nullptr; float* rgl_dev = nullptr;
-    bool rows_staged = false;
-    if (rows) {
-        rc_dev = (int32_t*)mapped_host_alias((const float*)row_cnt_h);
-        ri_dev = (int32_t*)mapped_host_alias((const float*)row_idx_h);
-        rgc_dev = const_cast<float*>(mapped_host_alias(gconf_rows_h));
-        rgl_dev = const_cast<float*>(mapped_host_alias(gloc_rows_h));
-        if (!rc_dev || !ri_dev || !rgc_dev || !rgl_dev) {
-            const size_t need_rows = (size_t)B * row_cap;
-            if (c->sp_rows < need_rows) {
-                void* old[] = {c->sp_cnt, c->sp_idx, c->sp_conf, c->sp_loc};
-                for (void* o : old) if (o) cudaFree(o);
-                c->sp_cnt = nullptr; c->sp_idx = nullptr; c->sp_conf = nullptr; c->sp_loc = nullptr; c->sp_rows = 0;
-                SSD_CHECK_CUDA(cudaMalloc(&c->sp_cnt, (size_t)c->maxB * 2 * 4));
-                SSD_CHECK_CUDA(cudaMalloc(&c->sp_idx, need_rows * 4));
-                SSD_CHECK_CUDA(cudaMalloc(&c->sp_conf, need_rows * C * 4));
-                SSD_CHECK_CUDA(cudaMalloc(&c->sp_loc, need_rows * 16));
-                c->sp_rows = need_rows;
-            }
-            rc_dev = c->sp_cnt; ri_dev = c->sp_idx; rgc_dev = c->sp_conf; rgl_dev = c->sp_loc;
-            rows_staged = true;
-        }
-    }
-    auto join_all = [&]() { if (sparse) c->pool.wait(); };     // the job references the caller's buffers: never return before it is done
-#define CTX_HOST_CHECK(expr) do { const int _rc = (expr); if (_rc) { join_all(); return _rc; } } while (0)
 
     // all input copies first (they depend on nothing), then the kernels chunk by chunk
-    for (int k = 0, b0 = 0; b0 < B; ++k, b0 += per) {
-        const int nb = std::min(per, B - b0);
-        const size_t r0 = (size_t)b0 * P, nr = (size_t)nb * P;
-        CTX_HOST_CHECK((int)cudaMemcpyAsync(c->conf + r0 * C, conf_h + r0 * C, nr * C * 4, cudaMemcpyHostToDevice, c->s_h2d));
+    for (int k = 0; k < nchunks; ++k) {
+        const auto& [b0, nb, r0, nr] = chunk[k];
+        SSD_CHECK_CUDA(cudaMemcpyAsync(c->conf + r0 * C, conf_h + r0 * C, nr * C * 4, cudaMemcpyHostToDevice, c->s_h2d));
         // the mining kernel reads loc only for the positive rows (~50 per image): page-locked loc is read in place
-        if (!loc_alias) CTX_HOST_CHECK((int)cudaMemcpyAsync(c->loc + r0 * 4, loc_h + r0 * 4, nr * 16, cudaMemcpyHostToDevice, c->s_h2d));
-        CTX_HOST_CHECK((int)cudaEventRecord(c->ev_in[k], c->s_h2d));
+        if (!loc_alias) SSD_CHECK_CUDA(cudaMemcpyAsync(c->loc + r0 * 4, loc_h + r0 * 4, nr * 16, cudaMemcpyHostToDevice, c->s_h2d));
+        SSD_CHECK_CUDA(cudaEventRecord(c->ev_in[k], c->s_h2d));
     }
-    for (int k = 0, b0 = 0; b0 < B; ++k, b0 += per) {
-        const int nb = std::min(per, B - b0);
-        const size_t r0 = (size_t)b0 * P, nr = (size_t)nb * P;
-        CTX_HOST_CHECK((int)cudaStreamWaitEvent(c->s_main, c->ev_in[k], 0));
+    for (int k = 0; k < nchunks; ++k) {
+        const auto& [b0, nb, r0, nr] = chunk[k];
+        SSD_CHECK_CUDA(cudaStreamWaitEvent(c->s_main, c->ev_in[k], 0));
         void* ws = (char*)c->ws_loss + (size_t)k * c->ws_loss_bytes;
-        float* gl = grads ? (sparse ? gl_alias + r0 * 4 : c->grad_loc + r0 * 4) : nullptr;
-        float* gc = grads ? (sparse ? gc_alias + r0 * C : c->grad_conf + r0 * C) : nullptr;
-        rc = ssdhead_ce_stream(c->conf + r0 * C, nb, P, C, nullptr, (sparse || rows) ? nullptr : gl, (sparse || rows) ? nullptr : gc, ws, c->ws_loss_bytes, c->s_main);
-        CTX_HOST_CHECK(rc);
-        if (k == 0) CTX_HOST_CHECK((int)cudaStreamWaitEvent(c->s_main, c->ev_join, 0));
-        if (sparse) c->pool.wait_chunk(k);                       // chunk k's slices are zero (condition variable, no spinning)
+        float* gl = gl_dev ? gl_dev + r0 * 4 : nullptr;
+        float* gc = gc_dev ? gc_dev + r0 * C : nullptr;
+        const bool zero_fill = ret == Grads::dense_staged;      // the streaming kernel writes the zero background
+        rc = ssdhead_ce_stream(c->conf + r0 * C, nb, P, C, nullptr, zero_fill ? gl : nullptr, zero_fill ? gc : nullptr, ws, c->ws_loss_bytes, c->s_main);
+        if (rc) return rc;
+        if (k == 0) SSD_CHECK_CUDA(cudaStreamWaitEvent(c->s_main, c->ev_join, 0));
+        if (ret == Grads::dense_in_place) c->pool.wait_chunk(k);  // chunk k's slices are zero (condition variable, no spinning)
         const float* loc_k = (loc_alias ? loc_alias : c->loc) + r0 * 4;
         if (rows)
             rc = ssdhead_mine_sparse(loc_k, c->conf + r0 * C, c->gt_xyxy, c->gt_cls, c->gt_off + b0, c->pri_xyxy, c->pri_cxcywh,
@@ -706,23 +667,20 @@ static int loss_host_impl(ssdhead_ctx* c, const float* loc_h, const float* conf_
             rc = ssdhead_mine(loc_k, c->conf + r0 * C, c->gt_xyxy, c->gt_cls, c->gt_off + b0, c->pri_xyxy, c->pri_cxcywh,
                               c->best_prior, c->npos + b0, npos_norm, c->cls_u8 + r0, nb, P, C, neg_ratio, pos_iou,
                               c->chunk_sums + 2 * k, c->losses, gl, gc, nullptr, nullptr, ws, c->ws_loss_bytes, c->s_main);
-        CTX_HOST_CHECK(rc);
-        if (grads && !sparse) {
-            CTX_HOST_CHECK((int)cudaEventRecord(c->ev_out[k], c->s_main));
-            CTX_HOST_CHECK((int)cudaStreamWaitEvent(c->s_d2h, c->ev_out[k], 0));
-            CTX_HOST_CHECK((int)cudaMemcpyAsync(grad_conf_h + r0 * C, gc, nr * C * 4, cudaMemcpyDeviceToHost, c->s_d2h));
-            CTX_HOST_CHECK((int)cudaMemcpyAsync(grad_loc_h + r0 * 4, gl, nr * 16, cudaMemcpyDeviceToHost, c->s_d2h));
+        if (rc) return rc;
+        if (ret == Grads::dense_staged) {
+            SSD_CHECK_CUDA(cudaEventRecord(c->ev_out[k], c->s_main));
+            SSD_CHECK_CUDA(cudaStreamWaitEvent(c->s_d2h, c->ev_out[k], 0));
+            SSD_CHECK_CUDA(cudaMemcpyAsync(grad_conf_h + r0 * C, gc, nr * C * 4, cudaMemcpyDeviceToHost, c->s_d2h));
+            SSD_CHECK_CUDA(cudaMemcpyAsync(grad_loc_h + r0 * 4, gl, nr * 16, cudaMemcpyDeviceToHost, c->s_d2h));
         }
-        used = k + 1;
     }
-    join_all();
-#undef CTX_HOST_CHECK
-    if (sharded) sum_chunks_xchg_kernel<<<1, 1, 0, c->s_main>>>(c->chunk_sums, used, npos_norm, c->sums, c->losses, xa);
-    else sum_chunks_kernel<<<1, 1, 0, c->s_main>>>(c->chunk_sums, used, npos_norm, c->sums, c->losses);
+    if (x) sum_chunks_xchg_kernel<<<1, 1, 0, c->s_main>>>(c->chunk_sums, nchunks, npos_norm, c->sums, c->losses, *x);
+    else sum_chunks_kernel<<<1, 1, 0, c->s_main>>>(c->chunk_sums, nchunks, npos_norm, c->sums, c->losses);
     count_launch();
     SSD_LAUNCH_CHECK();
     SSD_CHECK_CUDA(cudaMemcpyAsync(c->h_losses, c->losses, 2 * sizeof(float), cudaMemcpyDeviceToHost, c->s_main));
-    if (rows_staged) {
+    if (ret == Grads::rows_staged) {
         const size_t nrows = (size_t)B * row_cap;
         SSD_CHECK_CUDA(cudaMemcpyAsync(row_cnt_h, rc_dev, (size_t)B * 2 * 4, cudaMemcpyDeviceToHost, c->s_main));
         SSD_CHECK_CUDA(cudaMemcpyAsync(row_idx_h, ri_dev, nrows * 4, cudaMemcpyDeviceToHost, c->s_main));
@@ -730,7 +688,7 @@ static int loss_host_impl(ssdhead_ctx* c, const float* loc_h, const float* conf_
         SSD_CHECK_CUDA(cudaMemcpyAsync(gloc_rows_h, rgl_dev, nrows * 16, cudaMemcpyDeviceToHost, c->s_main));
     }
     SSD_CHECK_CUDA(cudaStreamSynchronize(c->s_main));
-    if (grads && !sparse) SSD_CHECK_CUDA(cudaStreamSynchronize(c->s_d2h));
+    if (ret == Grads::dense_staged) SSD_CHECK_CUDA(cudaStreamSynchronize(c->s_d2h));
     losses_h[0] = c->h_losses[0];
     losses_h[1] = c->h_losses[1];
     return 0;

@@ -666,13 +666,9 @@ struct MineParams {
     unsigned long long* best_key;   // match workspace: per-gt arg-max keys (left zeroed)
     int* npos_acc;                  //                  natural positives per image (left zeroed)
     unsigned long long* arrive_total;  // workspace word: CTAs that published (high half) | batch positive count (low), left zeroed
-    // cross-GPU exchange of the positive count and the loss sums over NVLink peer memory (xchg_R > 1):
+    // cross-GPU exchange of the positive count and the loss sums over NVLink peer memory (xchg.R > 1):
     // every rank owns an exchange buffer of XCHG_WORDS 64-bit words that its PEERS write into (and it spins on).
-    int xchg_R, xchg_rank;
-    unsigned int xchg_seq;          // step sequence number (>= 1); slots are double-buffered by its parity
-    unsigned long long* const* xchg_peers;   // [R] device table: peer-mapped exchange buffers, indexed by rank
-    unsigned long long* xchg_local;          // this rank's buffer
-    int* err_flag;                  // set to 1 if a bounded wait expired
+    Xchg xchg;
     // sparse gradient return (SPARSE = true; ssdhead_mine_sparse): the rows that carry a gradient, packed per image
     // instead of scattered into dense [B,P,*] tensors.  Slot s of image b: sp_idx[b*cap+s] = prior, sp_conf[(b*cap+s)*C..]
     // its conf-gradient row; the first sp_cnt[2b+1] slots are the positives and also own sp_loc[(b*cap+s)*4..].
@@ -893,13 +889,8 @@ __device__ __forceinline__ void mine_body(const MineParams& p, const LevelTab* _
             // one 64-bit atomic carries both the arrival (high word) and the image's positives (low word): whoever sees
             // gridDim.x arrivals sees the complete batch count in the same word - no fence between two atomics
             const unsigned long long before = atomicAdd(p.arrive_total, (1ull << 32) | (unsigned long long)(unsigned)nb);
-            if (p.xchg_R > 1 && (unsigned)(before >> 32) == gridDim.x - 1u) {
-                // last image of this GPU: its positive count is complete -> one 64-bit store (seq << 32 | count) into
-                // the exchange buffer of every rank (own included) over NVLink
-                const unsigned long long word = ((unsigned long long)p.xchg_seq << 32) | (unsigned)((unsigned)before + (unsigned)nb);
-                for (int q = 0; q < p.xchg_R; ++q)          // the word validates itself (seq in the high half): relaxed, pipelined stores
-                    st_relaxed_sys_u64(p.xchg_peers[q] + xchg_slot(p.xchg_seq, 0, p.xchg_rank), word);
-            }
+            if (p.xchg.R > 1 && (unsigned)(before >> 32) == gridDim.x - 1u)
+                xchg_publish_count(p.xchg, (unsigned)before + (unsigned)nb);    // last image of this GPU: the count is complete
         }
         __syncthreads();
         npos_b = s_fin_npos;
@@ -1071,22 +1062,13 @@ __device__ __forceinline__ void mine_body(const MineParams& p, const LevelTab* _
         // wait that expires is reported (trap on one GPU, err_flag for a peer that never arrived), never papered over
         __shared__ int s_total;
         if (t == 0) {
-            unsigned spins = 0;
-            if (p.xchg_R > 1) {
-                // sharded batch: the counts of all ranks, written into MY exchange buffer by their last CTAs
-                int tot = 0;
-                for (int q = 0; q < p.xchg_R; ++q) {
-                    unsigned long long w;
-                    while ((unsigned)((w = ld_acquire_sys_u64(p.xchg_local + xchg_slot(p.xchg_seq, 0, q))) >> 32) != p.xchg_seq &&
-                           ++spins < (1u << 27)) __nanosleep(64);
-                    tot += (int)(unsigned)w;
-                }
-                if (spins >= (1u << 27)) *p.err_flag = 1;
-                s_total = tot;
+            if (p.xchg.R > 1) {
+                s_total = xchg_gather_count(p.xchg);     // sharded batch: the counts of all ranks, written by their last CTAs
             } else {
                 // The launch is cooperative, so every CTA of the grid is resident and has published its count microseconds
                 // ago.  The spin is still bounded (~2 s) so that a broken launch contract cannot hang the GPU - but it
                 // never continues with a partial count: it traps, and the host sees a launch failure.
+                unsigned spins = 0;
                 unsigned long long w;
                 while ((unsigned)((w = ld_relaxed_gpu_u64(p.arrive_total)) >> 32) < gridDim.x && ++spins < (1u << 25)) __nanosleep(64);
                 if ((unsigned)(w >> 32) < gridDim.x) __trap();
@@ -1305,33 +1287,13 @@ __device__ __forceinline__ void mine_body(const MineParams& p, const LevelTab* _
         if (t == 0) {
             a = 0.0; c = 0.0;
             for (int w = 0; w < MN_W; ++w) { a += s_redd[0][w]; c += s_redd[1][w]; }
-            if (FIN && p.xchg_R > 1) {
-                // all-reduce of the two loss sums through the same peer buffers: values first, then the flag; the
-                // global sums are accumulated in rank order on every rank -> identical bits everywhere
-                for (int q = 0; q < p.xchg_R; ++q) {
-                    st_relaxed_sys_u64(p.xchg_peers[q] + xchg_slot(p.xchg_seq, 1, p.xchg_rank), (unsigned long long)__double_as_longlong(a));
-                    st_relaxed_sys_u64(p.xchg_peers[q] + xchg_slot(p.xchg_seq, 2, p.xchg_rank), (unsigned long long)__double_as_longlong(c));
-                }
-                __threadfence_system();
-                for (int q = 0; q < p.xchg_R; ++q)          // one system fence above orders all value stores before these flags
-                    st_relaxed_sys_u64(p.xchg_peers[q] + xchg_slot(p.xchg_seq, 3, p.xchg_rank), (unsigned long long)p.xchg_seq);
-                unsigned spins = 0;
-                a = 0.0; c = 0.0;
-                for (int q = 0; q < p.xchg_R; ++q) {
-                    while ((unsigned)ld_acquire_sys_u64(p.xchg_local + xchg_slot(p.xchg_seq, 3, q)) != p.xchg_seq && ++spins < (1u << 27)) __nanosleep(64);
-                    a += __longlong_as_double((long long)ld_relaxed_sys_u64(p.xchg_local + xchg_slot(p.xchg_seq, 1, q)));
-                    c += __longlong_as_double((long long)ld_relaxed_sys_u64(p.xchg_local + xchg_slot(p.xchg_seq, 2, q)));
-                }
-                if (spins >= (1u << 27)) *p.err_flag = 1;
-            }
+            if (FIN && p.xchg.R > 1) xchg_allreduce_sums(p.xchg, a, c);
             p.sums[0] = a;
             p.sums[1] = c;
-            const double N = (double)npos_total;
-            p.losses[0] = (float)(a / (4.0 * N));
-            p.losses[1] = (float)(c / N);
+            losses_from_sums(p.losses, a, c, npos_total);
             *p.done_counter = 0u;
             if (FIN) {                   // every CTA has read the total (it did so before it reported done)
-                p.npos_w[p.B] = (p.xchg_R > 1) ? (int)(unsigned)ld_cg_u64(p.arrive_total) : npos_total;    // this rank's own count
+                p.npos_w[p.B] = (p.xchg.R > 1) ? (int)(unsigned)ld_cg_u64(p.arrive_total) : npos_total;    // this rank's own count
                 *p.arrive_total = 0ull;
             }
         }
@@ -1369,9 +1331,7 @@ mine_levels_kernel(const MineParams p, const __grid_constant__ LevelTab lv)
 
 __global__ void finish_loss_kernel(const double* __restrict__ sums, const int* __restrict__ npos_norm, float* __restrict__ losses)
 {
-    const double N = (double)(*npos_norm);
-    losses[0] = (float)(sums[0] / (4.0 * N));
-    losses[1] = (float)(sums[1] / N);
+    losses_from_sums(losses, sums[0], sums[1], *npos_norm);
 }
 
 __global__ void __launch_bounds__(256)
@@ -1563,27 +1523,6 @@ static bool match_cull_enabled(int B, int sumG)
     return B > 0 && sumG >= (long long)min_avg * B && sumG <= SEED_CAP;
 }
 
-// The arguments of the loss entry points, in the order they take them; an entry point leaves what it does not take null.
-struct StepArgs {
-    const float *loc, *conf, *gt_xyxy, *gt_cls;
-    const int32_t* gt_off;
-    const float *pri_xyxy, *pri_cxcywh;
-    int B, P, C, sumG, neg_ratio;
-    float pos_iou;
-    double* sums;
-    float *losses, *grad_loc, *grad_conf;
-    uint8_t* cls_u8;
-    int32_t *best_prior, *npos;
-    uint32_t* mined_mask;
-    float* ce;
-    void* ws_loss; size_t ws_loss_bytes;
-    void* ws_match; size_t ws_match_bytes;
-    void* stream;
-};
-
-// The peer exchange of a batch sharded by image over R GPUs
-struct Xchg { int R, rank; unsigned seq; void* const* peers; void* local; int32_t* err_flag; };
-
 static int check_xchg(const Xchg& x, bool seq_required)
 {
     if (x.R < 1 || x.R > XCHG_MAX_R || x.rank < 0 || x.rank >= x.R || (seq_required && x.seq == 0u)) return SSDHEAD_E_BADARG;
@@ -1624,11 +1563,11 @@ static int check_match(const StepArgs& a)
     return a.ws_match_bytes < match_ws_bytes(a.B, a.sumG) ? SSDHEAD_E_WORKSPACE : 0;
 }
 
-static int check_resident(const StepArgs& a, const void* ws_rows, size_t ws_rows_bytes)
+static int check_resident(const StepArgs& a)
 {
-    if (!ws_rows || !a.grad_loc || !a.grad_conf || a.B < 0 || a.P <= 0 || a.P >= 65536) return SSDHEAD_E_BADARG;
-    if (!aligned16(ws_rows) || !aligned16(a.grad_loc)) return SSDHEAD_E_ALIGN;
-    if (ws_rows_bytes < resident_rows_bytes(a.B, a.P)) return SSDHEAD_E_WORKSPACE;
+    if (!a.ws_rows || !a.grad_loc || !a.grad_conf || a.B < 0 || a.P <= 0 || a.P >= 65536) return SSDHEAD_E_BADARG;
+    if (!aligned16(a.ws_rows) || !aligned16(a.grad_loc)) return SSDHEAD_E_ALIGN;
+    if (a.ws_rows_bytes < resident_rows_bytes(a.B, a.P)) return SSDHEAD_E_WORKSPACE;
     return 0;
 }
 
@@ -1717,7 +1656,7 @@ static int launch_mine_step(const StepArgs& a, const MineParams& prm, const Leve
     int rc = lv ? launch_mine<true>(mine_levels_kernel<21, GRADS, true>, a.B, a.P, st, prm, *lv)
                 : launch_mine<true>(mine_kernel<21, GRADS, true>, a.B, a.P, st, prm);
     if (rc != 1) return rc;
-    if (prm.xchg_R > 1) return SSDHEAD_E_UNSUPPORTED;
+    if (prm.xchg.R > 1) return SSDHEAD_E_UNSUPPORTED;
     rc = launch_finalize(a, mw, st);
     if (rc) return rc;
     return lv ? launch_mine<false>(mine_levels_kernel<21, GRADS, false>, a.B, a.P, st, prm, *lv)
@@ -1737,8 +1676,7 @@ static int step_impl(const StepArgs& a, const LevelTab* lv, const Xchg& x, void*
     const FusedMatch fm = bind_match(a, mw, obj, !lv && match_cull_enabled(a.B, a.sumG) ? lw.seed : nullptr);
     MineParams prm = bind_mine(a, lw, a.npos + a.B, &mw);
     prm.obj_u16 = obj;
-    prm.xchg_R = x.R; prm.xchg_rank = x.rank; prm.xchg_seq = x.seq;
-    prm.xchg_peers = (unsigned long long* const*)x.peers; prm.xchg_local = (unsigned long long*)x.local; prm.err_flag = x.err_flag;
+    prm.xchg = x;
     if (ws_rows) {
         prm.res_base = (unsigned char*)ws_rows;
         prm.res_stride = resident_row_stride(a.P);
@@ -1775,15 +1713,27 @@ static int step_flat(const StepArgs& a, const Xchg& x, void* ws_rows)
     return step_impl(a, nullptr, x, ws_rows);
 }
 
-static int step_levels(const ssdhead_levels* levels, const StepArgs& a, const Xchg& x)
+static int step_levels(const StepArgs& a, const Xchg& x)
 {
     LevelTab lv = {};
     int rc = check_mine(a, false);
     if (!rc) rc = check_match(a);
-    if (!rc) rc = check_levels(levels, a.B, a.P, &lv);
+    if (!rc) rc = check_levels(a.levels, a.B, a.P, &lv);
     if (rc || a.B == 0) return rc;
     if (!aligned16(a.pri_cxcywh)) return SSDHEAD_E_ALIGN;
     return step_impl(a, &lv, x, nullptr);
+}
+
+// A sharded step needs a sequence number; the resident step takes R = 1 with any as one GPU.
+int run_step(StepKind kind, const StepArgs& a, const Xchg* x)
+{
+    const bool resident = kind == StepKind::resident;
+    int rc = resident ? check_resident(a) : 0;
+    if (!rc && x) rc = check_xchg(*x, !resident || x->R > 1);
+    if (rc) return rc;
+    const Xchg none = {};
+    const Xchg& xr = x ? *x : none;
+    return kind == StepKind::levels ? step_levels(a, xr) : step_flat(a, xr, resident ? a.ws_rows : nullptr);
 }
 
 }  // namespace ssdhead
@@ -1847,14 +1797,15 @@ int ssdhead_multibox_step(const float* loc, const float* conf,
                           uint32_t* mined_mask, float* ce,
                           void* ws_loss, size_t ws_loss_bytes, void* ws_match, size_t ws_match_bytes, void* stream)
 {
-    const StepArgs a = {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off,
-                        .pri_xyxy = pri_xyxy, .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG,
-                        .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses,
-                        .grad_loc = grad_loc, .grad_conf = grad_conf, .cls_u8 = cls_u8, .best_prior = best_prior,
-                        .npos = npos, .mined_mask = mined_mask, .ce = ce, .ws_loss = ws_loss,
-                        .ws_loss_bytes = ws_loss_bytes, .ws_match = ws_match, .ws_match_bytes = ws_match_bytes,
-                        .stream = stream};
-    return step_flat(a, Xchg{}, nullptr);
+    return run_step(StepKind::flat,
+                    {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off,
+                     .pri_xyxy = pri_xyxy, .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG,
+                     .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses,
+                     .grad_loc = grad_loc, .grad_conf = grad_conf, .cls_u8 = cls_u8, .best_prior = best_prior,
+                     .npos = npos, .mined_mask = mined_mask, .ce = ce, .ws_loss = ws_loss,
+                     .ws_loss_bytes = ws_loss_bytes, .ws_match = ws_match, .ws_match_bytes = ws_match_bytes,
+                     .stream = stream},
+                    nullptr);
 }
 
 // The same two kernels for a batch sharded by image over R GPUs: the mining kernel exchanges the positive count (before
@@ -1871,15 +1822,15 @@ int ssdhead_multibox_step_sharded(const float* loc, const float* conf,
                           int R, int rank, unsigned int seq, void* const* peers_dev, void* xchg_local_dev, int32_t* err_flag_dev,
                           void* stream)
 {
-    const StepArgs a = {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off,
-                        .pri_xyxy = pri_xyxy, .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG,
-                        .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses,
-                        .grad_loc = grad_loc, .grad_conf = grad_conf, .cls_u8 = cls_u8, .best_prior = best_prior,
-                        .npos = npos, .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes, .ws_match = ws_match,
-                        .ws_match_bytes = ws_match_bytes, .stream = stream};
-    const Xchg x = {R, rank, seq, peers_dev, xchg_local_dev, err_flag_dev};
-    const int rc = check_xchg(x, true);
-    return rc ? rc : step_flat(a, x, nullptr);
+    const Xchg x = {R, rank, seq, (unsigned long long* const*)peers_dev, (unsigned long long*)xchg_local_dev, err_flag_dev};
+    return run_step(StepKind::flat,
+                    {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off,
+                     .pri_xyxy = pri_xyxy, .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG,
+                     .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses,
+                     .grad_loc = grad_loc, .grad_conf = grad_conf, .cls_u8 = cls_u8, .best_prior = best_prior,
+                     .npos = npos, .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes, .ws_match = ws_match,
+                     .ws_match_bytes = ws_match_bytes, .stream = stream},
+                    &x);
 }
 
 // ssdhead_multibox_step with RESIDENT gradient tensors: grad_loc / grad_conf are all-zero when first handed over (together
@@ -1899,18 +1850,16 @@ int ssdhead_multibox_step_resident(const float* loc, const float* conf,
                           int R, int rank, unsigned int seq, void* const* peers_dev, void* xchg_local_dev, int32_t* err_flag_dev,
                           void* stream)
 {
-    const StepArgs a = {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off,
-                        .pri_xyxy = pri_xyxy, .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG,
-                        .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses,
-                        .grad_loc = grad_loc, .grad_conf = grad_conf, .cls_u8 = cls_u8, .best_prior = best_prior,
-                        .npos = npos, .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes, .ws_match = ws_match,
-                        .ws_match_bytes = ws_match_bytes, .stream = stream};
-    Xchg x = {R, rank, seq, peers_dev, xchg_local_dev, err_flag_dev};
-    int rc = check_resident(a, ws_rows, ws_rows_bytes);
-    if (!rc) rc = check_xchg(x, R > 1);
-    if (rc) return rc;
-    if (R == 1) x.R = 0;                                 // one GPU: no exchange
-    return step_flat(a, x, ws_rows);
+    const Xchg x = {R, rank, seq, (unsigned long long* const*)peers_dev, (unsigned long long*)xchg_local_dev, err_flag_dev};
+    return run_step(StepKind::resident,
+                    {.loc = loc, .conf = conf, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off,
+                     .pri_xyxy = pri_xyxy, .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG,
+                     .neg_ratio = neg_ratio, .pos_iou = pos_iou, .sums = sums, .losses = losses,
+                     .grad_loc = grad_loc, .grad_conf = grad_conf, .cls_u8 = cls_u8, .best_prior = best_prior,
+                     .npos = npos, .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes, .ws_match = ws_match,
+                     .ws_match_bytes = ws_match_bytes, .ws_rows = ws_rows, .ws_rows_bytes = ws_rows_bytes,
+                     .stream = stream},
+                    &x);
 }
 
 // ssdhead_multibox_step on per-level head tensors (SURVEY.md 8(f) #3, Model.py:212-235 without the permute/cat copies)
@@ -1922,12 +1871,13 @@ int ssdhead_multibox_step_levels(const ssdhead_levels* levels,
                                  uint8_t* cls_u8, int32_t* best_prior, int32_t* npos,
                                  void* ws_loss, size_t ws_loss_bytes, void* ws_match, size_t ws_match_bytes, void* stream)
 {
-    const StepArgs a = {.gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off, .pri_xyxy = pri_xyxy,
-                        .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG, .neg_ratio = neg_ratio,
-                        .pos_iou = pos_iou, .sums = sums, .losses = losses, .cls_u8 = cls_u8,
-                        .best_prior = best_prior, .npos = npos, .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes,
-                        .ws_match = ws_match, .ws_match_bytes = ws_match_bytes, .stream = stream};
-    return step_levels(levels, a, Xchg{});
+    return run_step(StepKind::levels,
+                    {.levels = levels, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off, .pri_xyxy = pri_xyxy,
+                     .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG, .neg_ratio = neg_ratio,
+                     .pos_iou = pos_iou, .sums = sums, .losses = losses, .cls_u8 = cls_u8,
+                     .best_prior = best_prior, .npos = npos, .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes,
+                     .ws_match = ws_match, .ws_match_bytes = ws_match_bytes, .stream = stream},
+                    nullptr);
 }
 
 // the per-level step of a batch sharded by image over R GPUs (peer-memory exchange inside the mining kernel, as in
@@ -1942,14 +1892,14 @@ int ssdhead_multibox_step_levels_sharded(const ssdhead_levels* levels,
                                  int R, int rank, unsigned int seq, void* const* peers_dev, void* xchg_local_dev, int32_t* err_flag_dev,
                                  void* stream)
 {
-    const StepArgs a = {.gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off, .pri_xyxy = pri_xyxy,
-                        .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG, .neg_ratio = neg_ratio,
-                        .pos_iou = pos_iou, .sums = sums, .losses = losses, .cls_u8 = cls_u8,
-                        .best_prior = best_prior, .npos = npos, .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes,
-                        .ws_match = ws_match, .ws_match_bytes = ws_match_bytes, .stream = stream};
-    const Xchg x = {R, rank, seq, peers_dev, xchg_local_dev, err_flag_dev};
-    const int rc = check_xchg(x, true);
-    return rc ? rc : step_levels(levels, a, x);
+    const Xchg x = {R, rank, seq, (unsigned long long* const*)peers_dev, (unsigned long long*)xchg_local_dev, err_flag_dev};
+    return run_step(StepKind::levels,
+                    {.levels = levels, .gt_xyxy = gt_xyxy, .gt_cls = gt_cls, .gt_off = gt_off, .pri_xyxy = pri_xyxy,
+                     .pri_cxcywh = pri_cxcywh, .B = B, .P = P, .C = C, .sumG = sumG, .neg_ratio = neg_ratio,
+                     .pos_iou = pos_iou, .sums = sums, .losses = losses, .cls_u8 = cls_u8,
+                     .best_prior = best_prior, .npos = npos, .ws_loss = ws_loss, .ws_loss_bytes = ws_loss_bytes,
+                     .ws_match = ws_match, .ws_match_bytes = ws_match_bytes, .stream = stream},
+                    &x);
 }
 
 size_t ssdhead_xchg_bytes(void) { return (size_t)XCHG_WORDS * 8; }

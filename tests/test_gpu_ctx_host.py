@@ -47,12 +47,21 @@ def chunk_layout(B):
     return [(b0, min(per, B - b0)) for b0 in range(0, B, per)]
 
 
-def test_chunk_layout_matches_the_source():
+def test_chunk_table_matches_the_source():
     with open(os.path.join(ROOT, "objectdetection_ssd_b200", "csrc", "host_ctx.cu")) as f:
         src = f.read()
     assert re.search(r"const int nchunks = std::min\(8, std::max\(1, B / 8\)\);", src)
     assert re.search(r"const int per = \(B \+ nchunks - 1\) / nchunks;", src)
-    assert len(re.findall(r"for \(int k = 0, b0 = 0; b0 < B; \+\+k, b0 \+= per\)", src)) >= 3
+    assert re.search(r"constexpr int kMaxChunks = 8;", src)
+    # the chunk table is built once, by the only walk over the batch; the zeroing job, the copies and the kernels walk
+    # the table, and the fold adds all of its chunks
+    assert len(re.findall(r"b0 \+= per", src)) == 1
+    assert re.search(r"for \(int k = 0, b0 = 0; b0 < B; \+\+k, b0 \+= per\) \{\s*const int nb = std::min\(per, B - b0\);"
+                     r"\s*chunk\[k\] = \{b0, nb, \(size_t\)b0 \* P, \(size_t\)nb \* P\};", src)
+    assert len(re.findall(r"for \(int k = 0; k < nchunks; \+\+k\)", src)) == 3
+    assert re.search(r"sum_chunks_xchg_kernel<<<1, 1, 0, c->s_main>>>\(c->chunk_sums, nchunks,", src)
+    assert re.search(r"sum_chunks_kernel<<<1, 1, 0, c->s_main>>>\(c->chunk_sums, nchunks,", src)
+    assert all(len(chunk_layout(B)) == min(8, max(1, B // 8)) for B in range(1, 1025))
     # each chunk mines its own slices and workspace slot, and adds into its own partial sums
     for s in (r"c->gt_off \+ b0", r"c->npos \+ b0", r"c->cls_u8 \+ r0", r"c->chunk_sums \+ 2 \* k",
               r"\(char\*\)c->ws_loss \+ \(size_t\)k \* c->ws_loss_bytes"):
