@@ -12,8 +12,10 @@
  *     unless stated; "dev" pointers are CUDA device pointers, "host" pointers host memory.
  *   - return 0 = ok, <0 = SSDHEAD_E_* (bad argument / unsupported shape), >0 = cudaError_t.
  *   - device entry points are asynchronous on `stream` (a cudaStream_t passed as void*),
- *     allocate nothing, keep no global state and are re-entrant across streams when each
- *     call has its own workspace.  The caller owns every buffer.
+ *     allocate nothing, keep no global state and are re-entrant across streams and host
+ *     threads when each call has its own workspace (kernel launch settings are fixed once
+ *     per device, never per call).  They run on the current device, which must be the
+ *     device of `stream` and of the buffers.  The caller owns every buffer.
  *   - workspaces: sized by ssdhead_workspace_bytes(); must be zero-filled before their first use with a given
  *     (B, P, C, n) - the kernels leave every counter zeroed again, so steady-state steps contain no memsets, but the
  *     position of the counters depends on the shape: re-zero a buffer before reusing it with another shape.

@@ -16,6 +16,8 @@ boxes are not clamped.  An image without ground truth raises IndexError, as the 
 """
 from __future__ import annotations
 
+import threading
+
 import torch
 
 from . import Util as _U
@@ -34,20 +36,27 @@ device = torch.device("cuda" if use_cuda else "cpu")
 process_group = None        # set to a torch.distributed group when the batch is sharded by image over several GPUs
 
 _heads = {}
+_heads_lock = threading.Lock()
 _last = {}
 
 
 def _head(dev=None) -> MultiboxHead:
-    """MultiboxHead for the current module-global prior table (the reference reads ``ancs_xywh`` at call time,
-    Losses.py:23,129,181, so overwriting it - e.g. with a 24 564-prior table - must take effect)."""
+    """MultiboxHead of ``dev`` (default: the current device) for the current module-global prior table (the reference
+    reads ``ancs_xywh`` at call time, Losses.py:23,129,181, so overwriting it - e.g. with a 24 564-prior table - must take
+    effect).  One head per device; threads share it (its calls are ordered on its workspaces)."""
     if dev is None:
         dev = torch.device("cuda", torch.cuda.current_device()) if torch.cuda.is_available() else None
-    key = (str(dev), id(ancs_xywh), tuple(ancs_xywh.shape))
+    table = (id(ancs_xywh), tuple(ancs_xywh.shape))
+    key = (str(dev),) + table
     h = _heads.get(key)
     if h is None:
-        _heads.clear()
-        h = MultiboxHead(ancs_xywh, dev if dev is not None else "cuda")
-        _heads[key] = h
+        with _heads_lock:
+            h = _heads.get(key)
+            if h is None:
+                for k in [k for k in _heads if k[1:] != table]:      # heads of a prior table no longer in use
+                    del _heads[k]
+                h = MultiboxHead(ancs_xywh, dev if dev is not None else "cuda")
+                _heads[key] = h
     return h
 
 

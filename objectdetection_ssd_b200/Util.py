@@ -10,8 +10,9 @@ Mirrored (reference file:line):
   map_prior_to_bb        Util.py:333-352   | subsampling         Util.py:555-560 (used by Model.py)
   class_to_label / label_to_class  Util.py:26-31 | device  Util.py:12-13
 
-Like the reference, the functions move their inputs to ``device`` (CUDA when available) and return
-tensors there.  There is no CPU fallback for them: without a CUDA device they raise.  The one exception
+Like the reference, the functions move host inputs to ``device`` (CUDA when available) and return
+tensors there; inputs already on a CUDA device are computed on, and returned on, that device (the kernels run
+there whatever the current device is).  There is no CPU fallback for them: without a CUDA device they raise.  The one exception
 is ``get_jaccard_tensor11`` (and ``find_intersection`` when it is handed CPU tensors by it), which the
 reference keeps off the GPU deliberately because forked DataLoader workers must not touch CUDA
 (Util.py:305, Util.py:697).
@@ -42,9 +43,13 @@ class_to_label = ['aeroplane', 'bicycle', 'bird', 'boat', 'bottle', 'bus', 'car'
 label_to_class = {name: idx for idx, name in enumerate(class_to_label)}
 
 
-def _cuda_device() -> torch.device:
+def _cuda_device(*inputs) -> torch.device:
+    """The device of the first CUDA tensor among ``inputs``, else ``device``."""
     if not torch.cuda.is_available():
         raise RuntimeError("objectdetection_ssd_b200.Util: no CUDA device - these functions have no CPU fallback")
+    for t in inputs:
+        if isinstance(t, torch.Tensor) and t.is_cuda:
+            return t.device
     d = torch.device(device)
     if d.type != "cuda":
         d = torch.device("cuda")
@@ -66,17 +71,18 @@ def create_priors_ssd300():
 
 
 def _box_op(name, a, b=None):
-    dev = _cuda_device()
+    dev = _cuda_device(a, b)
     a = _f32(a, dev).reshape(-1, 4)
     out = torch.empty_like(a)
     lib = _lib.load()
-    if b is None:
-        rc = getattr(lib, name)(a.data_ptr(), out.data_ptr(), a.shape[0], _stream(dev))
-    else:
-        b = _f32(b, dev).reshape(-1, 4)
-        if b.shape[0] != a.shape[0]:
-            raise RuntimeError(f"The size of tensor a ({a.shape[0]}) must match the size of tensor b ({b.shape[0]})")
-        rc = getattr(lib, name)(a.data_ptr(), b.data_ptr(), out.data_ptr(), a.shape[0], _stream(dev))
+    with torch.cuda.device(dev):
+        if b is None:
+            rc = getattr(lib, name)(a.data_ptr(), out.data_ptr(), a.shape[0], _stream(dev))
+        else:
+            b = _f32(b, dev).reshape(-1, 4)
+            if b.shape[0] != a.shape[0]:
+                raise RuntimeError(f"The size of tensor a ({a.shape[0]}) must match the size of tensor b ({b.shape[0]})")
+            rc = getattr(lib, name)(a.data_ptr(), b.data_ptr(), out.data_ptr(), a.shape[0], _stream(dev))
     _lib.check(rc, name)
     return out
 
@@ -144,11 +150,12 @@ def get_offsets_coords(cxcy, priors_cxcy):
 
 
 def _pair_matrix(name, set_1, set_2):
-    dev = _cuda_device()
+    dev = _cuda_device(set_1, set_2)
     a, b = _f32(set_1, dev).reshape(-1, 4), _f32(set_2, dev).reshape(-1, 4)
     out = torch.empty(a.shape[0], b.shape[0], dtype=torch.float32, device=dev)
-    _lib.check(getattr(_lib.load(), name)(a.data_ptr(), a.shape[0], b.data_ptr(), b.shape[0], out.data_ptr(),
-                                          _stream(dev)), name)
+    with torch.cuda.device(dev):
+        _lib.check(getattr(_lib.load(), name)(a.data_ptr(), a.shape[0], b.data_ptr(), b.shape[0], out.data_ptr(),
+                                              _stream(dev)), name)
     return out
 
 
@@ -183,7 +190,7 @@ def get_jaccard_tensor11(box1_xyxy, box2_xyxy):
 def map_prior_to_bb(jacc, classes, threshold=0.5):
     """Single-image match from a jaccard matrix [n_objects, n_priors] (Util.py:333-352).
     Returns (class_forEach_prior float [P] with 20 = background, obj_forEach_prior int64 [P])."""
-    dev = _cuda_device()
+    dev = _cuda_device(jacc, classes)
     j = _f32(jacc, dev)
     if j.dim() != 2 or j.shape[0] == 0:
         raise IndexError("max(): Expected reduction dim 0 to have non-zero size.")
@@ -193,9 +200,10 @@ def map_prior_to_bb(jacc, classes, threshold=0.5):
     obj = torch.empty(P, dtype=torch.int64, device=dev)
     ov = torch.empty(P, dtype=torch.float32, device=dev)
     bp = torch.empty(G, dtype=torch.int32, device=dev)
-    _lib.check(_lib.load().ssdhead_match_from_iou(j.data_ptr(), cl.data_ptr(), G, P, float(threshold), 20,
-                                                  cls.data_ptr(), obj.data_ptr(), ov.data_ptr(), bp.data_ptr(),
-                                                  _stream(dev)), "ssdhead_match_from_iou")
+    with torch.cuda.device(dev):
+        _lib.check(_lib.load().ssdhead_match_from_iou(j.data_ptr(), cl.data_ptr(), G, P, float(threshold), 20,
+                                                      cls.data_ptr(), obj.data_ptr(), ov.data_ptr(), bp.data_ptr(),
+                                                      _stream(dev)), "ssdhead_match_from_iou")
     return cls.to(dtype=torch.as_tensor(classes).dtype), obj      # classes[obj] keeps the dtype of `classes`
 
 
@@ -205,7 +213,7 @@ def get_map(det_boxes, det_classes, det_scores, gt_boxes, gt_classes):
     Arguments as in the reference: per-image lists of tensors (detections: boxes [n,4], classes [n], scores [n];
     ground truth: boxes [m,4], classes [m]).  Returns ``{class_id: AP}`` for the 20 foreground classes (numpy
     float64).  Equal scores rank by the lower detection index (the reference's sort leaves ties open)."""
-    dev = _cuda_device()
+    dev = _cuda_device(*(x for lists in (det_boxes, det_scores, gt_boxes) for x in lists[:1]))
     n_img = len(det_boxes)
     if n_img == 0 or len(gt_boxes) != n_img:
         raise ValueError("get_map: detections and ground truth must be per-image lists of the same, non-zero length")
@@ -231,10 +239,11 @@ def get_map(det_boxes, det_classes, det_scores, gt_boxes, gt_classes):
     ap = torch.zeros(20, dtype=torch.float64, device=dev)
     lib = _lib.load()
     ws = torch.empty(int(lib.ssdhead_voc_ap_workspace_bytes(N, M, 20)), dtype=torch.uint8, device=dev)
-    _lib.check(lib.ssdhead_voc_ap(db.data_ptr() if N else None, dc.data_ptr() if N else None, ds.data_ptr() if N else None,
-                                  d_off.data_ptr(), N, gb.data_ptr() if M else None, gc.data_ptr() if M else None,
-                                  g_off.data_ptr(), M, n_img, 20, 0.5, levels.data_ptr(), ap.data_ptr(),
-                                  ws.data_ptr(), ws.numel(), _stream(dev)), "ssdhead_voc_ap")
+    with torch.cuda.device(dev):
+        _lib.check(lib.ssdhead_voc_ap(db.data_ptr() if N else None, dc.data_ptr() if N else None,
+                                      ds.data_ptr() if N else None, d_off.data_ptr(), N, gb.data_ptr() if M else None,
+                                      gc.data_ptr() if M else None, g_off.data_ptr(), M, n_img, 20, 0.5, levels.data_ptr(),
+                                      ap.data_ptr(), ws.data_ptr(), ws.numel(), _stream(dev)), "ssdhead_voc_ap")
     out = ap.cpu().numpy()
     return {c: out[c] for c in range(20)}
 

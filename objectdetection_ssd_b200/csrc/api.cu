@@ -2,7 +2,7 @@
 #include "common.cuh"
 
 namespace ssdhead {
-unsigned long long g_launch_count = 0;
+std::atomic<unsigned long long> g_launch_count{0};
 size_t loss_workspace_bytes(int B, int P, int C);          // loss.cu
 size_t detect_workspace_bytes(int B, int P, int C, int n); // detect.cu
 size_t resident_rows_bytes(int B, int P);                   // loss.cu
@@ -14,7 +14,7 @@ extern "C" {
 
 int ssdhead_abi_version(void) { return SSDHEAD_ABI_VERSION; }
 
-uint64_t ssdhead_launch_count(void) { return (uint64_t)g_launch_count; }
+uint64_t ssdhead_launch_count(void) { return (uint64_t)g_launch_count.load(std::memory_order_relaxed); }
 
 const char* ssdhead_error_string(int code)
 {

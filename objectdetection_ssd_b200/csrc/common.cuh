@@ -3,6 +3,10 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdlib.h>
+#include <atomic>
+#include <mutex>
+#include <utility>
+#include <vector>
 #include "../../include/ssdhead.h"
 
 #if defined(__CUDA_ARCH__) && (__CUDA_ARCH__ < 1000)
@@ -11,8 +15,8 @@
 
 namespace ssdhead {
 
-extern unsigned long long g_launch_count;   // host-side counter of kernel launches (api.cu)
-inline void count_launch(int n = 1) { g_launch_count += (unsigned long long)n; }
+extern std::atomic<unsigned long long> g_launch_count;   // host-side counter of kernel launches (api.cu)
+inline void count_launch(int n = 1) { g_launch_count.fetch_add((unsigned long long)n, std::memory_order_relaxed); }
 
 #define SSD_CHECK_CUDA(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) return (int)_e; } while (0)
 #define SSD_LAUNCH_CHECK() do { cudaError_t _e = cudaGetLastError(); if (_e != cudaSuccess) return (int)_e; } while (0)
@@ -203,6 +207,68 @@ static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 b
     cfg.numAttrs = COOP ? 2 : 1;
     return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
+
+// A cooperative launch alone: every CTA co-resident, and (unlike launch_pdl) the kernel starts only after everything in
+// front of it in the stream is complete.
+template <typename... KArgs, typename... Args>
+static inline cudaError_t launch_coop(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args)
+{
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeCooperative;
+    attr[0].val.cooperative = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Per-device state of the launches.  Host threads may call the entry points concurrently, on different devices, so
+// what a launch reads is either set once per device (and never lowered again) or kept per device in atomics.
+// ---------------------------------------------------------------------------------------------
+constexpr int MAX_DEVICES = 64;          // devices past this one are served without the caches
+
+// SM count of the current device
+inline int device_sm_count()
+{
+    static std::atomic<int> cache[MAX_DEVICES];
+    int dev = 0, n = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) { (void)cudaGetLastError(); return 148; }
+    if (dev < MAX_DEVICES && (n = cache[dev].load(std::memory_order_relaxed)) > 0) return n;
+    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) { (void)cudaGetLastError(); n = 148; }
+    if (dev < MAX_DEVICES) cache[dev].store(n, std::memory_order_relaxed);
+    return n;
+}
+
+// Raise `kernel`'s dynamic shared-memory limit on the current device to the most a CTA can opt into (the device's
+// limit less the kernel's static shared memory), once per kernel and device.  The argument checks bound every launch's
+// size below that, so no call sets the attribute again: a call can never lower it between another thread's occupancy
+// query or launch and the launch itself.
+inline cudaError_t smem_limit_once(const void* kernel)
+{
+    static std::mutex m;
+    static std::vector<std::pair<const void*, int>> done;
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    std::lock_guard<std::mutex> lk(m);
+    for (const auto& d : done)
+        if (d.first == kernel && d.second == dev) return cudaSuccess;
+    cudaFuncAttributes fa;
+    int optin = 0;
+    if ((e = cudaFuncGetAttributes(&fa, kernel)) != cudaSuccess ||
+        (e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess ||
+        (e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes)) != cudaSuccess)
+        return e;
+    done.emplace_back(kernel, dev);
+    return cudaSuccess;
+}
+template <typename... KArgs>
+inline cudaError_t smem_limit_once(void (*kernel)(KArgs...)) { return smem_limit_once((const void*)kernel); }
 
 // Workspace of the match (ssdhead_match, and the match fused into the loss steps), zero on entry and on exit:
 // best_key u64[sumG] | tile_counter u32[B] | npos_acc i32[B] | image_counter u32, and in the same 16-byte tail the

@@ -1332,8 +1332,9 @@ detect_nms_levels_kernel(const __grid_constant__ DetLevels dl, const float4* __r
 // SAMPLE (stream kernel only): before their first item the consumer warps compute the floors of the images
 // blockIdx.x, blockIdx.x + gridDim.x, ... and publish them (floor[b], then ready[b] with release) - while the producer's
 // first copies are already in flight; a producer that needs the floor of an image waits for its flag.  Every CTA of the
-// grid is resident (the grid is sized with the occupancy query) and no CTA waits before its own images are published, so
-// the flags always arrive.
+// grid is resident - the grid is sized with the occupancy query and launched cooperatively, so this holds even when
+// kernels of other streams occupy part of the GPU - and no CTA waits before its own images are published, so the flags
+// always arrive.
 struct ItemDesc {                  // what the producer tells the consumers about the item in a stage
     int item;                      // -1: no more items
     int b, r0, nrows, bulk;
@@ -1601,12 +1602,6 @@ static bool shortlist_enabled(int B, int P)
     return (long long)B * P >= 900000;
 }
 
-static int sm_count()
-{
-    static int n = 0;
-    if (!n) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev); }
-    return n;
-}
 
 template <bool FROM_SCORES>
 static int run_detect(const float* loc, const float* conf, const float* pri_cxcywh, int B, int P, int C,
@@ -1640,31 +1635,30 @@ static int run_detect(const float* loc, const float* conf, const float* pri_cxcy
         const size_t smem_stream = (size_t)SST * SCW * 32 * C * 4;
         const size_t smem_sweep = std::max(smem_nms, (size_t)2 * RCW * 32 * C * 4);
         int per_sm = 0;
-        // stream kernel (an ordinary launch: everything in front of this call is complete when it starts, which is what lets its
-        // producers request conf at once): floors + short lists; sweep kernel
+        // stream kernel (a cooperative launch without early start: everything in front of this call is complete when it
+        // starts, which lets its producers request conf at once, and its CTAs wait on each other's floors, so all of them
+        // must be resident even when other streams' kernels hold SMs): floors + short lists; sweep kernel
         if (dl) {
             auto ks = detect_stream_levels_kernel<21>;
             auto kw = detect_sweep_levels_kernel<21>;
-            SSD_CHECK_CUDA(cudaFuncSetAttribute(ks, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_stream));
-            SSD_CHECK_CUDA(cudaFuncSetAttribute(kw, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_sweep));
+            SSD_CHECK_CUDA(smem_limit_once(ks));
+            SSD_CHECK_CUDA(smem_limit_once(kw));
             SSD_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ks, (SCW + 1) * 32, smem_stream));
             if (per_sm < 1) return SSDHEAD_E_UNSUPPORTED;
-            const int grid = (int)std::min<long long>((long long)B * ipi_a, (long long)per_sm * sm_count());
-            ks<<<grid, (SCW + 1) * 32, smem_stream, st>>>(fl, B, P, ipi_a, *dl, w.cand, capI, T);
-            SSD_LAUNCH_CHECK();
+            const int grid = (int)std::min<long long>((long long)B * ipi_a, (long long)per_sm * device_sm_count());
+            SSD_CHECK_CUDA(launch_coop(ks, dim3(grid), dim3((SCW + 1) * 32), smem_stream, st, fl, B, P, ipi_a, *dl, w.cand, capI, T));
             SSD_CHECK_CUDA(launch_pdl(kw, dim3(B), dim3(NT), smem_sweep, st, fl, ipi_a, ipi_b, *dl, (const float4*)pri_cxcywh,
                                       w.cand, w.scr_a, w.scr_b, img_wh, P, NF, T, capI, top_k, iou_thr,
                                       (float4*)out_boxes, out_prob, out_cls, out_prior, out_cnt));
         } else {
             auto ks = detect_stream_kernel<21, FROM_SCORES>;
             auto kw = detect_sweep_kernel<21, FROM_SCORES>;
-            SSD_CHECK_CUDA(cudaFuncSetAttribute(ks, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_stream));
-            SSD_CHECK_CUDA(cudaFuncSetAttribute(kw, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_sweep));
+            SSD_CHECK_CUDA(smem_limit_once(ks));
+            SSD_CHECK_CUDA(smem_limit_once(kw));
             SSD_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ks, (SCW + 1) * 32, smem_stream));
             if (per_sm < 1) return SSDHEAD_E_UNSUPPORTED;
-            const int grid = (int)std::min<long long>((long long)B * ipi_a, (long long)per_sm * sm_count());
-            ks<<<grid, (SCW + 1) * 32, smem_stream, st>>>(fl, conf, B, P, ipi_a, w.cand, capI, T);
-            SSD_LAUNCH_CHECK();
+            const int grid = (int)std::min<long long>((long long)B * ipi_a, (long long)per_sm * device_sm_count());
+            SSD_CHECK_CUDA(launch_coop(ks, dim3(grid), dim3((SCW + 1) * 32), smem_stream, st, fl, conf, B, P, ipi_a, w.cand, capI, T));
             SSD_CHECK_CUDA(launch_pdl(kw, dim3(B), dim3(NT), smem_sweep, st, fl, conf, ipi_a, ipi_b, (const float4*)loc, (const float4*)pri_cxcywh,
                                       w.cand, w.scr_a, w.scr_b, img_wh, P, NF, T, capI, top_k, iou_thr,
                                       (float4*)out_boxes, out_prob, out_cls, out_prior, out_cnt));
@@ -1676,7 +1670,7 @@ static int run_detect(const float* loc, const float* conf, const float* pri_cxcy
     // the exhaustive route
     const dim3 g1(T, B);
     if (dl) {
-        SSD_CHECK_CUDA(cudaFuncSetAttribute(detect_nms_levels_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_nms));
+        SSD_CHECK_CUDA(smem_limit_once(detect_nms_levels_kernel));
         SSD_CHECK_CUDA(launch_pdl(detect_score_levels_kernel<21>, g1, dim3(SC_T), 0, st,
                                   P, min_score, capI, w.cand, w.cand_cnt, w.dir, w.dir_base, w.overflow, w.flag_cnt, *dl));
         SSD_CHECK_CUDA(launch_pdl(detect_nms_levels_kernel, dim3(B), dim3(NT), smem_nms, st,
@@ -1684,7 +1678,7 @@ static int run_detect(const float* loc, const float* conf, const float* pri_cxcy
                                   (const unsigned int*)w.dir_base, w.cand_cnt, w.overflow, img_wh, P, NF, T, capI, top_k, iou_thr,
                                   (float4*)out_boxes, out_prob, out_cls, out_prior, out_cnt));
     } else {
-        SSD_CHECK_CUDA(cudaFuncSetAttribute(detect_nms_kernel<FROM_SCORES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_nms));
+        SSD_CHECK_CUDA(smem_limit_once(detect_nms_kernel<FROM_SCORES>));
         SSD_CHECK_CUDA(launch_pdl(detect_score_kernel<21, FROM_SCORES>, g1, dim3(SC_T), 0, st,
                                   conf, P, min_score, capI, w.cand, w.cand_cnt, w.dir, w.dir_base, w.overflow, w.flag_cnt));
         SSD_CHECK_CUDA(launch_pdl(detect_nms_kernel<FROM_SCORES>, dim3(B), dim3(NT), smem_nms, st,

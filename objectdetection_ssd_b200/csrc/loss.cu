@@ -1394,16 +1394,7 @@ size_t resident_rows_bytes(int B, int P)
     return (size_t)B * resident_row_stride(P);
 }
 
-static int g_num_sms = 0;
-static int num_sms()
-{
-    if (g_num_sms == 0) {
-        int dev = 0, n = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
-        g_num_sms = n;
-    }
-    return g_num_sms;
-}
+static int num_sms() { return device_sm_count(); }
 
 // The streaming CE kernel over [B*P] rows (lv == nullptr) or over the per-level tensors of lv
 template <int C, bool GRADS, bool MATCH>
@@ -1418,7 +1409,7 @@ static int launch_ce_stream(const float* conf, float* ce, float* grad_conf, floa
         const int stride = std::max(SEED_STRIDE, (fm.P + SEED_MAX - 1) / SEED_MAX);
         const int nsamp = (fm.P + stride - 1) / stride;
         const size_t smem_seed = (size_t)nsamp * 16;
-        SSD_CHECK_CUDA(cudaFuncSetAttribute(match_seed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_seed));
+        SSD_CHECK_CUDA(smem_limit_once(match_seed_kernel));
         const int grid_seed = std::min((fm.sumG + 7) / 8, 2 * num_sms());      // sized by the capacity
         const int B = (int)(rows / fm.P);                                       // rows = B * P in every caller
         match_seed_kernel<<<grid_seed, 256, smem_seed, st>>>(fm.gt_xyxy, fm.gt_off, B, fm.pri_xyxy, nsamp, stride,
@@ -1428,7 +1419,7 @@ static int launch_ce_stream(const float* conf, float* ce, float* grad_conf, floa
     }
     if (MATCH && lv) {
         auto kce = ce_stream_levels_kernel<C, GRADS>;
-        SSD_CHECK_CUDA(cudaFuncSetAttribute(kce, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ce));
+        SSD_CHECK_CUDA(smem_limit_once(kce));
         // stride ~ 0.618 T, coprime with T: consecutive visits land in different levels in proportion to their sizes
         LevelTab lt = *lv;
         const long long T = lt.tile0[lt.n];
@@ -1440,7 +1431,7 @@ static int launch_ce_stream(const float* conf, float* ce, float* grad_conf, floa
         SSD_CHECK_CUDA(launch_pdl(kce, dim3(grid_ce), dim3(CE_THREADS), smem_ce, st, ce, rows, fm, lt));
     } else {
         auto kce = ce_stream_kernel<C, GRADS, MATCH>;
-        SSD_CHECK_CUDA(cudaFuncSetAttribute(kce, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ce));
+        SSD_CHECK_CUDA(smem_limit_once(kce));
         const int use_tma = (aligned16(conf) && (!GRADS || (aligned16(grad_conf) && aligned16(grad_loc)))) ? 1 : 0;
         SSD_CHECK_CUDA(launch_pdl(kce, dim3(grid_ce), dim3(CE_THREADS), smem_ce, st, conf, ce, grad_conf, grad_loc, rows, use_tma, fm));
     }
@@ -1461,12 +1452,12 @@ static bool stream_capturing(cudaStream_t st)
 }
 
 // Whether a grid of B CTAs of the mining kernel kmn can be co-resident (*fits); the kernel's dynamic shared memory limit
-// is raised first, as its launch needs and the occupancy query reads it.
+// is raised first (once per device), as its launch needs and the occupancy query reads it.
 template <typename... KArgs>
 static int mine_fits_coresident(void (*kmn)(KArgs...), int B, int P, bool* fits)
 {
     const size_t smem_mn = mine_smem_bytes(P);
-    SSD_CHECK_CUDA(cudaFuncSetAttribute(kmn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_mn));
+    SSD_CHECK_CUDA(smem_limit_once(kmn));
     int per_sm = 0;
     SSD_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kmn, MN_T, smem_mn));
     *fits = (long long)per_sm * num_sms() >= B;
@@ -1481,7 +1472,7 @@ static int launch_mine(void (*kmn)(KArgs...), int B, int P, cudaStream_t st, Arg
 {
     const size_t smem_mn = mine_smem_bytes(P);
     if (!FIN) {
-        SSD_CHECK_CUDA(cudaFuncSetAttribute(kmn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_mn));
+        SSD_CHECK_CUDA(smem_limit_once(kmn));
         SSD_CHECK_CUDA(launch_pdl(kmn, dim3(B), dim3(MN_T), smem_mn, st, args...));
         count_launch();
         return 0;
@@ -1492,15 +1483,21 @@ static int launch_mine(void (*kmn)(KArgs...), int B, int P, cudaStream_t st, Arg
     // cooperative (co-residency guaranteed) AND programmatic stream serialization (the grid may become resident while
     // the streaming kernel drains; it waits in pdl_wait()).  Runtimes that refuse the combination get the plain
     // cooperative launch.  The combination is first tried on an eager launch: a refused launch inside a stream capture
-    // would invalidate the capture, so a capture takes it only once an eager launch has shown it is accepted.
-    static int with_pdl = 0;                                 // 0: not tried yet, 1: accepted, -1: refused
-    const bool capturing = with_pdl >= 0 && stream_capturing(st);
-    if (with_pdl == 1 || (with_pdl == 0 && !capturing)) {
+    // would invalidate the capture, so a capture takes it only once an eager launch has shown it is accepted.  What was
+    // learnt is kept per device (threads may launch on several at once).
+    static std::atomic<int> pdl_state[MAX_DEVICES];          // 0: not tried yet, 1: accepted, -1: refused
+    int dev = 0;
+    SSD_CHECK_CUDA(cudaGetDevice(&dev));
+    std::atomic<int> untracked{0};
+    std::atomic<int>& with_pdl = dev < MAX_DEVICES ? pdl_state[dev] : untracked;
+    const int known = with_pdl.load(std::memory_order_relaxed);
+    const bool capturing = known >= 0 && stream_capturing(st);
+    if (known == 1 || (known == 0 && !capturing)) {
         const cudaError_t e = launch_pdl<true>(kmn, dim3(B), dim3(MN_T), smem_mn, st, args...);
-        if (e == cudaSuccess) { with_pdl = 1; count_launch(); return 0; }
+        if (e == cudaSuccess) { with_pdl.store(1, std::memory_order_relaxed); count_launch(); return 0; }
         if (capturing) return (int)e;
         (void)cudaGetLastError();
-        with_pdl = -1;
+        with_pdl.store(-1, std::memory_order_relaxed);
     }
     static_assert(std::is_same<std::tuple<std::decay_t<Args>...>, std::tuple<std::decay_t<KArgs>...>>::value,
                   "the cooperative launch passes the arguments by address: they must have the kernel's parameter types");

@@ -10,6 +10,8 @@ Reference call sites this layer serves: ``ssd`` (Losses.py:119-134), ``ssd1_`` (
 """
 from __future__ import annotations
 
+import threading
+from contextlib import contextmanager
 from typing import List, Optional, Sequence
 
 import numpy as np
@@ -42,6 +44,7 @@ def require_cuda(dev) -> torch.device:
 
 
 _staging_pool = None     # pinned.StagingPool, created with the first host-list batch
+_staging_pool_lock = threading.Lock()
 
 
 def refuse_capture(what: str) -> None:
@@ -88,7 +91,9 @@ class PackedGT:
             global _staging_pool
             if _staging_pool is None:
                 from .pinned import StagingPool
-                _staging_pool = StagingPool()
+                with _staging_pool_lock:
+                    if _staging_pool is None:
+                        _staging_pool = StagingPool()
             from .pinned import gt_layout
             st = _staging_pool.acquire(self.sumG, self.B)
             try:
@@ -98,8 +103,8 @@ class PackedGT:
                 raise
             blk = torch.empty(st.nbytes, dtype=torch.uint8, device=dev)
             blk.copy_(st.raw_t, non_blocking=True)
-            if st.event is None:
-                st.event = torch.cuda.Event()
+            if st.event is None or st.event_dev != dev:         # an event is recorded on streams of one device only
+                st.event, st.event_dev = torch.cuda.Event(), dev
             st.event.record(torch.cuda.current_stream(dev))
             _staging_pool.release(st, st.event)
             o0, o1, o2, _ = gt_layout(st.capacity, self.B)
@@ -149,7 +154,12 @@ def _staging_views(st):
 
 
 class MultiboxHead:
-    """Prior tables and workspaces of one CUDA device."""
+    """Prior tables and workspaces of one CUDA device.
+
+    One head may be used from several streams and host threads: every library call runs under the head's lock, on the
+    head's device, and waits for the last use of each workspace it takes when that use was on another stream."""
+
+    _ordered = True          # calls on different streams are ordered on the workspaces (see _calls)
 
     def __init__(self, priors_cxcywh: torch.Tensor, device=None, num_classes: int = 21):
         self.dev = require_cuda(device if device is not None else "cuda")
@@ -161,8 +171,28 @@ class MultiboxHead:
         self.pri_xyxy = cxcywh_to_xyxy_host(pc).to(self.dev)     # same fp32 ops as Util.py:93-96
         self._ws = {}
         self._ws_need = {}
+        self._ws_last = {}       # which -> (event recorded behind the workspace's last use, id of that use's stream)
+        self._lock = threading.RLock()
 
     # ------------------------------------------------------------------ workspaces
+    @contextmanager
+    def _calls(self, *specs):
+        """Context of one or more library calls: this head's lock and device, and the workspaces ``specs`` (``(which, B,
+        n)`` each, as ``_workspace`` takes them) ready for the current stream.  One event recorded behind the calls marks
+        the new last use of those workspaces, so a later call on another stream (or from another thread) waits for it
+        before it grows, re-zeroes or uses one of them."""
+        with self._lock, torch.cuda.device(self.dev):
+            bufs = [self._workspace(*sp) for sp in specs]
+            try:
+                yield bufs
+            finally:
+                if specs and self._ordered:
+                    cur = torch.cuda.current_stream(self.dev)
+                    ev = torch.cuda.Event()
+                    ev.record(cur)
+                    for sp in specs:
+                        self._ws_last[sp[0]] = (ev, cur.cuda_stream)
+
     def _workspace(self, which: int, B: int, n: int) -> torch.Tensor:
         # sized for n rounded up to a multiple of 1024 (the gt count changes every training step; a larger buffer is
         # always accepted), so the size query leaves the per-step path
@@ -178,13 +208,25 @@ class MultiboxHead:
         # a buffer that was zero-filled once stays valid when only the gt count `n` changes (it does on every training
         # step).  A change of the batch size is re-zeroed anyway - it is rare and keeps the header's contract
         # (include/ssdhead.h, "re-zero a buffer before reusing it with another shape") to the letter.
+        # On another stream than its last use, the current stream first waits for that use: the zero-fill, the replacement and
+        # the call are then ordered after it.  A buffer used on a stream other than the one that allocated it is recorded on
+        # that stream, so the caching allocator does not hand its memory out again before that stream is done with it.
         key = B
-        cur, last = self._ws.get(which, (None, None))
+        st = torch.cuda.current_stream(self.dev)
+        used = self._ws_last.get(which)
+        if used is not None and used[1] != st.cuda_stream:
+            st.wait_event(used[0])
+        cur, last, home = self._ws.get(which, (None, None, None))
         if cur is None or cur.numel() < need:
-            cur = torch.zeros(max(need, 2 * (cur.numel() if cur is not None else 0)) + 4096, dtype=torch.uint8, device=self.dev)
+            with torch.cuda.device(self.dev):
+                cur = torch.zeros(max(need, 2 * (cur.numel() if cur is not None else 0)) + 4096, dtype=torch.uint8,
+                                  device=self.dev)
+            home = st.cuda_stream
         elif last != key:
             cur.zero_()
-        self._ws[which] = (cur, key)
+        if st.cuda_stream != home:
+            cur.record_stream(st)
+        self._ws[which] = (cur, key, home)
         return cur
 
     def _dense_f32(self, t: torch.Tensor) -> torch.Tensor:
@@ -208,12 +250,12 @@ class MultiboxHead:
         """Losses.py:150-171.  Returns dict(best_prior, npos[B+1], cls_u8[B,P], obj[B,P]|None, cls[B,P]|None)."""
         B = gt.B
         o = outs if outs is not None else self._match_outputs(gt, want_maps)
-        ws = self._workspace(_lib.WS_MATCH, B, gt.sumG)
-        _lib.check(self.lib.ssdhead_match(
-            _ptr(gt.boxes), _ptr(gt.classes), _ptr(gt.off), _ptr(self.pri_xyxy),
-            B, self.P, self.C, gt.sumG, pos_iou,
-            _ptr(o["best_prior"]), _ptr(o["npos"]), _ptr(o["cls_u8"]), _ptr(o["obj"]), _ptr(o["cls"]),
-            _ptr(ws), ws.numel(), _stream(self.dev)), "ssdhead_match")
+        with self._calls((_lib.WS_MATCH, B, gt.sumG)) as (ws,):
+            _lib.check(self.lib.ssdhead_match(
+                _ptr(gt.boxes), _ptr(gt.classes), _ptr(gt.off), _ptr(self.pri_xyxy),
+                B, self.P, self.C, gt.sumG, pos_iou,
+                _ptr(o["best_prior"]), _ptr(o["npos"]), _ptr(o["cls_u8"]), _ptr(o["obj"]), _ptr(o["cls"]),
+                _ptr(ws), ws.numel(), _stream(self.dev)), "ssdhead_match")
         return o
 
     # ------------------------------------------------------------------ loss
@@ -240,13 +282,19 @@ class MultiboxHead:
         if taps:
             mined = torch.empty(B, (P + 31) // 32, dtype=torch.int32, device=self.dev)
             ce = torch.empty(B, P, dtype=torch.float32, device=self.dev)
-        ws = self._workspace(_lib.WS_LOSS, B, 0)
-        cur = torch.cuda.current_stream(self.dev)
         m = match
+        specs = [(_lib.WS_LOSS, B, 0)] + ([(_lib.WS_MATCH, B, gt.sumG)] if m is None else [])
+        with self._calls(*specs) as wss:
+            return self._loss_calls(loc, conf, gt, B, P, C, neg_ratio, pos_iou, group, m, wss, sums, losses, grad_loc,
+                                    grad_conf, mined, ce)
+
+    def _loss_calls(self, loc, conf, gt, B, P, C, neg_ratio, pos_iou, group, m, wss, sums, losses, grad_loc, grad_conf,
+                    mined, ce):
+        ws, wm = wss[0], (wss[1] if len(wss) > 1 else None)
+        cur = torch.cuda.current_stream(self.dev)
         if m is None and group is None:
             # hot path, one GPU: two kernels (streaming CE + fused natural match; mining + fused forced-match finaliser)
             m = self._match_outputs(gt, False)
-            wm = self._workspace(_lib.WS_MATCH, B, gt.sumG)
             _lib.check(self.lib.ssdhead_multibox_step(
                 _ptr(loc), _ptr(conf), _ptr(gt.boxes), _ptr(gt.classes), _ptr(gt.off),
                 _ptr(self.pri_xyxy), _ptr(self.pri_cxcywh), B, P, C, gt.sumG, int(neg_ratio), float(pos_iou),
@@ -260,7 +308,6 @@ class MultiboxHead:
             # sharded batch: the natural match rides inside the CE streaming kernel, a small finaliser applies the
             # forced-match override; the positive count is all-reduced before the mining kernel
             m = self._match_outputs(gt, False)
-            wm = self._workspace(_lib.WS_MATCH, B, gt.sumG)
             _lib.check(self.lib.ssdhead_ce_match_stream(
                 _ptr(conf), _ptr(gt.boxes), _ptr(gt.classes), _ptr(gt.off), _ptr(self.pri_xyxy),
                 B, P, C, gt.sumG, float(pos_iou), _ptr(ce), _ptr(grad_loc), _ptr(grad_conf),
@@ -342,22 +389,22 @@ class MultiboxHead:
         sums = torch.empty(2, dtype=torch.float64, device=self.dev)
         losses = torch.empty(2, dtype=torch.float32, device=self.dev)
         m = self._match_outputs(gt, False)
-        ws = self._workspace(_lib.WS_LOSS, B, 0)
-        wm = self._workspace(_lib.WS_MATCH, B, gt.sumG)
         import ctypes
-        _lib.check(self.lib.ssdhead_multibox_step_levels(
-            ctypes.addressof(st), _ptr(gt.boxes), _ptr(gt.classes), _ptr(gt.off),
-            _ptr(self.pri_xyxy), _ptr(self.pri_cxcywh), B, self.P, self.C, gt.sumG, int(neg_ratio), float(pos_iou),
-            _ptr(sums), _ptr(losses), _ptr(m["cls_u8"]), _ptr(m["best_prior"]), _ptr(m["npos"]),
-            _ptr(ws), ws.numel(), _ptr(wm), wm.numel(), _stream(self.dev)), "ssdhead_multibox_step_levels")
+        with self._calls((_lib.WS_LOSS, B, 0), (_lib.WS_MATCH, B, gt.sumG)) as (ws, wm):
+            _lib.check(self.lib.ssdhead_multibox_step_levels(
+                ctypes.addressof(st), _ptr(gt.boxes), _ptr(gt.classes), _ptr(gt.off),
+                _ptr(self.pri_xyxy), _ptr(self.pri_cxcywh), B, self.P, self.C, gt.sumG, int(neg_ratio), float(pos_iou),
+                _ptr(sums), _ptr(losses), _ptr(m["cls_u8"]), _ptr(m["best_prior"]), _ptr(m["npos"]),
+                _ptr(ws), ws.numel(), _ptr(wm), wm.numel(), _stream(self.dev)), "ssdhead_multibox_step_levels")
         return dict(losses=losses, sums=sums, npos=m["npos"], grad_loc=grads[0] if grads else None,
                     grad_conf=grads[1] if grads else None, best_prior=m["best_prior"], cls_u8=m["cls_u8"],
                     _keep=(locs, confs))
 
     def scale_grads(self, grad_loc: torch.Tensor, grad_conf: torch.Tensor, gout: torch.Tensor):
-        _lib.check(self.lib.ssdhead_scale_grads(_ptr(grad_loc), grad_loc.numel(), _ptr(grad_conf),
-                                                grad_conf.numel(), _ptr(gout), _stream(self.dev)),
-                   "ssdhead_scale_grads")
+        with self._calls():
+            _lib.check(self.lib.ssdhead_scale_grads(_ptr(grad_loc), grad_loc.numel(), _ptr(grad_conf),
+                                                    grad_conf.numel(), _ptr(gout), _stream(self.dev)),
+                       "ssdhead_scale_grads")
 
 
 def _upstream(head, g_loc_loss, g_conf_loss) -> torch.Tensor:
@@ -426,19 +473,19 @@ def _detect(head: MultiboxHead, a: torch.Tensor, b: torch.Tensor, min_score: flo
                cls=torch.empty(B, top_k, dtype=torch.int32, device=dev),
                prior=torch.empty(B, top_k, dtype=torch.int32, device=dev),
                cnt=torch.empty(B, dtype=torch.int32, device=dev))
-    ws = head._workspace(_lib.WS_DETECT, B, int(max_candidates))
-    if from_scores:
-        rc = head.lib.ssdhead_detect_from_scores(
-            _ptr(a), _ptr(b), B, P, C, float(min_score), float(iou_thr), int(top_k), _ptr(wh), int(max_candidates),
-            _ptr(out["boxes"]), _ptr(out["prob"]), _ptr(out["cls"]), _ptr(out["prior"]), _ptr(out["cnt"]),
-            _ptr(ws), ws.numel(), _stream(dev))
-    else:
-        rc = head.lib.ssdhead_detect(
-            _ptr(a), _ptr(b), _ptr(head.pri_cxcywh), B, P, C, float(min_score), float(iou_thr), int(top_k),
-            _ptr(wh), int(max_candidates),
-            _ptr(out["boxes"]), _ptr(out["prob"]), _ptr(out["cls"]), _ptr(out["prior"]), _ptr(out["cnt"]),
-            _ptr(ws), ws.numel(), _stream(dev))
-    _lib.check(rc, "ssdhead_detect")
+    with head._calls((_lib.WS_DETECT, B, int(max_candidates))) as (ws,):
+        if from_scores:
+            rc = head.lib.ssdhead_detect_from_scores(
+                _ptr(a), _ptr(b), B, P, C, float(min_score), float(iou_thr), int(top_k), _ptr(wh), int(max_candidates),
+                _ptr(out["boxes"]), _ptr(out["prob"]), _ptr(out["cls"]), _ptr(out["prior"]), _ptr(out["cnt"]),
+                _ptr(ws), ws.numel(), _stream(dev))
+        else:
+            rc = head.lib.ssdhead_detect(
+                _ptr(a), _ptr(b), _ptr(head.pri_cxcywh), B, P, C, float(min_score), float(iou_thr), int(top_k),
+                _ptr(wh), int(max_candidates),
+                _ptr(out["boxes"]), _ptr(out["prob"]), _ptr(out["cls"]), _ptr(out["prior"]), _ptr(out["cnt"]),
+                _ptr(ws), ws.numel(), _stream(dev))
+        _lib.check(rc, "ssdhead_detect")
     return out
 
 
@@ -446,10 +493,10 @@ def detect_fallbacks(head: MultiboxHead, B: int, max_candidates: int = 0) -> int
     """Images of the LAST detect call with this batch size that the short-list route could not decide (they were served
     by the exhaustive kernels; the output is the same either way).  Synchronises the stream."""
     import ctypes
-    ws = head._workspace(_lib.WS_DETECT, B, int(max_candidates))
     n = ctypes.c_int32(-1)
-    _lib.check(head.lib.ssdhead_detect_fallbacks(_ptr(ws), ws.numel(), B, head.P, head.C, int(max_candidates),
-                                                 ctypes.addressof(n), _stream(head.dev)), "ssdhead_detect_fallbacks")
+    with head._calls((_lib.WS_DETECT, B, int(max_candidates))) as (ws,):
+        _lib.check(head.lib.ssdhead_detect_fallbacks(_ptr(ws), ws.numel(), B, head.P, head.C, int(max_candidates),
+                                                     ctypes.addressof(n), _stream(head.dev)), "ssdhead_detect_fallbacks")
     return int(n.value)
 
 
@@ -510,12 +557,12 @@ def detect_levels(head: MultiboxHead, loc_levels, conf_levels, min_score=0.2, io
                cls=torch.empty(B, top_k, dtype=torch.int32, device=dev),
                prior=torch.empty(B, top_k, dtype=torch.int32, device=dev),
                cnt=torch.empty(B, dtype=torch.int32, device=dev))
-    ws = head._workspace(_lib.WS_DETECT, B, int(max_candidates))
-    _lib.check(head.lib.ssdhead_detect_levels(
-        ctypes.addressof(st), _ptr(head.pri_cxcywh), B, head.P, head.C, float(min_score), float(iou_thr), int(top_k),
-        _ptr(wh), int(max_candidates),
-        _ptr(out["boxes"]), _ptr(out["prob"]), _ptr(out["cls"]), _ptr(out["prior"]), _ptr(out["cnt"]),
-        _ptr(ws), ws.numel(), _stream(dev)), "ssdhead_detect_levels")
+    with head._calls((_lib.WS_DETECT, B, int(max_candidates))) as (ws,):
+        _lib.check(head.lib.ssdhead_detect_levels(
+            ctypes.addressof(st), _ptr(head.pri_cxcywh), B, head.P, head.C, float(min_score), float(iou_thr), int(top_k),
+            _ptr(wh), int(max_candidates),
+            _ptr(out["boxes"]), _ptr(out["prob"]), _ptr(out["cls"]), _ptr(out["prior"]), _ptr(out["cnt"]),
+            _ptr(ws), ws.numel(), _stream(dev)), "ssdhead_detect_levels")
     return out
 
 
@@ -525,7 +572,10 @@ class _FixedWorkspaces(MultiboxHead):
     """A MultiboxHead whose workspaces are allocated and zero-filled by the first call that needs each of them, outside
     any capture, and then never resized, moved or re-zeroed: a captured graph keeps pointing at them, and the kernels
     leave every counter zeroed again.  Its callers keep the batch size and the gt capacity fixed, so each workspace has
-    one size."""
+    one size.  No events: an event recorded inside a capture cannot be waited on outside it, so the caller keeps its calls
+    and replays on one stream."""
+
+    _ordered = False
 
     def _workspace(self, which: int, B: int, n: int) -> torch.Tensor:
         cur = self._ws.get(which)
@@ -536,7 +586,8 @@ class _FixedWorkspaces(MultiboxHead):
             need = int(self.lib.ssdhead_workspace_bytes(which, B, self.P, self.C, n))
             if need == 0:
                 raise RuntimeError(f"ssdhead: unsupported shape for this entry point (B={B}, P={self.P}, C={self.C})")
-            cur = torch.zeros(need, dtype=torch.uint8, device=self.dev)
+            with torch.cuda.device(self.dev):
+                cur = torch.zeros(need, dtype=torch.uint8, device=self.dev)
             self._ws[which] = cur
         return cur
 

@@ -12,6 +12,7 @@ the copy that read the block.
 from __future__ import annotations
 
 import ctypes as C
+import threading
 from typing import List, Optional, Tuple
 
 import numpy as np
@@ -77,38 +78,46 @@ class Staging:
         self.offsets = self.block.view(o2, self.B + 1, np.int32)
         self.raw = self.block.view(0, total, np.uint8)
         self.event = None                      # torch.cuda.Event recorded after the copy that last read the block
+        self.event_dev = None                  # the device of that copy's stream
 
 
 class StagingPool:
     """Grow-on-demand pool of ``Staging`` blocks of one (capacity, B) class; a block is handed out again only after the
-    CUDA event recorded behind its last upload has completed (normally long ago: no wait)."""
+    CUDA event recorded behind its last upload has completed (normally long ago: no wait).  Host threads may share a
+    pool: a block is handed to one caller at a time."""
 
     def __init__(self, max_free: int = 8):
         self.free: List[Staging] = []
         self.max_free = max_free
+        self._lock = threading.Lock()
 
     def acquire(self, capacity: int, B: int, exact: bool = False) -> Staging:
         """A block for ``capacity`` gts of ``B`` images.  ``exact``: exactly that capacity, so the block has the layout
         of a device buffer made with ``gt_layout(capacity, B)`` and goes up in one copy."""
         def fits(s):
             return s.B == B and (s.capacity == capacity if exact else s.capacity >= capacity)
-        best: Optional[int] = None
-        for i, s in enumerate(self.free):
-            if fits(s) and (s.event is None or s.event.query()):
-                if best is None or s.capacity < self.free[best].capacity:
-                    best = i
-        if best is not None:
-            return self.free.pop(best)
-        for i, s in enumerate(self.free):      # everything of this shape is still in flight: wait for the oldest
-            if fits(s) and len(self.free) >= self.max_free:
-                s = self.free.pop(i)
-                s.event.synchronize()
-                return s
+        oldest = None
+        with self._lock:
+            best: Optional[int] = None
+            for i, s in enumerate(self.free):
+                if fits(s) and (s.event is None or s.event.query()):
+                    if best is None or s.capacity < self.free[best].capacity:
+                        best = i
+            if best is not None:
+                return self.free.pop(best)
+            for i, s in enumerate(self.free):  # everything of this shape is still in flight: wait for the oldest
+                if fits(s) and len(self.free) >= self.max_free:
+                    oldest = self.free.pop(i)
+                    break
+        if oldest is not None:
+            oldest.event.synchronize()         # outside the lock: other threads keep using the pool meanwhile
+            return oldest
         cap = capacity if exact else max(64, 1 << (max(capacity, 1) - 1).bit_length())   # round up: ragged batches reuse one block
         return Staging(cap, B)
 
     def release(self, s: Staging, event) -> None:
         s.event = event
-        self.free.append(s)
-        if len(self.free) > 4 * self.max_free:                         # shapes that stopped occurring
-            self.free = self.free[-2 * self.max_free:]
+        with self._lock:
+            self.free.append(s)
+            if len(self.free) > 4 * self.max_free:                     # shapes that stopped occurring
+                self.free = self.free[-2 * self.max_free:]

@@ -105,3 +105,26 @@ def test_head_levels_are_views_of_the_reference_layout():
     assert torch.equal(torch.cat(confs_cl, 1), ref_conf)
     # 1x1 maps have ambiguous strides; every other NHWC conv output is consumed in place
     assert all(v.data_ptr() == m.data_ptr() and v.is_contiguous() for v, m in zip(confs_cl[:5], cl[:5]))
+
+
+def test_kernel_attributes_are_set_once_per_device_not_per_call():
+    """The per-call launch path never sets a function attribute: a call that lowered a kernel's shared-memory limit
+    could break another thread's launch of a larger shape between that thread's set and its launch.  The only
+    cudaFuncSetAttribute of the library is the once-per-kernel-and-device raise in common.cuh."""
+    import glob
+    import os
+    import re
+    csrc = os.path.join(os.path.dirname(PR.__file__), "csrc")
+    hits = {}
+    for path in glob.glob(os.path.join(csrc, "*.cu*")):
+        with open(path) as f:
+            text = re.sub(r"//[^\n]*", "", f.read())
+        n = len(re.findall(r"\bcudaFuncSetAttribute\s*\(", text))
+        if n:
+            hits[os.path.basename(path)] = n
+    assert hits == {"common.cuh": 1}, hits
+    with open(os.path.join(csrc, "common.cuh")) as f:
+        text = f.read()
+    body = text[text.index("inline cudaError_t smem_limit_once(const void* kernel)"):]
+    body = body[:body.index("\n}\n")]
+    assert "cudaFuncSetAttribute" in body and "std::lock_guard" in body
